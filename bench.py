@@ -2,6 +2,7 @@
 """bench.py -- the driver's measurement contract for the DDRL4NAV actor-learner hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload pong|navlaser|navimg|navlaser3] [--impl reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -13,6 +14,16 @@ e2e     = the same through the public API (BackwardModule.train_on) from PINNED 
           batch and D2H of the losses inside the timed region, every step.
 extra   = Forward-module actions/s (PPO.act), GAE elements/s, per-kernel-class device time.
 --impl reference = the reference's CPU path (oracle port, torch CPU, all host threads), rank 0 only.
+--dump-outputs DIR = after the K timed learn calls, rank 0 writes what the last one handed its caller: DIR/losses.npy (float64
+          [iterations, 4]: PpoTotalLoss, ActorLoss, VLoss, EntLoss) and DIR/param.<name>.npy (float32, every parameter after
+          the call).  Inputs, initial weights and sampling draws are seeded, and the whole run uses the engine's deterministic
+          mode (DESIGN.md section 3; config.deterministic in the JSON line): the default mode adds block partials with
+          unordered atomics, and Adam amplifies their last-bit differences from iteration to iteration (weights 1e-2 apart
+          after 5 learn calls), so only deterministic mode writes the same files every run.  Two builds that add in a
+          different order still differ in the last bits, which Adam amplifies the same way: compare them with a tolerance.
+          The whole run, timings included, is of deterministic mode, which covers the tc3 engine only (--gemm-mode tc3) and
+          is slower (Pong: 67 vs 48 ms per step on one B200 at a 1000 W power limit); time the default mode without
+          --dump-outputs.
 Prints ONE JSON line on rank 0.
 """
 import argparse
@@ -221,6 +232,10 @@ def run_ours(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
+    # the initial weights, the actions sampled for the batch and the old log-prob noise come from torch's global generators
+    torch.manual_seed(1000 + rank)
+    if args.dump_outputs:
+        kernels.set_deterministic(True)
     # host threads and the pinned buffers they allocate next to the GPU's PCIe root (ddrl4nav_b200.dist.bind_host_to_device);
     # DDRL_NO_NUMA_BIND=1 leaves the placement to the scheduler
     from ddrl4nav_b200.dist import bind_host_to_device
@@ -265,10 +280,13 @@ def run_ours(args):
 
     # ---- headline: K learn calls, inputs resident in HBM
     last_losses = {}
+    step_losses = []                    # the loss dicts of the latest learn call, one per iteration
 
     def step_resident():
+        step_losses.clear()
         for loss, upd, last in net.learn(exp_dev):
             last_losses.update(loss)
+            step_losses.append(loss)
 
     if args.profile_step:
         for _ in range(args.warmup):
@@ -290,6 +308,8 @@ def run_ours(args):
     launches = kernels.launch_count()
     clocks = sampler.stop()
     value = world * B * ITERS * args.steps / sec
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_losses, net)
 
     # ---- e2e: same metric through BackwardModule.train_on from pinned host buffers (H2D + D2H per step)
     bm = BackwardModule(net, device=dev)
@@ -462,6 +482,7 @@ def run_ours(args):
             "data": "synthetic",
             "config": {"workload": wl["desc"], "rows_per_gpu": B, "global_batch": B * world, "iters_per_step": ITERS,
                        "parallelism": "dp%d" % world, "gemm_mode": args.gemm_mode, "collective": collective,
+                       "deterministic": bool(args.dump_outputs),
                        "l2": "inputs larger than L2 (%.0f MB observations per GPU)" % (B * wl["obs_bytes"] / 1e6),
                        "host_affinity": ("CPUs of NUMA node %d (the GPU's)" % host_bind[1]) if host_bind is not None else "unchanged"},
             "e2e": {"value": round(e2e_value, 1), "unit": "learner sample-iterations/s", "h2d_bytes_per_step": h2d_bytes,
@@ -490,6 +511,23 @@ def run_ours(args):
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()
+
+
+LOSS_KEYS = ("PpoTotalLoss", "ActorLoss", "VLoss", "EntLoss")
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, step_losses, net):
+    """What one learn call hands its caller: the per-iteration losses and the parameters it leaves behind (PpoBackUpTime,
+    a wall-clock time, is left out)."""
+    arrays = {"losses": np.array([[l[k] for k in LOSS_KEYS] for l in step_losses], dtype=np.float64)}
+    for name, p in net.named_parameters():
+        arrays["param." + name] = p.detach().float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, "outputs of %d bytes exceed the %d-byte dump budget" % (total, DUMP_LIMIT)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def quick_workload(kind, gemm_mode, dev, dist, world=1, rank=0, rows=None, forward=True):
@@ -627,7 +665,18 @@ def main():
                     help="warm up, then run ONE learn step between cudaProfilerStart/Stop and exit (for ncu --profile-from-start off)")
     ap.add_argument("--profile-forward", dest="profile_forward", action="store_true",
                     help="run ONE Forward tick (wire bytes in, replies out) and one GAE scan between cudaProfilerStart/Stop and exit")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="run in deterministic mode and write the losses and parameters of the last timed learn call as "
+                         "DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the product arm (--impl ours)")
+    if args.dump_outputs and (args.profile_step or args.profile_forward):
+        ap.error("--dump-outputs needs the timed steps, which --profile-step / --profile-forward skip")
+    if args.dump_outputs and args.gemm_mode != "tc3":
+        ap.error("--dump-outputs runs in deterministic mode, which covers the tc3 engine only (--gemm-mode tc3)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.workload == "navlaser3":
         # non-reference variant: the reference has no encoder for it, so there is no CPU arm to put beside it
