@@ -27,6 +27,14 @@ class PPOHparams(C.Structure):
                 ("beta1", C.c_float), ("beta2", C.c_float), ("adam_eps", C.c_float)]
 
 
+class GatherJob(C.Structure):
+    _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("row_bytes", C.c_int64), ("src_stride", C.c_int64),
+                ("dst_stride", C.c_int64), ("src_rows", C.c_int64)]
+
+
+GATHER_MAX_JOBS = 12       # DDRL_GATHER_MAX_JOBS
+
+
 class ConvDesc(C.Structure):
     _fields_ = [(k, C.c_int32) for k in ("B", "H", "W", "Cin", "Cout", "KH", "KW", "stride", "pad")]
 
@@ -78,6 +86,8 @@ SIGNATURES = {
     "ddrl_net_backward": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _I, _P]),
     "ddrl_net_backward_segment": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _I, _I, C.POINTER(_I), _P]),
     "ddrl_net_tensor_segment": (_I, [_P, _I]),
+    "ddrl_net_backward_minibatch": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _P]),
+    "ddrl_gather_rows": (_I, [_P, _I, C.POINTER(GatherJob), _I, _P]),
     "ddrl_set_deterministic": (_I, [_I]),
     "ddrl_peer_allreduce_flag_bytes": (_I, []),
     "ddrl_peer_allreduce_f32": (_I, [C.POINTER(_P), _P, C.POINTER(_P), _I, _I, C.c_int64, C.c_int64, C.c_uint32, _P]),

@@ -184,6 +184,10 @@ struct ddrl_net {
   unsigned long long graph_clock = 0;
   cudaStream_t cap_stream = nullptr;
   bool graphs_off = false;
+  // minibatch passes (ddrl_net_backward_minibatch): a failed capture turns off only these graphs; a key runs on the stream
+  // the first time it is seen (that call performs the one-time allocations a capture must not contain)
+  bool mb_graphs_off = false;
+  std::vector<std::string> mb_seen;
   double* sumsq_dev = nullptr;     // clip+Adam norm scratch of THIS net
   // weight preparation as three dependent multi-job launches (prep.cu): [re-packs + amax-slot zeroing] -> [amax + tf32
   // mirrors] -> [fp16 splits]; and the gradient un-permutation that ends a backward pass as one more
@@ -1056,6 +1060,7 @@ static void graph_entry_destroy(ddrl_net::GraphEntry& e) {
 static void graphs_clear(ddrl_net* n) {
   for (auto& e : n->graphs) graph_entry_destroy(e);
   n->graphs.clear();
+  n->mb_seen.clear();
 }
 // Segment cut of the backward pass (see ddrl_net::Capture): ends segment n->cap.seg.  Inside a capture the gradients of the
 // segment are un-permuted, the current graph is closed and the next one opened; outside it does nothing.
@@ -1088,9 +1093,10 @@ static std::string graph_key(const char* tag, std::initializer_list<const void*>
 }
 // Runs `body(stream)` through a cached graph: the first call with this key captures it on the net's private capture stream
 // (nothing executes during capture; side-stream forks inside `body` become parallel branches), later calls replay.  A
-// failed capture switches graphs off for this net and runs the body on the caller's stream.
+// failed capture sets *off (default: n->graphs_off, all graphs of this net) and runs the body on the caller's stream.
 template <class F>
-static int run_graphed(ddrl_net* n, const std::string& key, cudaStream_t s, F&& body, ddrl_net::GraphEntry** out = nullptr) {
+static int run_graphed(ddrl_net* n, const std::string& key, cudaStream_t s, F&& body, ddrl_net::GraphEntry** out = nullptr,
+                       bool* off = nullptr) {
   ddrl_net::GraphEntry* e = nullptr;
   for (auto& g : n->graphs) if (g.key == key) { e = &g; break; }
   if (!e) {
@@ -1122,7 +1128,7 @@ static int run_graphed(ddrl_net* n, const std::string& key, cudaStream_t s, F&& 
       c = ddrl_net::Capture();
       cudaGetLastError();
       g_launches = l0;
-      n->graphs_off = true;
+      *(off ? off : &n->graphs_off) = true;
       if (out) *out = nullptr;
       return body(s);
     }
@@ -1821,6 +1827,40 @@ extern "C" int ddrl_net_backward_segment(ddrl_net* n, const float* const* obs, i
   if (segment < 0 || !n_segments) return DDRL_E_ARG;
   return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, hp, obs_unchanged, segment, n_segments,
                        (cudaStream_t)stream);
+}
+
+// One minibatch step: new rows at the addresses of an earlier call.  The observations are always restaged (reuse_obs = false),
+// so the pass depends on no staging left by an earlier call; the staged observations it leaves belong to no full-batch call.
+extern "C" int ddrl_net_backward_minibatch(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
+                                           const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                           const ddrl_ppo_hparams* hp, void* stream) {
+  if (!n || !hp || B_local < 0 || B_global < B_local || B_global < 1) return DDRL_E_ARG;
+  if (!n->params || !n->grads) return DDRL_E_STATE;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (B_local == 0) {
+    DDRL_CUDA(cudaMemsetAsync(n->grads, 0, sizeof(float) * (size_t)(n->P + 8), s));
+    if (n->packed_base) DDRL_CUDA(cudaMemsetAsync(n->packed_base + n->packed_grad_off, 0, n->packed_grad_bytes, s));
+    return DDRL_OK;
+  }
+  TRY(check_obs(n, obs, n_obs));
+  if (!actions || !old_logp || !adv || !returns) return DDRL_E_ARG;
+  TRY(ensure_workspace(n, B_local, true));
+  if (n->dirty) TRY(repack(n, s));
+  n->cols_obs0 = nullptr;            // a later ddrl_net_backward(obs_unchanged) restages
+  n->cols_rows = -1;
+  auto body = [&](cudaStream_t cs) {
+    return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, hp, false, cs);
+  };
+  if (B_local > n->MB || !n->extra.empty() || !graphs_enabled(n) || n->mb_graphs_off) return body(s);
+  const std::string key = graph_key("bwd_mb", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, actions,
+                                               old_logp, adv, returns, n->params, n->grads, n->ws.base},
+                                    {B_local, B_global}, hp, sizeof(*hp));
+  if (std::find(n->mb_seen.begin(), n->mb_seen.end(), key) == n->mb_seen.end()) {
+    if (n->mb_seen.size() >= 16) n->mb_seen.erase(n->mb_seen.begin());
+    n->mb_seen.push_back(key);
+    return body(s);
+  }
+  return run_graphed(n, key, s, body, nullptr, &n->mb_graphs_off);
 }
 
 // backward segment after which the gradient of parameter tensor `index` is final in the flat gradient buffer

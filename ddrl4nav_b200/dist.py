@@ -38,6 +38,23 @@ def global_rows(local_rows: int, device, group=None) -> int:
     return int(t.item())
 
 
+def global_chunk_rows(chunk_rows, device, group=None):
+    """Per minibatch k: the sum over ranks of the local chunk-k row counts (the 1/B_global of step k), all M sums from ONE
+    int64 all-reduce.  Raises DDRLError on every rank together when some global chunk is empty."""
+    import torch.distributed as dist
+    from ._lib import DDRLError
+    sums = [int(x) for x in chunk_rows]
+    _, ws = world(group)
+    if ws > 1:
+        t = torch.tensor(sums, dtype=torch.int64, device=device)
+        dist.all_reduce(t, group=group)
+        sums = [int(x) for x in t.tolist()]
+    if any(x < 1 for x in sums):
+        raise DDRLError("minibatch plan has an empty global chunk (rows per chunk over all ranks: %s); lower MINI_BATCH_NUM"
+                        % sums)
+    return sums
+
+
 def allreduce_grads(flat_grads_with_tail: torch.Tensor, n_params: int, group=None) -> None:
     """In-place sum over ranks of grads[0 : P+4] (P parameters + {actor, v, entropy, -} loss sums)."""
     import torch.distributed as dist

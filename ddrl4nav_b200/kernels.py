@@ -219,6 +219,37 @@ def conv_nhwc(op: int, x, w, dy=None, bias=None, stride: int = 1, pad: int = 0, 
     return out
 
 
+def gather_jobs(pairs, n_rows: int):
+    """ddrl_gather_job array for `pairs` [(src, dst), ...]: a row is everything after dim 0 and must be contiguous; dst needs
+    >= n_rows rows of the same size and dtype."""
+    jobs = (_lib.GatherJob * max(len(pairs), 1))()
+    for j, (src, dst) in enumerate(pairs):
+        require_cuda(src, dst)
+        if src.dtype != dst.dtype or src.device != dst.device:
+            raise DDRLError("gather_rows: job %d mixes %s/%s with %s/%s" % (j, src.dtype, src.device, dst.dtype, dst.device))
+        row = src[0].numel() if src.dim() > 1 else 1
+        drow = dst[0].numel() if dst.dim() > 1 else 1
+        contiguous = lambda t: t.dim() <= 1 or t[0:1].is_contiguous()
+        if row != drow or dst.shape[0] < n_rows or not (contiguous(src) and contiguous(dst)):
+            raise DDRLError("gather_rows: job %d has src %s / dst %s (rows must be contiguous and of one size, dst >= %d rows)"
+                            % (j, tuple(src.shape), tuple(dst.shape), n_rows))
+        es = src.element_size()
+        jobs[j] = _lib.GatherJob(src.data_ptr() or None, dst.data_ptr() or None, row * es, src.stride(0) * es,
+                                 dst.stride(0) * es, src.shape[0])
+    return jobs
+
+
+def gather_rows(rows: torch.Tensor, pairs) -> None:
+    """dst[i] = src[rows[i]] for every (src, dst) in `pairs`, i < len(rows), in ONE launch (ddrl_gather_rows).  rows: int32
+    device tensor; indices outside [0, len(src)) are clamped."""
+    require_cuda(rows)
+    if rows.dtype != torch.int32 or not rows.is_contiguous():
+        raise DDRLError("gather_rows: rows must be a contiguous int32 tensor (got %s)" % rows.dtype)
+    n = rows.numel()
+    jobs = gather_jobs(pairs, n)
+    check(_lib.load().ddrl_gather_rows(ptr(rows), n, jobs, len(pairs), current_stream()), "ddrl_gather_rows")
+
+
 def launch_count() -> int:
     return int(_lib.load().ddrl_launch_count())
 

@@ -72,6 +72,18 @@ class PPO(Basenn):
         self.v_loss_theta, self.ent_loss_theta = self.hp.v_coef, self.hp.ent_coef
         self.ppo_clip, self.duel_ppo_clip = self.hp.ppo_clip, self.hp.dual_clip
         self.training_iter_time = _cfg(config_nn, "TRAINING_ITER_TIME", 10)
+        # minibatch epochs (non-reference option): every epoch shuffles the batch and takes one optimiser step per chunk
+        self.mini_batch_num = _cfg(config_nn, "MINI_BATCH_NUM", 1)
+        if isinstance(self.mini_batch_num, bool) or not isinstance(self.mini_batch_num, (int, np.integer)) or self.mini_batch_num < 1:
+            raise DDRLError("MINI_BATCH_NUM must be an integer >= 1 (got %r)" % (self.mini_batch_num,))
+        self.mini_batch_num = int(self.mini_batch_num)
+        seed = _cfg(config_nn, "MINI_BATCH_SEED", None)
+        if seed is not None and (isinstance(seed, bool) or not isinstance(seed, (int, np.integer))):
+            raise DDRLError("MINI_BATCH_SEED must be an integer or None (got %r)" % (seed,))
+        self._mb_seed = None if seed is None else int(seed)
+        self._mb_gen = None             # torch.Generator on the net's device (the minibatch shuffles)
+        self._mb = None                 # persistent minibatch buffers (_minibatch_buffers)
+        self.last_minibatch_perms = []  # per epoch of the last minibatch learn call: int32 device permutation of the rows
         self.gemm_mode = os.environ.get("DDRL_GEMM_MODE", _cfg(config_nn, "GEMM_MODE", "tc3"))
         self.update_time = 0
         self._adam_step = 0
@@ -277,7 +289,7 @@ class PPO(Basenn):
     def named_grads(self):
         return {n: self._grads[o:o + p.numel()].view(p.shape) for (n, p), o in zip(self.named_parameters(), self._offsets)}
 
-    def _obs_ptrs(self, states):
+    def _obs_ptrs(self, states, allow_empty=False):
         lib = _lib.load()
         n_obs = lib.ddrl_net_num_obs(self._h)
         if len(states) < n_obs:
@@ -292,7 +304,7 @@ class PPO(Basenn):
             per = lib.ddrl_net_obs_elems(self._h, i)
             if B is None:
                 B = t.shape[0]
-            if t.shape[0] != B or (t.numel() // max(B, 1)) != per:
+            if t.shape[0] != B or ((B or not allow_empty) and (t.numel() // max(B, 1)) != per):
                 raise DDRLError("state slot %d has shape %s; expected [B=%d, %d elements/sample]" % (i, tuple(t.shape), B, per))
             keep.append(t)
         arr = (C.c_void_p * n_obs)(*[t.data_ptr() for t in keep])
@@ -426,9 +438,9 @@ class PPO(Basenn):
         dist.broadcast_params(self._flat, src=src, group=self._dp_group)
         self._weights_changed()
 
-    def _bwd_args(self, states, advs, actions, old_logps, returns, b_global, obs_unchanged):
+    def _bwd_args(self, states, advs, actions, old_logps, returns, b_global, obs_unchanged, allow_empty=False):
         """Device-side argument list shared by ddrl_net_backward / ddrl_net_backward_segment (+ the tensors it points into)."""
-        keep, arr, n_obs, B = self._obs_ptrs(states)
+        keep, arr, n_obs, B = self._obs_ptrs(states, allow_empty)
         dev = self._flat.device
         f = lambda t: t.to(device=dev, dtype=torch.float32).contiguous()
         advs, actions, old_logps, returns = f(advs), f(actions), f(old_logps), f(returns)
@@ -447,23 +459,28 @@ class PPO(Basenn):
         return args, (keep, advs, actions, old_logps, returns, rows), B
 
     @_on_device
-    def backward_only(self, states, advs, actions, old_logps, returns, b_global=None, obs_unchanged=False):
-        """forward + fused loss + backward for the local rows; grads (scaled 1/B_global) stay in flat_grads()."""
+    def backward_only(self, states, advs, actions, old_logps, returns, b_global=None, obs_unchanged=False, minibatch=False):
+        """forward + fused loss + backward for the local rows; grads (scaled 1/B_global) stay in flat_grads().
+        minibatch: the inputs are the persistent minibatch buffers (ddrl_net_backward_minibatch; 0 rows allowed)."""
         self._ensure_engine()
         lib = _lib.load()
-        args, held, B = self._bwd_args(states, advs, actions, old_logps, returns, b_global, obs_unchanged)
+        args, held, B = self._bwd_args(states, advs, actions, old_logps, returns, b_global, obs_unchanged, minibatch)
         keep, rows = held[0], held[-1]
         dev = self._flat.device
         V = len(self._critics)
-        check(lib.ddrl_net_backward(*args, current_stream()), "ddrl_net_backward")
+        if minibatch:
+            check(lib.ddrl_net_backward_minibatch(*args[:-1], current_stream()), "ddrl_net_backward_minibatch")
+        else:
+            check(lib.ddrl_net_backward(*args, current_stream()), "ddrl_net_backward")
         if V > 1 and self.prenet is not None:
             self._extra_grads_to_params()
         if V > 1 and self.prenet is None and self.gail_critic:
             # unshared: gailv_loss.backward() only reaches the extra critic's own tower (ppo.py:101-104,122-123)
             k = V - 2
             aux = self._aux_net(k)
-            zeros = torch.zeros(B, dtype=torch.float32, device=dev)
-            aux.backward_only(keep, zeros, zeros, zeros, rows[-1].contiguous(), b_global, obs_unchanged)
+            # (a minibatch pass keeps its inputs at fixed addresses: the persistent zeros of the minibatch buffers)
+            zeros = self._mb["zeros"][:B] if minibatch else torch.zeros(B, dtype=torch.float32, device=dev)
+            aux.backward_only(keep, zeros, zeros, zeros, rows[-1].contiguous(), b_global, obs_unchanged, minibatch)
             if self._dp_world > 1:
                 dist.allreduce_grads(aux._grads, aux._P, self._dp_group)      # its loss sum rides in the tail, as ours does
             for n, g in aux.named_grads().items():
@@ -550,7 +567,12 @@ class PPO(Basenn):
     def learn(self, data):
         """Generator with the reference's contract (nn/ppo.py:77-142): TRAINING_ITER_TIME full-batch iterations
         over `data` (an Experience whose tensors are on the device), yielding
-        ({PpoTotalLoss, ActorLoss, VLoss, EntLoss, PpoBackUpTime}, update_time, True) per iteration."""
+        ({PpoTotalLoss, ActorLoss, VLoss, EntLoss, PpoBackUpTime}, update_time, True) per iteration.
+        MINI_BATCH_NUM = M > 1: TRAINING_ITER_TIME shuffled epochs of M minibatches, one optimiser step and one yield
+        per minibatch (_learn_minibatch)."""
+        if self.mini_batch_num > 1:
+            yield from self._learn_minibatch(data)
+            return
         b_local = len(data.states[0])
         b_global = b_local
         if self._dp_world > 1:
@@ -568,6 +590,92 @@ class PPO(Basenn):
             loss_log = {"PpoTotalLoss": loss4[0], "ActorLoss": loss4[1], "VLoss": loss4[2], "EntLoss": loss4[3],
                         "PpoBackUpTime": time.time() - start_time}
             yield loss_log, self.update_time, True
+
+    # ------------------------------------------------------------------ minibatch epochs (non-reference option)
+    @staticmethod
+    def minibatch_plan(b_local, m):
+        """[lo, hi) of each of the m chunks of one shuffled epoch (positions in the permutation); sizes differ by <= 1."""
+        return [dist.shard_rows(b_local, k, m) for k in range(m)]
+
+    def _minibatch_sources(self, data):
+        """fp32 contiguous device tensors the minibatch rows are gathered from: state slots, actions, old log-probs,
+        advantages, and the return rows [V, B]."""
+        dev = self._flat.device
+        f = lambda t: (t if torch.is_tensor(t) else torch.as_tensor(np.asarray(t))).to(device=dev, dtype=torch.float32).contiguous()
+        n_obs = _lib.load().ddrl_net_num_obs(self._h)
+        if len(data.states) < n_obs:
+            raise DDRLError("expected %d state slots, got %d" % (n_obs, len(data.states)))
+        values = f(data.values)
+        values = values if values.dim() == 2 else values.view(1, -1)
+        src = dict(states=[f(data.states[i]) for i in range(n_obs)], actions=f(data.actions), old_logps=f(data.old_logps),
+                   advs=f(data.advs), values=values)
+        if len(src["states"]) + 3 + values.shape[0] > _lib.GATHER_MAX_JOBS:
+            raise DDRLError("minibatch gather: %d return rows exceed the job limit" % values.shape[0])
+        return src
+
+    def _minibatch_buffers(self, src, b_local, mb_rows):
+        """Persistent buffers of the largest chunk (smaller chunks use the leading rows).  They keep their addresses while
+        b_local, M and the shapes stay the same, which is what lets ddrl_net_backward_minibatch replay its graph."""
+        dev = self._flat.device
+        key = (b_local, self.mini_batch_num, dev, tuple(tuple(t.shape[1:]) for t in src["states"]), tuple(src["actions"].shape[1:]),
+               src["values"].shape[0])
+        if self._mb is None or self._mb["key"] != key:
+            rows = max(mb_rows, 1)
+            e = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
+            self._mb = dict(key=key, states=[e(rows, *t.shape[1:]) for t in src["states"]],
+                            actions=e(rows, *src["actions"].shape[1:]), old_logps=e(rows), advs=e(rows),
+                            values=e(src["values"].shape[0] * rows), zeros=torch.zeros(rows, dtype=torch.float32, device=dev))
+        return self._mb
+
+    @_on_device
+    def _gather_minibatch(self, src, rows):
+        """Gathers the rows `rows` (int32 device) of every source into the minibatch buffers in ONE launch; returns the
+        (states, advs, actions, old_logps, returns [V, n]) views backward_only takes."""
+        mb, n = self._mb, rows.numel()
+        V = src["values"].shape[0]
+        ret = mb["values"][:V * n]
+        if n:
+            pairs = [(s, d) for s, d in zip(src["states"], mb["states"])]
+            pairs += [(src["actions"], mb["actions"]), (src["old_logps"], mb["old_logps"]), (src["advs"], mb["advs"])]
+            pairs += [(src["values"][v], ret[v * n:(v + 1) * n]) for v in range(V)]
+            kernels.gather_rows(rows, pairs)
+        return [t[:n] for t in mb["states"]], mb["advs"][:n], mb["actions"][:n], mb["old_logps"][:n], ret.view(V, n)
+
+    def _learn_minibatch(self, data):
+        """TRAINING_ITER_TIME epochs; each draws a permutation of the local rows (net-owned generator) and cuts it into
+        M chunks; per chunk: gather, backward, all-reduce (data-parallel), clip+Adam, yield.  Data-parallel: global
+        minibatch k is chunk k of every rank; its B_global is the sum of the ranks' chunk-k sizes."""
+        m = self.mini_batch_num
+        b_local = len(data.states[0])
+        if self._dp_world == 1 and m > b_local:
+            raise DDRLError("MINI_BATCH_NUM=%d exceeds the %d rows of the batch" % (m, b_local))
+        self._ensure_engine()
+        dev = self._flat.device
+        plan = self.minibatch_plan(b_local, m)
+        sizes = [hi - lo for lo, hi in plan]
+        b_globals = dist.global_chunk_rows(sizes, dev, self._dp_group) if self._dp_world > 1 else sizes
+        src = self._minibatch_sources(data)
+        self._minibatch_buffers(src, b_local, max(sizes))
+        if self._mb_gen is None or self._mb_gen.device != dev:
+            if self._mb_seed is None:           # MINI_BATCH_SEED=None: drawn once from torch's default generator
+                self._mb_seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+            self._mb_gen = torch.Generator(device=dev)
+            self._mb_gen.manual_seed(self._mb_seed)
+        self.last_minibatch_perms = []
+        for _ in range(self.training_iter_time):
+            perm = torch.randperm(b_local, generator=self._mb_gen, device=dev, dtype=torch.int32)
+            self.last_minibatch_perms.append(perm)
+            for (lo, hi), b_global in zip(plan, b_globals):
+                start_time = time.time()
+                states, advs, actions, old_logps, returns = self._gather_minibatch(src, perm[lo:hi])
+                self.backward_only(states, advs, actions, old_logps, returns, b_global, minibatch=True)
+                if self._dp_world > 1:
+                    self._allreduce_grads()
+                loss4 = self.optimizer_step().tolist()
+                self.update_time += 1
+                loss_log = {"PpoTotalLoss": loss4[0], "ActorLoss": loss4[1], "VLoss": loss4[2], "EntLoss": loss4[3],
+                            "PpoBackUpTime": time.time() - start_time}
+                yield loss_log, self.update_time, True
 
     def add_critic(self, critic):
         """nn/ppo.py:63-64.  The extra critic's values come back from forward()/act() as further rows; its value loss joins

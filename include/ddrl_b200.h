@@ -287,6 +287,28 @@ int ddrl_net_tensor_segment(const ddrl_net* net, int index);
 int ddrl_peer_allreduce_flag_bytes(void);
 int ddrl_peer_allreduce_f32(float* const* peer_bufs, float* multicast_buf, void* const* peer_flags, int rank, int world,
                             int64_t offset, int64_t count, uint32_t seq, void* stream);
+/* Multi-tensor row gather (minibatch PPO epochs, nn/ppo.py learn with MINI_BATCH_NUM > 1): for every job, dst row i =
+ * src row rows[i] (i < n_rows), all jobs in ONE launch.  Strides and row_bytes are in bytes; row_bytes, strides and
+ * pointers must be multiples of 4 (16 everywhere selects 16-byte accesses).  Indices outside [0, src_rows) are clamped.
+ * rows: device int32 [n_rows].  jobs: HOST array of n_jobs (1..DDRL_GATHER_MAX_JOBS) descriptors, passed to the kernel by
+ * value (no host->device copy; the launch can be captured in a CUDA graph). */
+#define DDRL_GATHER_MAX_JOBS 12
+typedef struct {
+  const void* src;
+  void* dst;
+  int64_t row_bytes;
+  int64_t src_stride;
+  int64_t dst_stride;
+  int64_t src_rows;
+} ddrl_gather_job;
+int ddrl_gather_rows(const int32_t* rows, int n_rows, const ddrl_gather_job* jobs, int n_jobs, void* stream);
+/* ddrl_net_backward for one minibatch of a minibatch epoch: the inputs sit at the same addresses as in an earlier call of
+ * this entry point and hold NEW rows.  The pass always restages the observations.  From the second call with the same
+ * arguments on, it replays a CUDA graph captured for them (micro-batched rows, extra critics and DDRL_NO_GRAPH=1 run on the
+ * stream).  A failed capture here leaves the graphs of ddrl_net_backward / ddrl_net_clip_adam on. */
+int ddrl_net_backward_minibatch(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
+                                const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                const ddrl_ppo_hparams* hp, void* stream);
 /* second half (nn/ppo.py:115-129): global-norm clip + the two (or one) Adam steps; then refreshes
  * the packed weights.  loss4_out (device, 4 floats, optional) = {total, actor, v, entropy}. */
 int ddrl_net_clip_adam(ddrl_net* net, int step, const ddrl_ppo_hparams* hp, float* loss4_out, void* stream);
