@@ -24,7 +24,8 @@ class PPOHparams(C.Structure):
     _fields_ = [("ppo_clip", C.c_float), ("dual_clip", C.c_float), ("v_coef", C.c_float), ("ent_coef", C.c_float),
                 ("max_grad_norm", C.c_float), ("clip_grad", C.c_int32), ("smooth_l1", C.c_int32),
                 ("lr", C.c_float), ("lr_actor", C.c_float), ("lr_critic", C.c_float),
-                ("beta1", C.c_float), ("beta2", C.c_float), ("adam_eps", C.c_float)]
+                ("beta1", C.c_float), ("beta2", C.c_float), ("adam_eps", C.c_float),
+                ("value_clip", C.c_float), ("ppo_stats", C.c_int32)]
 
 
 class GatherJob(C.Structure):
@@ -67,6 +68,12 @@ SIGNATURES = {
     "ddrl_gaussian_head": (_I, [_P, _I, _P, _P, _I, _I, _P, _P, _P]),
     "ddrl_ppo_loss_categorical": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P]),
     "ddrl_ppo_loss_gaussian": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P, _P]),
+"ddrl_ppo_loss_categorical_v": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P, _P,
+                                        _P]),
+    "ddrl_ppo_loss_gaussian_v": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P, _P,
+                                     _P, _P]),
+    "ddrl_adv_moments": (_I, [_P, _I, _P, _P]),
+    "ddrl_adv_normalize": (_I, [_P, _I, _P, _F, _P, _P]),
     "ddrl_value_loss": (_I, [_P, _P, _I, _F, C.POINTER(PPOHparams), _I, _P, _P, _P]),
     "ddrl_clip_adam": (_I, [_P, _P, _P, _P, _L, C.POINTER(_L), C.POINTER(_F), _I, _I, C.POINTER(PPOHparams), _P, _P]),
     "ddrl_gemm_f32": (_I, [_I, _I, _I, _I, _I, _P, _I, _P, _I, _P, _I, _P, _I, _I, _P]),
@@ -84,9 +91,11 @@ SIGNATURES = {
     "ddrl_net_forward": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P, _P, _P, _P]),
     "ddrl_net_encode": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P]),
     "ddrl_net_backward": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _I, _P]),
+    "ddrl_net_backward_v": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, _P, C.POINTER(PPOHparams), _I, _P]),
     "ddrl_net_backward_segment": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _I, _I, C.POINTER(_I), _P]),
     "ddrl_net_tensor_segment": (_I, [_P, _I]),
     "ddrl_net_backward_minibatch": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _P]),
+    "ddrl_net_backward_minibatch_v": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, _P, C.POINTER(PPOHparams), _P]),
     "ddrl_gather_rows": (_I, [_P, _I, C.POINTER(GatherJob), _I, _P]),
     "ddrl_set_deterministic": (_I, [_I]),
     "ddrl_peer_allreduce_flag_bytes": (_I, []),

@@ -1077,6 +1077,10 @@ static int seg_cut(ddrl_net* n, cudaStream_t s) {
   if (cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal) != cudaSuccess) { c.failed = true; return DDRL_E_CUDA; }
   return DDRL_OK;
 }
+// the value clip needs the rollout's values of critic 0, and old values without a clip width would be ignored
+static bool value_clip_ok(const ddrl_ppo_hparams* hp, const float* old_values) {
+  return old_values ? hp->value_clip > 0.f : !(hp->value_clip > 0.f);
+}
 static bool graphs_enabled(ddrl_net* n) {
   const char* e = getenv("DDRL_NO_GRAPH");
   return !(e && e[0] == '1') && !n->graphs_off && !g_prof_on;
@@ -1707,14 +1711,15 @@ namespace ddrl {
 // zero the gradients, then per micro-batch: forward (act = data.actions), fused loss, heads and encoders backward; finally
 // the packed weight gradients are un-permuted into the reference layout
 static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int B_global, const float* actions,
-                         const float* old_logp, const float* adv, const float* returns, const ddrl_ppo_hparams* hp, bool reuse_obs,
-                         cudaStream_t s) {
+                         const float* old_logp, const float* adv, const float* returns, const float* old_values,
+                         const ddrl_ppo_hparams* hp, bool reuse_obs, cudaStream_t s) {
   // zero the flat grads (+ loss tail) and the packed grads: everything below accumulates
   DDRL_CUDA(cudaMemsetAsync(n->grads, 0, sizeof(float) * (size_t)(n->P + 8), s));
   if (n->packed_base) DDRL_CUDA(cudaMemsetAsync(n->packed_base + n->packed_grad_off, 0, n->packed_grad_bytes, s));
   const int A = n->d.act_dim, F = n->d.feat;
   const float invB = 1.0f / (float)B_global;
   float* loss_sums = n->grads + n->P;
+  float* stats = hp->ppo_stats ? loss_sums + 3 : nullptr;      // {approx KL, clip fraction} sums in tail slots 3 and 4
   Tower& ta = n->towers[0];
   Tower& tc = n->towers[n->d.shared ? 0 : 1];
   float* aw = n->params + n->T[n->t_aw].offset;
@@ -1725,12 +1730,14 @@ static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int 
     amax_new_pass(n, s, reuse_obs);
     TRY(forward_chunk(n, obs, r0, mb, true, s, reuse_obs));
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
-      TRY(ddrl_ppo_loss_categorical(n->logits, n->ldA, actions + r0, old_logp + r0, adv + r0, returns + r0, n->vout, mb, A,
-                                    invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums, s));
+      TRY(ddrl_ppo_loss_categorical_v(n->logits, n->ldA, actions + r0, old_logp + r0, adv + r0, returns + r0, n->vout, mb, A,
+                                      invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
+                                      old_values ? old_values + r0 : nullptr, stats, s));
     } else {
-      TRY(ddrl_ppo_loss_gaussian(n->logits, n->ldA, n->params + n->T[n->t_logstd].offset, actions + r0 * A, old_logp + r0,
-                                 adv + r0, returns + r0, n->vout, mb, A, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv,
-                                 n->grads + n->T[n->t_logstd].offset, loss_sums, s));
+      TRY(ddrl_ppo_loss_gaussian_v(n->logits, n->ldA, n->params + n->T[n->t_logstd].offset, actions + r0 * A, old_logp + r0,
+                                   adv + r0, returns + r0, n->vout, mb, A, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv,
+                                   n->grads + n->T[n->t_logstd].offset, loss_sums, old_values ? old_values + r0 : nullptr, stats,
+                                   s));
     }
     // heads backward (nn/actor.py:91 actor_linear, nn/critic.py:21 critic_linear)
     TRY(skinny_wgrad(n->dlogits, n->ldA, ta.h, F, mb, A, F, n->grads + n->T[n->t_aw].offset, n->grads + n->T[n->t_ab].offset, s));
@@ -1761,9 +1768,10 @@ static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int 
 // seg < 0: the whole pass.  seg >= 0: segment `seg` only (seg 0 validates, prepares and -- when the pass is not replayable as
 // a graph chain -- runs everything and reports one segment).
 static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global, const float* actions,
-                         const float* old_logp, const float* adv, const float* returns, const ddrl_ppo_hparams* hp,
-                         int obs_unchanged, int seg, int* nseg_out, cudaStream_t s) {
+                         const float* old_logp, const float* adv, const float* returns, const float* old_values,
+                         const ddrl_ppo_hparams* hp, int obs_unchanged, int seg, int* nseg_out, cudaStream_t s) {
   if (!n || !hp || B_local < 0 || B_global < B_local || B_global < 1) return DDRL_E_ARG;
+  if (B_local > 0 && !value_clip_ok(hp, old_values)) return DDRL_E_ARG;
   if (!n->params || !n->grads) return DDRL_E_STATE;
   if (nseg_out) *nseg_out = 1;
   if (B_local == 0) {
@@ -1775,7 +1783,7 @@ static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_
   TRY(check_obs(n, obs, n_obs));
   if (!actions || !old_logp || !adv || !returns) return DDRL_E_ARG;
   const std::string key = graph_key("bwd", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, actions, old_logp,
-                                            adv, returns, n->params, n->grads, n->ws.base},
+                                            adv, returns, old_values, n->params, n->grads, n->ws.base},
                                     {B_local, B_global}, hp, sizeof(*hp));
   auto launch_seg = [&](ddrl_net::GraphEntry* e, int k) {
     const int pre = (int)e->pre_execs.size();
@@ -1804,20 +1812,27 @@ static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_
   if (reuse_obs && n->extra.empty() && graphs_enabled(n)) {
     ddrl_net::GraphEntry* e = nullptr;
     TRY(run_graphed(n, key, s, [&](cudaStream_t cs) {
-      return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, hp, true, cs);
+      return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, hp, true, cs);
     }, seg < 0 ? nullptr : &e));
     if (seg < 0 || !e) return DDRL_OK;             // launched whole / capture failed: the body already ran on the stream
     if (nseg_out) *nseg_out = (int)e->pre_execs.size() + 1;
     return launch_seg(e, 0);
   }
-  return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, hp, reuse_obs, s);
+  return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, hp, reuse_obs, s);
 }
 
 extern "C" int ddrl_net_backward(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
                                  const float* actions, const float* old_logp, const float* adv, const float* returns,
                                  const ddrl_ppo_hparams* hp, int obs_unchanged, void* stream) {
-  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, hp, obs_unchanged, -1, nullptr,
+  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, nullptr, hp, obs_unchanged, -1, nullptr,
                        (cudaStream_t)stream);
+}
+
+extern "C" int ddrl_net_backward_v(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
+                                   const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                   const float* old_values, const ddrl_ppo_hparams* hp, int obs_unchanged, void* stream) {
+  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, old_values, hp, obs_unchanged, -1,
+                       nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int ddrl_net_backward_segment(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
@@ -1825,16 +1840,17 @@ extern "C" int ddrl_net_backward_segment(ddrl_net* n, const float* const* obs, i
                                          const ddrl_ppo_hparams* hp, int obs_unchanged, int segment, int* n_segments,
                                          void* stream) {
   if (segment < 0 || !n_segments) return DDRL_E_ARG;
-  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, hp, obs_unchanged, segment, n_segments,
-                       (cudaStream_t)stream);
+  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, nullptr, hp, obs_unchanged, segment,
+                       n_segments, (cudaStream_t)stream);
 }
 
 // One minibatch step: new rows at the addresses of an earlier call.  The observations are always restaged (reuse_obs = false),
 // so the pass depends on no staging left by an earlier call; the staged observations it leaves belong to no full-batch call.
-extern "C" int ddrl_net_backward_minibatch(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
-                                           const float* actions, const float* old_logp, const float* adv, const float* returns,
-                                           const ddrl_ppo_hparams* hp, void* stream) {
+extern "C" int ddrl_net_backward_minibatch_v(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
+                                             const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                             const float* old_values, const ddrl_ppo_hparams* hp, void* stream) {
   if (!n || !hp || B_local < 0 || B_global < B_local || B_global < 1) return DDRL_E_ARG;
+  if (B_local > 0 && !value_clip_ok(hp, old_values)) return DDRL_E_ARG;
   if (!n->params || !n->grads) return DDRL_E_STATE;
   cudaStream_t s = (cudaStream_t)stream;
   if (B_local == 0) {
@@ -1849,11 +1865,11 @@ extern "C" int ddrl_net_backward_minibatch(ddrl_net* n, const float* const* obs,
   n->cols_obs0 = nullptr;            // a later ddrl_net_backward(obs_unchanged) restages
   n->cols_rows = -1;
   auto body = [&](cudaStream_t cs) {
-    return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, hp, false, cs);
+    return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, hp, false, cs);
   };
   if (B_local > n->MB || !n->extra.empty() || !graphs_enabled(n) || n->mb_graphs_off) return body(s);
   const std::string key = graph_key("bwd_mb", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, actions,
-                                               old_logp, adv, returns, n->params, n->grads, n->ws.base},
+                                               old_logp, adv, returns, old_values, n->params, n->grads, n->ws.base},
                                     {B_local, B_global}, hp, sizeof(*hp));
   if (std::find(n->mb_seen.begin(), n->mb_seen.end(), key) == n->mb_seen.end()) {
     if (n->mb_seen.size() >= 16) n->mb_seen.erase(n->mb_seen.begin());
@@ -1861,6 +1877,12 @@ extern "C" int ddrl_net_backward_minibatch(ddrl_net* n, const float* const* obs,
     return body(s);
   }
   return run_graphed(n, key, s, body, nullptr, &n->mb_graphs_off);
+}
+
+extern "C" int ddrl_net_backward_minibatch(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
+                                           const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                           const ddrl_ppo_hparams* hp, void* stream) {
+  return ddrl_net_backward_minibatch_v(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, nullptr, hp, stream);
 }
 
 // backward segment after which the gradient of parameter tensor `index` is final in the flat gradient buffer
@@ -1884,17 +1906,19 @@ extern "C" int ddrl_net_debug_buffer(ddrl_net* n, int tower, int idx, float* out
 }
 
 namespace ddrl {
-__global__ void finish_losses_kernel(const float* __restrict__ sums, float v_coef, float ent_coef, float* __restrict__ out) {
+__global__ void finish_losses_kernel(const float* __restrict__ sums, float v_coef, float ent_coef, int stats,
+                                     float* __restrict__ out) {
   const float a = sums[0], v = sums[1], e = sums[2];
   out[0] = a + v * v_coef - e * ent_coef;      // nn/ppo.py:108
   out[1] = a; out[2] = v; out[3] = e;
+  if (stats) { out[4] = sums[3]; out[5] = sums[4]; }
 }
 }  // namespace ddrl
 
 namespace ddrl {
 static int clip_adam_body(ddrl_net* n, int step, const ddrl_ppo_hparams* hp, float* loss4_out, cudaStream_t s) {
   if (loss4_out) {
-    finish_losses_kernel<<<1, 1, 0, s>>>(n->grads + n->P, hp->v_coef, hp->ent_coef, loss4_out);
+    finish_losses_kernel<<<1, 1, 0, s>>>(n->grads + n->P, hp->v_coef, hp->ent_coef, hp->ppo_stats, loss4_out);
     DDRL_LAUNCHED("finish_losses_kernel");
   }
   long long sb[3] = {n->seg_begin[0], n->seg_begin[1], n->seg_begin[2]};

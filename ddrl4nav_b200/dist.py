@@ -55,12 +55,23 @@ def global_chunk_rows(chunk_rows, device, group=None):
     return sums
 
 
-def allreduce_grads(flat_grads_with_tail: torch.Tensor, n_params: int, group=None) -> None:
-    """In-place sum over ranks of grads[0 : P+4] (P parameters + {actor, v, entropy, -} loss sums)."""
+def allreduce_grads(flat_grads_with_tail: torch.Tensor, n_params: int, group=None, tail: int = 4) -> None:
+    """In-place sum over ranks of grads[0 : P+tail]: P parameters + the loss sums {actor, v, entropy, -} (tail 4), or
+    {actor, v, entropy, approx KL, clip fraction} (tail 5, PPO_STATS)."""
     import torch.distributed as dist
     _, ws = world(group)
     if ws > 1:
-        dist.all_reduce(flat_grads_with_tail[:n_params + 4], group=group)
+        dist.all_reduce(flat_grads_with_tail[:n_params + tail], group=group)
+
+
+def global_moments(m3: torch.Tensor, group=None) -> torch.Tensor:
+    """In-place sum over ranks of the float64 advantage moments {n, sum a, sum a^2} (kernels.adv_moments): afterwards every
+    rank normalises its rows with the statistics of the global minibatch (NORM_ADV)."""
+    import torch.distributed as dist
+    _, ws = world(group)
+    if ws > 1:
+        dist.all_reduce(m3, group=group)
+    return m3
 
 
 def broadcast_params(flat_params: torch.Tensor, src: int = 0, group=None) -> None:

@@ -10,10 +10,11 @@ from ._lib import DDRLError, PPOHparams, check, current_stream, ptr, require_cud
 
 def make_hparams(ppo_clip=0.2, dual_clip=3.0, v_coef=1.0, ent_coef=0.05, max_grad_norm=0.5, clip_grad=True,
                  smooth_l1=False, lr=2e-4, lr_actor=5e-5, lr_critic=1e-3, beta1=0.9, beta2=0.999,
-                 adam_eps=1e-8) -> PPOHparams:
-    """Defaults = USTC_lab/config/config_nn.py:27-57 and torch.optim.Adam's."""
+                 adam_eps=1e-8, value_clip=0.0, ppo_stats=False) -> PPOHparams:
+    """Defaults = USTC_lab/config/config_nn.py:27-57 and torch.optim.Adam's; value_clip / ppo_stats are the non-reference
+    VALUE_CLIP / PPO_STATS options (0 = off)."""
     return PPOHparams(ppo_clip, dual_clip, v_coef, ent_coef, max_grad_norm, int(bool(clip_grad)), int(bool(smooth_l1)),
-                      lr, lr_actor, lr_critic, beta1, beta2, adam_eps)
+                      lr, lr_actor, lr_critic, beta1, beta2, adam_eps, value_clip, int(bool(ppo_stats)))
 
 
 def _f32c(t: torch.Tensor) -> torch.Tensor:
@@ -248,6 +249,35 @@ def gather_rows(rows: torch.Tensor, pairs) -> None:
     n = rows.numel()
     jobs = gather_jobs(pairs, n)
     check(_lib.load().ddrl_gather_rows(ptr(rows), n, jobs, len(pairs), current_stream()), "ddrl_gather_rows")
+
+
+def adv_moments(adv: torch.Tensor, m3: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """{n, sum a, sum a^2} of the fp32 vector `adv` in float64 (ddrl_adv_moments), into `m3` [3] when given."""
+    adv = _f32c(adv)
+    if m3 is None:
+        m3 = torch.empty(3, dtype=torch.float64, device=adv.device)
+    if m3.dtype != torch.float64 or m3.numel() != 3 or not m3.is_contiguous() or m3.device != adv.device:
+        raise DDRLError("adv_moments: m3 must be a contiguous float64 [3] tensor on %s" % adv.device)
+    check(_lib.load().ddrl_adv_moments(ptr(adv), adv.numel(), ptr(m3), current_stream()), "ddrl_adv_moments")
+    return m3
+
+
+def adv_normalize(adv: torch.Tensor, m3: Optional[torch.Tensor] = None, eps: float = 1e-8,
+                  out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """(adv - mean) / (std + eps), std unbiased, over the moments `m3` (adv_moments, possibly summed over ranks) or over adv
+    itself when m3 is None (ddrl_adv_normalize, one launch).  out may be adv (in place)."""
+    require_cuda(adv)
+    if adv.dtype != torch.float32 or not adv.is_contiguous():
+        raise DDRLError("adv_normalize: adv must be a contiguous fp32 tensor")
+    if out is None:
+        out = torch.empty_like(adv)
+    if out.dtype != torch.float32 or not out.is_contiguous() or out.numel() != adv.numel() or out.device != adv.device:
+        raise DDRLError("adv_normalize: out must be a contiguous fp32 tensor shaped like adv")
+    if m3 is not None and (m3.dtype != torch.float64 or m3.numel() != 3 or m3.device != adv.device):
+        raise DDRLError("adv_normalize: m3 must be a float64 [3] tensor on %s" % adv.device)
+    check(_lib.load().ddrl_adv_normalize(ptr(adv), adv.numel(), ptr(m3), float(eps), ptr(out), current_stream()),
+          "ddrl_adv_normalize")
+    return out
 
 
 def launch_count() -> int:

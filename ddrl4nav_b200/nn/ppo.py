@@ -16,6 +16,7 @@ clip+Adam kernel walks it once.  No autograd graph is ever built.
 """
 import ctypes as C
 import functools
+import math
 import os
 import time
 
@@ -46,6 +47,22 @@ def _cfg(obj, name, default):
     return getattr(obj, name, default) if obj is not None else default
 
 
+def _flag_option(config_nn, name):
+    v = _cfg(config_nn, name, False)
+    if not isinstance(v, (bool, np.bool_)):
+        raise DDRLError("%s must be True or False (got %r)" % (name, v))
+    return bool(v)
+
+
+def _positive_option(config_nn, name):
+    v = _cfg(config_nn, name, None)
+    if v is None:
+        return None
+    if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)) or not math.isfinite(v) or v <= 0:
+        raise DDRLError("%s must be a finite number > 0 or None (got %r)" % (name, v))
+    return float(v)
+
+
 class PPO(Basenn):
     def __init__(self, actor, critic, prenet=None, rnd=None, config=None, config_nn=None):
         super().__init__(config, config_nn)
@@ -61,12 +78,19 @@ class PPO(Basenn):
         self.share_cnn_net = _cfg(config_nn, "SHARE_CNN_NET", prenet is not None)
         if bool(self.share_cnn_net) != (prenet is not None):
             raise DDRLError("SHARE_CNN_NET=%s but prenet is %s" % (self.share_cnn_net, type(prenet).__name__))
+        # PPO training options (non-reference, all off by default): per-step advantage normalisation, clipped value loss of
+        # critic 0, approx-KL / clip-fraction statistics, and a KL target that ends the learn call (it implies the statistics)
+        self.norm_adv = _flag_option(config_nn, "NORM_ADV")
+        self.value_clip = _positive_option(config_nn, "VALUE_CLIP")
+        self.target_kl = _positive_option(config_nn, "TARGET_KL")
+        self.ppo_stats = _flag_option(config_nn, "PPO_STATS") or self.target_kl is not None
         self.hp = kernels.make_hparams(
             ppo_clip=_cfg(config_nn, "PPO_CLIP", 0.2), dual_clip=_cfg(config_nn, "DUEL_PPO_CLIP", 3),
             v_coef=_cfg(config_nn, "V_LOSS_THETA", 1.0), ent_coef=_cfg(config_nn, "ENTROPY_LOSS_THETA", 0.05),
             max_grad_norm=_cfg(config_nn, "CLIP_GRID_NUM", 0.5), clip_grad=_cfg(config_nn, "CLIP_GRID", True),
             smooth_l1=_cfg(config_nn, "SMOOTH_L1_LOSS", False), lr=_cfg(config_nn, "LEARNING_RATE", 2e-4),
-            lr_actor=_cfg(config_nn, "ACTOR_LEARNING_RATE", 5e-5), lr_critic=_cfg(config_nn, "CRITIC_LEARNING_RATE", 1e-3))
+            lr_actor=_cfg(config_nn, "ACTOR_LEARNING_RATE", 5e-5), lr_critic=_cfg(config_nn, "CRITIC_LEARNING_RATE", 1e-3),
+            value_clip=self.value_clip or 0.0, ppo_stats=self.ppo_stats)
         self.clip_grad = bool(self.hp.clip_grad)
         self.clip_grad_num = self.hp.max_grad_norm
         self.v_loss_theta, self.ent_loss_theta = self.hp.v_coef, self.hp.ent_coef
@@ -83,6 +107,8 @@ class PPO(Basenn):
         self._mb_seed = None if seed is None else int(seed)
         self._mb_gen = None             # torch.Generator on the net's device (the minibatch shuffles)
         self._mb = None                 # persistent minibatch buffers (_minibatch_buffers)
+        self._fb = None                 # persistent full-batch buffers of the PPO options (_full_batch_inputs)
+        self._m3 = None                 # float64 [3] advantage moments of a data-parallel NORM_ADV step
         self.last_minibatch_perms = []  # per epoch of the last minibatch learn call: int32 device permutation of the rows
         self.gemm_mode = os.environ.get("DDRL_GEMM_MODE", _cfg(config_nn, "GEMM_MODE", "tc3"))
         self.update_time = 0
@@ -248,7 +274,8 @@ class PPO(Basenn):
             if old_m is not None and old_m.numel() == P:       # keep Adam state across a .to()/re-flatten
                 self._m.copy_(old_m)
                 self._v.copy_(old_v)
-            self._loss4 = torch.zeros(4, dtype=torch.float32, device=dev)
+            # {total, actor, v, entropy} (+ {approx KL, clip fraction, -, -} with PPO_STATS): one D2H copy per step
+            self._loss4 = torch.zeros(8 if self.ppo_stats else 4, dtype=torch.float32, device=dev)
         with torch.no_grad():
             for (pname, p), o in zip(plist, offsets):
                 view = flat[o:o + p.numel()].view(p.shape)
@@ -422,15 +449,17 @@ class PPO(Basenn):
         self._peer = st
 
     def _allreduce_grads(self):
-        """Sum of grads[0 : P+4] over the ranks, in place: the peer-memory kernel when the buffer is symmetric, else NCCL."""
+        """Sum of grads[0 : P+4] (P+5 with PPO_STATS) over the ranks, in place: the peer-memory kernel when the buffer is
+        symmetric, else NCCL."""
         st = self._peer
+        tail = 5 if self.ppo_stats else 4
         if st is not None and st["grads"] is self._grads:
             st["seq"] += 1
-            count = (self._P + 4 + 3) // 4 * 4                 # the buffer holds P + 8 floats
+            count = (self._P + tail + 3) // 4 * 4              # the buffer holds P + 8 floats
             check(_lib.load().ddrl_peer_allreduce_f32(st["bufs"], st["mc"], st["flag_ptrs"], st["rank"], st["world"], 0, count,
                                                       st["seq"], current_stream()), "ddrl_peer_allreduce_f32")
         else:
-            dist.allreduce_grads(self._grads, self._P, self._dp_group)
+            dist.allreduce_grads(self._grads, self._P, self._dp_group, tail)
 
     @_on_device
     def broadcast_parameters(self, src=0):
@@ -459,19 +488,25 @@ class PPO(Basenn):
         return args, (keep, advs, actions, old_logps, returns, rows), B
 
     @_on_device
-    def backward_only(self, states, advs, actions, old_logps, returns, b_global=None, obs_unchanged=False, minibatch=False):
+    def backward_only(self, states, advs, actions, old_logps, returns, b_global=None, obs_unchanged=False, minibatch=False,
+                      old_values=None):
         """forward + fused loss + backward for the local rows; grads (scaled 1/B_global) stay in flat_grads().
-        minibatch: the inputs are the persistent minibatch buffers (ddrl_net_backward_minibatch; 0 rows allowed)."""
+        minibatch: the inputs are the persistent minibatch buffers (ddrl_net_backward_minibatch; 0 rows allowed).
+        old_values: critic 0's rollout values [B], needed exactly when VALUE_CLIP is set."""
         self._ensure_engine()
         lib = _lib.load()
         args, held, B = self._bwd_args(states, advs, actions, old_logps, returns, b_global, obs_unchanged, minibatch)
         keep, rows = held[0], held[-1]
         dev = self._flat.device
         V = len(self._critics)
+        if old_values is not None:
+            old_values = old_values.to(device=dev, dtype=torch.float32).contiguous()
+        # the old-value pointer goes in before the hyper-parameters (ddrl_net_backward_v / _minibatch_v)
+        args = args[:9] + (ptr(old_values),) + args[9:]
         if minibatch:
-            check(lib.ddrl_net_backward_minibatch(*args[:-1], current_stream()), "ddrl_net_backward_minibatch")
+            check(lib.ddrl_net_backward_minibatch_v(*args[:-1], current_stream()), "ddrl_net_backward_minibatch_v")
         else:
-            check(lib.ddrl_net_backward(*args, current_stream()), "ddrl_net_backward")
+            check(lib.ddrl_net_backward_v(*args, current_stream()), "ddrl_net_backward_v")
         if V > 1 and self.prenet is not None:
             self._extra_grads_to_params()
         if V > 1 and self.prenet is None and self.gail_critic:
@@ -569,7 +604,9 @@ class PPO(Basenn):
         over `data` (an Experience whose tensors are on the device), yielding
         ({PpoTotalLoss, ActorLoss, VLoss, EntLoss, PpoBackUpTime}, update_time, True) per iteration.
         MINI_BATCH_NUM = M > 1: TRAINING_ITER_TIME shuffled epochs of M minibatches, one optimiser step and one yield
-        per minibatch (_learn_minibatch)."""
+        per minibatch (_learn_minibatch).
+        PPO_STATS adds ApproxKL and ClipFrac to every dict; with TARGET_KL the call ends after the first step whose ApproxKL
+        exceeds the target (that step is applied and yielded)."""
         if self.mini_batch_num > 1:
             yield from self._learn_minibatch(data)
             return
@@ -578,18 +615,74 @@ class PPO(Basenn):
         if self._dp_world > 1:
             self._ensure_engine()
             b_global = dist.global_rows(b_local, self._flat.device, self._dp_group)
+        options = self.norm_adv or self.value_clip is not None or self.ppo_stats
+        advs, old_values = self._full_batch_inputs(data) if options else (data.advs, None)
         for it in range(self.training_iter_time):
             start_time = time.time()
-            if self._dp_world > 1:
+            if self._dp_world > 1 and not options:
                 self._backward_allreduce(data, b_global, obs_unchanged=it > 0)
             else:
-                self.backward_only(data.states, data.advs, data.actions, data.old_logps, data.values, b_global,
-                                   obs_unchanged=it > 0)
-            loss4 = self.optimizer_step().tolist()          # ONE 16-byte D2H per iteration (reference: four .item())
-            self.update_time += 1
-            loss_log = {"PpoTotalLoss": loss4[0], "ActorLoss": loss4[1], "VLoss": loss4[2], "EntLoss": loss4[3],
-                        "PpoBackUpTime": time.time() - start_time}
+                # the options take the whole (not the segmented) backward, as extra critics do
+                self.backward_only(data.states, advs, data.actions, data.old_logps, data.values, b_global,
+                                   obs_unchanged=it > 0, old_values=old_values)
+                if self._dp_world > 1:
+                    self._allreduce_grads()
+            loss_log = self._step_and_log(start_time)
             yield loss_log, self.update_time, True
+            if self._kl_stop(loss_log):
+                return
+
+    def _step_and_log(self, start_time):
+        """clip+Adam, then the loss dict of the step from ONE D2H copy (reference: four .item())."""
+        loss = self.optimizer_step().tolist()
+        self.update_time += 1
+        loss_log = {"PpoTotalLoss": loss[0], "ActorLoss": loss[1], "VLoss": loss[2], "EntLoss": loss[3],
+                    "PpoBackUpTime": time.time() - start_time}
+        if self.ppo_stats:
+            loss_log["ApproxKL"] = loss[4]
+            loss_log["ClipFrac"] = loss[5]
+        return loss_log
+
+    def _kl_stop(self, loss_log):
+        # every rank of a data-parallel learner holds the same all-reduced ApproxKL, so all of them stop at the same step
+        return self.target_kl is not None and loss_log["ApproxKL"] > self.target_kl
+
+    def _old_values(self, data, advs, values):
+        """Critic 0's rollout values for VALUE_CLIP: data.old_values when the batch carries them, else values[0] - advs from
+        the raw advantages (the GAE of agent/gae.py makes returns = values + g and advs = g[0])."""
+        ov = getattr(data, "old_values", None)
+        if ov is not None:
+            return ov.to(device=self._flat.device, dtype=torch.float32).contiguous()
+        return values[0] - advs
+
+    def _normalize_advs(self, adv, out):
+        """NORM_ADV: out = (adv - mean) / (std + 1e-8) over the rows of the global step (all ranks' rows)."""
+        m3 = None
+        if self._dp_world > 1:
+            if self._m3 is None or self._m3.device != adv.device:
+                self._m3 = torch.zeros(3, dtype=torch.float64, device=adv.device)
+            m3 = dist.global_moments(kernels.adv_moments(adv, self._m3), self._dp_group)
+        kernels.adv_normalize(adv, m3, 1e-8, out)
+
+    @_on_device
+    def _full_batch_inputs(self, data):
+        """(advantages, old values) of a full-batch learn call with the PPO options: the advantages normalised once into a
+        persistent buffer (the caller's data.advs is never written) and the old values of VALUE_CLIP."""
+        self._ensure_engine()
+        dev = self._flat.device
+        advs = data.advs.to(device=dev, dtype=torch.float32).contiguous()
+        old_values = None
+        if self.value_clip is not None:
+            values = data.values.to(device=dev, dtype=torch.float32)
+            old_values = self._old_values(data, advs, values if values.dim() == 2 else values.view(1, -1))
+        if self.norm_adv:
+            key = (advs.numel(), dev)
+            if self._fb is None or self._fb["key"] != key:
+                self._fb = dict(key=key, advs=torch.empty(advs.numel(), dtype=torch.float32, device=dev))
+            out = self._fb["advs"]
+            self._normalize_advs(advs.view(-1), out)
+            advs = out
+        return advs, old_values
 
     # ------------------------------------------------------------------ minibatch epochs (non-reference option)
     @staticmethod
@@ -609,7 +702,9 @@ class PPO(Basenn):
         values = values if values.dim() == 2 else values.view(1, -1)
         src = dict(states=[f(data.states[i]) for i in range(n_obs)], actions=f(data.actions), old_logps=f(data.old_logps),
                    advs=f(data.advs), values=values)
-        if len(src["states"]) + 3 + values.shape[0] > _lib.GATHER_MAX_JOBS:
+        if self.value_clip is not None:
+            src["old_values"] = self._old_values(data, src["advs"], values)     # from the raw advantages, once per call
+        if len(src["states"]) + 3 + values.shape[0] + ("old_values" in src) > _lib.GATHER_MAX_JOBS:
             raise DDRLError("minibatch gather: %d return rows exceed the job limit" % values.shape[0])
         return src
 
@@ -618,19 +713,22 @@ class PPO(Basenn):
         b_local, M and the shapes stay the same, which is what lets ddrl_net_backward_minibatch replay its graph."""
         dev = self._flat.device
         key = (b_local, self.mini_batch_num, dev, tuple(tuple(t.shape[1:]) for t in src["states"]), tuple(src["actions"].shape[1:]),
-               src["values"].shape[0])
+               src["values"].shape[0], "old_values" in src)
         if self._mb is None or self._mb["key"] != key:
             rows = max(mb_rows, 1)
             e = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
             self._mb = dict(key=key, states=[e(rows, *t.shape[1:]) for t in src["states"]],
                             actions=e(rows, *src["actions"].shape[1:]), old_logps=e(rows), advs=e(rows),
                             values=e(src["values"].shape[0] * rows), zeros=torch.zeros(rows, dtype=torch.float32, device=dev))
+            if "old_values" in src:
+                self._mb["old_values"] = e(rows)
         return self._mb
 
     @_on_device
     def _gather_minibatch(self, src, rows):
-        """Gathers the rows `rows` (int32 device) of every source into the minibatch buffers in ONE launch; returns the
-        (states, advs, actions, old_logps, returns [V, n]) views backward_only takes."""
+        """Gathers the rows `rows` (int32 device) of every source into the minibatch buffers in ONE launch, then normalises
+        the gathered advantages in place (NORM_ADV); returns the (states, advs, actions, old_logps, returns [V, n],
+        old_values | None) views backward_only takes."""
         mb, n = self._mb, rows.numel()
         V = src["values"].shape[0]
         ret = mb["values"][:V * n]
@@ -638,8 +736,13 @@ class PPO(Basenn):
             pairs = [(s, d) for s, d in zip(src["states"], mb["states"])]
             pairs += [(src["actions"], mb["actions"]), (src["old_logps"], mb["old_logps"]), (src["advs"], mb["advs"])]
             pairs += [(src["values"][v], ret[v * n:(v + 1) * n]) for v in range(V)]
+            if "old_values" in src:
+                pairs.append((src["old_values"], mb["old_values"]))
             kernels.gather_rows(rows, pairs)
-        return [t[:n] for t in mb["states"]], mb["advs"][:n], mb["actions"][:n], mb["old_logps"][:n], ret.view(V, n)
+        if self.norm_adv:
+            self._normalize_advs(mb["advs"][:n], mb["advs"][:n])   # in place: the buffers keep their graph-replay addresses
+        old_values = mb["old_values"][:n] if "old_values" in src else None
+        return [t[:n] for t in mb["states"]], mb["advs"][:n], mb["actions"][:n], mb["old_logps"][:n], ret.view(V, n), old_values
 
     def _learn_minibatch(self, data):
         """TRAINING_ITER_TIME epochs; each draws a permutation of the local rows (net-owned generator) and cuts it into
@@ -667,15 +770,14 @@ class PPO(Basenn):
             self.last_minibatch_perms.append(perm)
             for (lo, hi), b_global in zip(plan, b_globals):
                 start_time = time.time()
-                states, advs, actions, old_logps, returns = self._gather_minibatch(src, perm[lo:hi])
-                self.backward_only(states, advs, actions, old_logps, returns, b_global, minibatch=True)
+                states, advs, actions, old_logps, returns, old_values = self._gather_minibatch(src, perm[lo:hi])
+                self.backward_only(states, advs, actions, old_logps, returns, b_global, minibatch=True, old_values=old_values)
                 if self._dp_world > 1:
                     self._allreduce_grads()
-                loss4 = self.optimizer_step().tolist()
-                self.update_time += 1
-                loss_log = {"PpoTotalLoss": loss4[0], "ActorLoss": loss4[1], "VLoss": loss4[2], "EntLoss": loss4[3],
-                            "PpoBackUpTime": time.time() - start_time}
+                loss_log = self._step_and_log(start_time)
                 yield loss_log, self.update_time, True
+                if self._kl_stop(loss_log):
+                    return
 
     def add_critic(self, critic):
         """nn/ppo.py:63-64.  The extra critic's values come back from forward()/act() as further rows; its value loss joins

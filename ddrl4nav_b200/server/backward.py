@@ -33,7 +33,8 @@ class BackwardModule:
         if self._prefetched is not None and self._prefetched[0] is train_data:
             main = torch.cuda.current_stream(torch.device(self.device))
             main.wait_event(self._prefetched[1])
-            for t in list(train_data.states) + [train_data.advs, train_data.actions, train_data.old_logps, train_data.values]:
+            extra = [train_data.old_values] if getattr(train_data, "old_values", None) is not None else []
+            for t in list(train_data.states) + [train_data.advs, train_data.actions, train_data.old_logps, train_data.values] + extra:
                 t.record_stream(main)
             self._prefetched = None
         else:

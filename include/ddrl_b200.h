@@ -73,6 +73,9 @@ typedef struct {     /* config/config_nn.py:27-57; torch.optim.Adam defaults */
   float lr_actor;        /* ACTOR_LEARNING_RATE */
   float lr_critic;       /* CRITIC_LEARNING_RATE */
   float beta1, beta2, adam_eps;
+  /* non-reference PPO options (0 = off; appended so that a struct built from the fields above stays valid) */
+  float value_clip;      /* VALUE_CLIP: clip width c > 0 of critic 0's value loss around the rollout's values (old_values) */
+  int32_t ppo_stats;     /* PPO_STATS: the net's loss sums also accumulate the approx KL and the clip fraction */
 } ddrl_ppo_hparams;
 
 /* ---- library ------------------------------------------------------------------------- */
@@ -171,6 +174,31 @@ int ddrl_ppo_loss_gaussian(const float* mu, int ld, const float* log_std, const 
                            const float* old_logp, const float* adv, const float* returns, const float* v,
                            int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
                            float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums, void* stream);
+/* The same with the non-reference options.  old_values [B] (rollout values of critic 0) or NULL: when given, critic 0's value
+ * loss is clipped, v_c = old_values + clamp(v - old_values, -hp->value_clip, hp->value_clip) and loss = max(vloss(R, v),
+ * vloss(R, v_c)) per row (clamp's gradient passes on the closed interval, ties of max split 1/2-1/2); it must be given exactly
+ * when hp->value_clip > 0 (else DDRL_E_ARG).  stats (2 floats) or NULL: stats[0] += inv_B_global * sum((r - 1) - log r)
+ * (approx KL) and stats[1] += inv_B_global * #{|r - 1| > hp->ppo_clip} (clip fraction), r = this pass's ratio.  With both
+ * NULL these are the calls above, which write nothing past loss_sums[2]. */
+int ddrl_ppo_loss_categorical_v(const float* logits, int ld, const float* actions, const float* old_logp,
+                                const float* adv, const float* returns, const float* v, int B, int A,
+                                float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                                float* dlogits, int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
+                                void* stream);
+int ddrl_ppo_loss_gaussian_v(const float* mu, int ld, const float* log_std, const float* actions,
+                             const float* old_logp, const float* adv, const float* returns, const float* v,
+                             int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                             float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums, const float* old_values,
+                             float* stats, void* stream);
+
+/* ---- advantage normalisation (non-reference option NORM_ADV) -------------------------------
+ * ddrl_adv_moments: m3[0..2] = {n, sum a, sum a^2} of adv[0..n) in fp64 (m3: DEVICE, 3 doubles); a data-parallel learner sums
+ * them over the ranks.  ddrl_adv_normalize: out[i] = (adv[i] - mean) / (std + eps) with std the unbiased standard deviation of
+ * the moments m3, or of adv[0..n) itself when m3 is NULL (one launch); a moment count <= 1 copies adv unchanged.  Both run as
+ * ONE block with a fixed reduction order, so their results are bit-reproducible without deterministic mode, and both can be
+ * captured in a graph.  out may be adv. */
+int ddrl_adv_moments(const float* adv, int n, double* m3, void* stream);
+int ddrl_adv_normalize(const float* adv, int n, const double* m3, float eps, float* out, void* stream);
 
 /* Value loss of ONE extra critic head (nn/ppo.py:97-104: rndv_loss / gailv_loss = vlossf(data.values[k], values[k])):
  * dv[b] = d(loss)/d(v[b]) (times v_coef when shared, ppo.py:108), loss_sums[1] += contribution scaled by inv_B_global. */
@@ -224,7 +252,8 @@ int64_t ddrl_net_num_params(const ddrl_net* net);
 int ddrl_net_tensor_info(const ddrl_net* net, int i, char* name, int name_cap,
                          int64_t* shape4, int* ndim, int64_t* offset);
 /* flat device buffers (reference layout/order).  grads has num_params + 8 floats: the tail
- * [P .. P+3] carries {actor, v, entropy, unused} loss sums so one all-reduce covers both.
+ * [P .. P+3] carries {actor, v, entropy, unused} loss sums so one all-reduce covers both; with hp->ppo_stats the backward
+ * passes write [P .. P+4] = {actor, v, entropy, approx-KL, clip-fraction} sums.
  * grads/m/v may be NULL for an inference-only net. */
 int ddrl_net_bind(ddrl_net* net, float* params, float* grads, float* adam_m, float* adam_v);
 /* Extra value heads (nn/ppo.py:63-64 `add_critic`, :75 `[critic(states) for critic in self._critics]`, :95-105 the V > 1
@@ -260,18 +289,24 @@ int ddrl_net_encode(ddrl_net* net, const float* const* obs, int n_obs, int B, in
 /* One learn iteration, first half (nn/ppo.py:82-123): forward with act=data.actions, fused loss,
  * backward through heads and encoders.  Leaves d(loss)/d(params) for the LOCAL B rows, scaled
  * by 1/B_global, in the flat grads buffer and the loss sums in its tail.  In a data-parallel
- * learner the caller all-reduces grads[0 .. P+4) (sum) before ddrl_net_clip_adam.
+ * learner the caller all-reduces grads[0 .. P+4) (sum; [0 .. P+5) with hp->ppo_stats) before ddrl_net_clip_adam.
  * obs_unchanged != 0: the caller guarantees obs[] hold the same bytes as in the previous backward call
  * (iterations 2..10 of PPO.learn); observation-side staging is then reused. */
 int ddrl_net_backward(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
                       const float* actions, const float* old_logp, const float* adv, const float* returns,
                       const ddrl_ppo_hparams* hp, int obs_unchanged, void* stream);
+/* ddrl_net_backward with old_values [B_local] (critic 0's rollout values) for hp->value_clip > 0 (ddrl_ppo_loss_*_v); NULL
+ * otherwise.  hp->value_clip > 0 with old_values NULL returns DDRL_E_ARG.  ddrl_net_backward passes NULL. */
+int ddrl_net_backward_v(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
+                        const float* actions, const float* old_logp, const float* adv, const float* returns,
+                        const float* old_values, const ddrl_ppo_hparams* hp, int obs_unchanged, void* stream);
 /* The same pass in SEGMENTS, for a data-parallel learner that overlaps the gradient all-reduce with the rest of the
  * backward (nn/ppo.py:113-123 runs the actor and the critic backward one after the other; server/backward.py:167 "TODO multi
  * GPU").  Call with segment = 0, 1, ..., *n_segments - 1 in order and the SAME arguments; after segment k returns (stream
  * order), every parameter tensor i with ddrl_net_tensor_segment(net, i) == k holds its final gradient in the flat buffer
  * and may be reduced on another stream while segment k + 1 runs.  A pass that cannot be cut (first iteration of a learn
  * call, micro-batched rows, extra critics) runs whole in segment 0 and reports *n_segments = 1. */
+/* The segmented pass takes no old_values: hp->value_clip > 0 returns DDRL_E_ARG. */
 int ddrl_net_backward_segment(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
                               const float* actions, const float* old_logp, const float* adv, const float* returns,
                               const ddrl_ppo_hparams* hp, int obs_unchanged, int segment, int* n_segments, void* stream);
@@ -309,8 +344,13 @@ int ddrl_gather_rows(const int32_t* rows, int n_rows, const ddrl_gather_job* job
 int ddrl_net_backward_minibatch(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
                                 const float* actions, const float* old_logp, const float* adv, const float* returns,
                                 const ddrl_ppo_hparams* hp, void* stream);
+/* ddrl_net_backward_minibatch with old_values, as ddrl_net_backward_v. */
+int ddrl_net_backward_minibatch_v(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
+                                  const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                  const float* old_values, const ddrl_ppo_hparams* hp, void* stream);
 /* second half (nn/ppo.py:115-129): global-norm clip + the two (or one) Adam steps; then refreshes
- * the packed weights.  loss4_out (device, 4 floats, optional) = {total, actor, v, entropy}. */
+ * the packed weights.  loss4_out (device, 4 floats, optional) = {total, actor, v, entropy}; with hp->ppo_stats it must
+ * hold 6 floats and receives {total, actor, v, entropy, approx KL, clip fraction}. */
 int ddrl_net_clip_adam(ddrl_net* net, int step, const ddrl_ppo_hparams* hp, float* loss4_out, void* stream);
 /* bytes of device workspace currently held */
 int64_t ddrl_net_workspace_bytes(const ddrl_net* net);
