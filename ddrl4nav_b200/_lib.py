@@ -74,6 +74,10 @@ SIGNATURES = {
                                      _P, _P]),
     "ddrl_adv_moments": (_I, [_P, _I, _P, _P]),
     "ddrl_adv_normalize": (_I, [_P, _I, _P, _F, _P, _P]),
+    "ddrl_obs_moments_ws_bytes": (_L, [_I, _I]),
+    "ddrl_obs_moments": (_I, [_P, _I, _I, _P, _P, _P, _L, _P]),
+    "ddrl_obs_rms_update": (_I, [_P, _P, _P, _P, C.c_double, _I, _P, _P, _P]),
+    "ddrl_obs_normalize": (_I, [_P, _I, _I, _P, _P, _F, _P, _P]),
     "ddrl_value_loss": (_I, [_P, _P, _I, _F, C.POINTER(PPOHparams), _I, _P, _P, _P]),
     "ddrl_clip_adam": (_I, [_P, _P, _P, _P, _L, C.POINTER(_L), C.POINTER(_F), _I, _I, C.POINTER(PPOHparams), _P, _P]),
     "ddrl_gemm_f32": (_I, [_I, _I, _I, _I, _I, _P, _I, _P, _I, _P, _I, _P, _I, _I, _P]),

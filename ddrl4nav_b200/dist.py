@@ -74,6 +74,17 @@ def global_moments(m3: torch.Tensor, group=None) -> torch.Tensor:
     return m3
 
 
+def global_obs_sums(sums: torch.Tensor, group=None) -> torch.Tensor:
+    """In-place sum over ranks of the float64 observation moments of every normalised slot, concatenated into ONE buffer
+    (kernels.obs_moments, NORM_OBS): every rank shifts by the same running mean, so the sums add, and every rank then merges
+    the same global batch into its statistics.  One collective per learn call."""
+    import torch.distributed as dist
+    _, ws = world(group)
+    if ws > 1:
+        dist.all_reduce(sums, group=group)
+    return sums
+
+
 def broadcast_params(flat_params: torch.Tensor, src: int = 0, group=None) -> None:
     import torch.distributed as dist
     _, ws = world(group)

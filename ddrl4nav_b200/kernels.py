@@ -280,6 +280,82 @@ def adv_normalize(adv: torch.Tensor, m3: Optional[torch.Tensor] = None, eps: flo
     return out
 
 
+def _rows_of(x: torch.Tensor, D: int, what: str) -> int:
+    """Rows of x read as a row-major [B, D] fp32 block."""
+    require_cuda(x)
+    if x.dtype != torch.float32 or not x.is_contiguous():
+        raise DDRLError("%s: x must be a contiguous fp32 tensor" % what)
+    B = x.shape[0] if x.dim() else 1
+    if x.numel() != B * D:
+        raise DDRLError("%s: x has shape %s; expected [B, %d elements/row]" % (what, tuple(x.shape), D))
+    return B
+
+
+def _f64_vec(t: torch.Tensor, n: int, dev, what: str):
+    if t.dtype != torch.float64 or t.numel() != n or not t.is_contiguous() or t.device != dev:
+        raise DDRLError("%s must be a contiguous float64 [%d] tensor on %s" % (what, n, dev))
+
+
+def obs_moments(x: torch.Tensor, shift: torch.Tensor, sums: Optional[torch.Tensor] = None,
+                ws: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Column sums {sum (x - shift), sum (x - shift)^2} of x read as [B, D] (D = shift.numel()), in float64, into `sums` [2D]
+    (ddrl_obs_moments; bit-reproducible for given (B, D)).  ws: a byte workspace of at least obs_moments_ws_bytes(B, D), else
+    one is allocated."""
+    D = shift.numel()
+    B = _rows_of(x, D, "obs_moments")
+    _f64_vec(shift, D, x.device, "obs_moments: shift")
+    if sums is None:
+        sums = torch.empty(2 * D, dtype=torch.float64, device=x.device)
+    _f64_vec(sums, 2 * D, x.device, "obs_moments: sums")
+    need = obs_moments_ws_bytes(B, D)
+    if need and (ws is None or ws.numel() * ws.element_size() < need):
+        ws = torch.empty(need, dtype=torch.uint8, device=x.device)
+    nbytes = ws.numel() * ws.element_size() if ws is not None else 0
+    check(_lib.load().ddrl_obs_moments(ptr(x), B, D, ptr(shift), ptr(sums), ptr(ws), nbytes, current_stream()),
+          "ddrl_obs_moments")
+    return sums
+
+
+def obs_moments_ws_bytes(B: int, D: int) -> int:
+    return int(_lib.load().ddrl_obs_moments_ws_bytes(int(B), int(D)))
+
+
+def obs_rms_update(mean: torch.Tensor, var: torch.Tensor, count: torch.Tensor, sums: Optional[torch.Tensor], n: float,
+                   mean32: torch.Tensor, scale32: torch.Tensor) -> None:
+    """Merges the batch of `n` rows whose moments (obs_moments around `mean`) are `sums` into the running float64 {mean, var,
+    count} in place, then writes the applied form mean32 / scale32 (ddrl_obs_rms_update).  n = 0: the applied form only."""
+    D = mean.numel()
+    dev = mean.device
+    require_cuda(mean)
+    for t, k, what in ((mean, D, "mean"), (var, D, "var"), (count, 1, "count")):
+        _f64_vec(t, k, dev, "obs_rms_update: " + what)
+    if n > 0:
+        _f64_vec(sums, 2 * D, dev, "obs_rms_update: sums")
+    for t, what in ((mean32, "mean32"), (scale32, "scale32")):
+        if t.dtype != torch.float32 or t.numel() != D or not t.is_contiguous() or t.device != dev:
+            raise DDRLError("obs_rms_update: %s must be a contiguous fp32 [%d] tensor on %s" % (what, D, dev))
+    check(_lib.load().ddrl_obs_rms_update(ptr(mean), ptr(var), ptr(count), ptr(sums) if n > 0 else None, float(n), D,
+                                          ptr(mean32), ptr(scale32), current_stream()), "ddrl_obs_rms_update")
+
+
+def obs_normalize(x: torch.Tensor, mean32: torch.Tensor, scale32: torch.Tensor, clip: Optional[float],
+                  out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """clamp((x - mean32) * scale32, -clip, clip) per column of x read as [B, D] (D = mean32.numel()); clip None: no clamp
+    (ddrl_obs_normalize, one launch).  out may be x (in place)."""
+    D = mean32.numel()
+    B = _rows_of(x, D, "obs_normalize")
+    if out is None:
+        out = torch.empty_like(x)
+    if out.dtype != torch.float32 or not out.is_contiguous() or out.numel() != x.numel() or out.device != x.device:
+        raise DDRLError("obs_normalize: out must be a contiguous fp32 tensor shaped like x")
+    for t, what in ((mean32, "mean32"), (scale32, "scale32")):
+        if t.dtype != torch.float32 or t.numel() != D or not t.is_contiguous() or t.device != x.device:
+            raise DDRLError("obs_normalize: %s must be a contiguous fp32 [%d] tensor on %s" % (what, D, x.device))
+    check(_lib.load().ddrl_obs_normalize(ptr(x), B, D, ptr(mean32), ptr(scale32), float(clip or 0.0), ptr(out),
+                                         current_stream()), "ddrl_obs_normalize")
+    return out
+
+
 def launch_count() -> int:
     return int(_lib.load().ddrl_launch_count())
 

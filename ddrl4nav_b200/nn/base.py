@@ -3,7 +3,8 @@
 Weight (de)serialisation keeps the reference's wire format (base.py:38-54): for every
 ``named_parameters()`` entry, in order, ``>I ndim | >I*ndim shape | raw fp32 bytes``.  Unlike
 the reference (one ``.cpu()`` and one ``bytes +=`` per parameter) the blob is produced from a
-single device->host copy of the flat parameter buffer.
+single device->host copy of the flat parameter buffer.  A subclass may append further records
+in the same format after the parameters (``_state_records``): ``PPO`` does so for its NORM_OBS statistics only.
 """
 import struct
 
@@ -47,8 +48,15 @@ class Basenn(torch.nn.Module):
         """[(name, np.ndarray)] in named_parameters() order; subclasses with a flat buffer override."""
         return [(k, v.detach().cpu().numpy()) for k, v in self.named_parameters()]
 
+    def _state_records(self):
+        """[np.ndarray] written after the parameter records, in the same record format (none here)."""
+        return []
+
+    def _load_state_records(self, view):
+        """Reads what _state_records wrote from `view`, the bytes after the parameter records (nothing here)."""
+
     def model_bytes(self) -> bytes:
-        return b"".join(self._encode_wb(a) for _, a in self._params_to_host())
+        return b"".join(self._encode_wb(a) for a in [a for _, a in self._params_to_host()] + self._state_records())
 
     def nn2redis(self, pipe, update_key, key=None):
         pipe.set(key if key else self.model_key, self.model_bytes())
@@ -63,6 +71,7 @@ class Basenn(torch.nn.Module):
                 wb, used = self._decode_wb(view[index:])
                 index += used
                 p.copy_(torch.from_numpy(np.ascontiguousarray(wb)).to(p.device))
+        self._load_state_records(view[index:])
         self._weights_changed()
 
     def updatenn_by_redis(self, conn, key=None):

@@ -14,10 +14,12 @@ order); ``p.data`` of every ``nn.Parameter`` is a view into it.  Gradients, Adam
 buffers of the same layout, so the data-parallel learner all-reduces one buffer and the fused
 clip+Adam kernel walks it once.  No autograd graph is ever built.
 """
+import copy
 import ctypes as C
 import functools
 import math
 import os
+import struct
 import time
 
 import numpy as np
@@ -28,6 +30,7 @@ from torch.distributions.normal import Normal
 from .. import _lib, dist, kernels
 from .._lib import DDRLError, NetDesc, check, current_stream, ptr
 from .base import Basenn
+from .obs_rms import ObsRMS
 
 
 def _on_device(fn):
@@ -54,13 +57,26 @@ def _flag_option(config_nn, name):
     return bool(v)
 
 
-def _positive_option(config_nn, name):
-    v = _cfg(config_nn, name, None)
+def _positive_option(config_nn, name, default=None):
+    v = _cfg(config_nn, name, default)
     if v is None:
         return None
     if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)) or not math.isfinite(v) or v <= 0:
         raise DDRLError("%s must be a finite number > 0 or None (got %r)" % (name, v))
     return float(v)
+
+
+def _slots_option(config_nn, name):
+    """False (off), True (every observation slot) or a list / tuple of distinct slot indices -> None (off), "all" or a sorted
+    tuple.  Indices beyond the net's slots are rejected when the engine is built (ObsRMS.bind)."""
+    v = _cfg(config_nn, name, False)
+    if isinstance(v, (bool, np.bool_)):
+        return "all" if v else None
+    ok = isinstance(v, (list, tuple)) and len(v) > 0 and all(
+        isinstance(s, (int, np.integer)) and not isinstance(s, (bool, np.bool_)) and s >= 0 for s in v)
+    if not ok or len(set(int(s) for s in v)) != len(v):
+        raise DDRLError("%s must be True, False or a non-empty list of distinct slot indices >= 0 (got %r)" % (name, v))
+    return tuple(sorted(int(s) for s in v))
 
 
 class PPO(Basenn):
@@ -84,6 +100,14 @@ class PPO(Basenn):
         self.value_clip = _positive_option(config_nn, "VALUE_CLIP")
         self.target_kl = _positive_option(config_nn, "TARGET_KL")
         self.ppo_stats = _flag_option(config_nn, "PPO_STATS") or self.target_kl is not None
+        # running observation normalisation (non-reference, off by default): float64 statistics of the chosen slots in the
+        # submodule obs_rms (state_dict keys obs_rms.{mean,var,count}_<slot>), applied by act / forward / encode / learn
+        norm_obs = _slots_option(config_nn, "NORM_OBS")
+        clip = _positive_option(config_nn, "NORM_OBS_CLIP", 10.0)
+        self.obs_rms = None if norm_obs is None else ObsRMS(None if norm_obs == "all" else norm_obs, clip)
+        self._obs_act = {}              # NORM_OBS: per slot, the act / encode scratch (grows with B)
+        self._obs_learn = {}            # NORM_OBS: per slot, the learner's persistent normalised batch
+        self._obs_n = 0                 # NORM_OBS: rows of the global batch of the current learn call
         self.hp = kernels.make_hparams(
             ppo_clip=_cfg(config_nn, "PPO_CLIP", 0.2), dual_clip=_cfg(config_nn, "DUEL_PPO_CLIP", 3),
             v_coef=_cfg(config_nn, "V_LOSS_THETA", 1.0), ent_coef=_cfg(config_nn, "ENTROPY_LOSS_THETA", 0.05),
@@ -246,6 +270,12 @@ class PPO(Basenn):
         h = C.c_void_p()
         check(lib.ddrl_net_create(C.byref(desc), C.byref(h)), "ddrl_net_create")
         self._h = h
+        if self.obs_rms is not None:
+            try:
+                self.obs_rms.bind(lib.ddrl_net_num_obs(h), lambda i: lib.ddrl_net_obs_elems(h, i), dev)
+            except DDRLError:
+                self._destroy()
+                raise
         nt = lib.ddrl_net_num_tensors(h)
         P = lib.ddrl_net_num_params(h)
         if nt != len(plist):
@@ -309,6 +339,36 @@ class PPO(Basenn):
         host = self._flat.detach().cpu().numpy()               # ONE D2H copy for the whole model blob
         return [(n, host[o:o + p.numel()].reshape(tuple(p.shape))) for (n, p), o in zip(self.named_parameters(), self._offsets)]
 
+    @_on_device
+    def _state_records(self):
+        """NORM_OBS: per normalised slot, in slot order, the records mean32 [D], scale32 [D] and count [1] after the
+        parameters, so that a predictor loading the blob acts with exactly the learner's applied form."""
+        if self.obs_rms is None:
+            return []
+        self._ensure_engine()
+        return self.obs_rms.records()
+
+    @_on_device
+    def _load_state_records(self, view):
+        if self.obs_rms is None:
+            return
+        self._ensure_engine()
+        rms, recs, index = self.obs_rms, [], 0
+        for s in rms.slots:
+            got = []
+            for what, n in (("mean32", rms.dims[s]), ("scale32", rms.dims[s]), ("count", 1)):
+                try:
+                    wb, used = self._decode_wb(view[index:])
+                except (struct.error, ValueError):
+                    wb, used = None, 0
+                if wb is None or wb.shape != (n,):
+                    raise DDRLError("model blob has no NORM_OBS %s record [%d] for slot %d after the parameters (written by a net "
+                                    "without NORM_OBS, or with other slots?)" % (what, n, s))
+                got.append(wb)
+                index += used
+            recs.append(got)
+        rms.load_records(recs)
+
     def flat_grads(self):
         """View of the flat gradient buffer (reference parameter order) of the last backward."""
         return self._grads[:self._P]
@@ -337,6 +397,27 @@ class PPO(Basenn):
         arr = (C.c_void_p * n_obs)(*[t.data_ptr() for t in keep])
         return keep, arr, n_obs, B
 
+    def _normalized_obs(self, states, bufs):
+        """NORM_OBS: `states` with every normalised slot replaced by its normalised copy in bufs[slot] (the persistent learner
+        buffers, or the act scratch, which grows with B); the caller's tensors are never written."""
+        rms = self.obs_rms
+        rms.refresh()
+        dev = self._flat.device
+        out = list(states)
+        for s in rms.slots:
+            if s >= len(out):
+                break                   # _obs_ptrs reports the missing slot
+            x = out[s] if torch.is_tensor(out[s]) else torch.as_tensor(np.asarray(out[s]))
+            x = x.to(device=dev, dtype=torch.float32).contiguous()
+            B = x.shape[0] if x.dim() else 0
+            if x.dim() == 0 or x.numel() != B * rms.dims[s]:
+                raise DDRLError("state slot %d has shape %s; expected [B=%d, %d elements/sample]" % (s, tuple(x.shape), B, rms.dims[s]))
+            buf = bufs.get(s)
+            if buf is None or buf.shape[0] < B or buf.shape[1:] != x.shape[1:]:
+                buf = bufs[s] = torch.empty(x.shape, dtype=torch.float32, device=dev)
+            out[s] = rms.normalize(s, x, buf[:B])
+        return out
+
     # ------------------------------------------------------------------ Forward module
     @_on_device
     def act(self, states, draw=None, play_mode=False, want_pi=False):
@@ -347,6 +428,8 @@ class PPO(Basenn):
         critics (1 unless add_critic was called)."""
         self._ensure_engine()
         lib = _lib.load()
+        if self.obs_rms is not None:
+            states = self._normalized_obs(states, self._obs_act)
         keep, arr, n_obs, B = self._obs_ptrs(states)
         dev = self._flat.device
         A = self.actor.actor_linear.out_features
@@ -373,8 +456,10 @@ class PPO(Basenn):
     @_on_device
     def encode(self, states, tower=0):
         """Features [B, feat] of one encoder tower (0 = prenet / actor.pre, 1 = critic.pre): the stand-alone encoder
-        forward of the reference (nn/atari_encoder.py:25-32, nn/nav_encoder.py:35-43,115-128)."""
+        forward of the reference (nn/atari_encoder.py:25-32, nn/nav_encoder.py:35-43,115-128).  NORM_OBS normalises first."""
         self._ensure_engine()
+        if self.obs_rms is not None:
+            states = self._normalized_obs(states, self._obs_act)
         keep, arr, n_obs, B = self._obs_ptrs(states)
         out = torch.empty(B, self.actor.actor_linear.in_features, dtype=torch.float32, device=self._flat.device)
         check(_lib.load().ddrl_net_encode(self._h, arr, n_obs, B, int(tower), ptr(out), current_stream()), "ddrl_net_encode")
@@ -492,7 +577,8 @@ class PPO(Basenn):
                       old_values=None):
         """forward + fused loss + backward for the local rows; grads (scaled 1/B_global) stay in flat_grads().
         minibatch: the inputs are the persistent minibatch buffers (ddrl_net_backward_minibatch; 0 rows allowed).
-        old_values: critic 0's rollout values [B], needed exactly when VALUE_CLIP is set."""
+        old_values: critic 0's rollout values [B], needed exactly when VALUE_CLIP is set.
+        This is the engine-level pass: with NORM_OBS it takes `states` as given, so they must already be normalised."""
         self._ensure_engine()
         lib = _lib.load()
         args, held, B = self._bwd_args(states, advs, actions, old_logps, returns, b_global, obs_unchanged, minibatch)
@@ -606,7 +692,9 @@ class PPO(Basenn):
         MINI_BATCH_NUM = M > 1: TRAINING_ITER_TIME shuffled epochs of M minibatches, one optimiser step and one yield
         per minibatch (_learn_minibatch).
         PPO_STATS adds ApproxKL and ClipFrac to every dict; with TARGET_KL the call ends after the first step whose ApproxKL
-        exceeds the target (that step is applied and yielded)."""
+        exceeds the target (that step is applied and yielded).
+        NORM_OBS: every step sees the observations normalised with the statistics held when the call started (those the
+        Forward module acted with); the call's batch is folded into the statistics once, before the final step's yield."""
         if self.mini_batch_num > 1:
             yield from self._learn_minibatch(data)
             return
@@ -615,6 +703,8 @@ class PPO(Basenn):
         if self._dp_world > 1:
             self._ensure_engine()
             b_global = dist.global_rows(b_local, self._flat.device, self._dp_group)
+        if self.obs_rms is not None:
+            data = self._obs_norm_begin(data, b_global)
         options = self.norm_adv or self.value_clip is not None or self.ppo_stats
         advs, old_values = self._full_batch_inputs(data) if options else (data.advs, None)
         for it in range(self.training_iter_time):
@@ -628,9 +718,38 @@ class PPO(Basenn):
                 if self._dp_world > 1:
                     self._allreduce_grads()
             loss_log = self._step_and_log(start_time)
+            stop = self._kl_stop(loss_log)
+            if self.obs_rms is not None and (stop or it == self.training_iter_time - 1):
+                self._obs_norm_end()
             yield loss_log, self.update_time, True
-            if self._kl_stop(loss_log):
+            if stop:
                 return
+
+    @_on_device
+    def _obs_norm_begin(self, data, n_global):
+        """NORM_OBS at the start of a learn call: the moments of the raw batch around the current running mean (summed over
+        the ranks of a data-parallel learner: one collective), and the batch normalised with the current statistics into
+        the persistent buffers.  Returns a shallow copy of `data` holding the normalised states."""
+        self._ensure_engine()
+        rms = self.obs_rms
+        raw = {}
+        for s in rms.slots:
+            if s < len(data.states):
+                t = data.states[s]
+                t = t if torch.is_tensor(t) else torch.as_tensor(np.asarray(t))
+                raw[s] = t.to(device=self._flat.device, dtype=torch.float32).contiguous()
+        states = self._normalized_obs([raw.get(i, x) for i, x in enumerate(data.states)], self._obs_learn)
+        rms.moments(raw)
+        if self._dp_world > 1:
+            dist.global_obs_sums(rms.sums, self._dp_group)
+        self._obs_n = n_global
+        out = copy.copy(data)
+        out.states = states
+        return out
+
+    @_on_device
+    def _obs_norm_end(self):
+        self.obs_rms.merge(self._obs_n)
 
     def _step_and_log(self, start_time):
         """clip+Adam, then the loss dict of the step from ONE D2H copy (reference: four .item())."""
@@ -757,6 +876,8 @@ class PPO(Basenn):
         plan = self.minibatch_plan(b_local, m)
         sizes = [hi - lo for lo, hi in plan]
         b_globals = dist.global_chunk_rows(sizes, dev, self._dp_group) if self._dp_world > 1 else sizes
+        if self.obs_rms is not None:
+            data = self._obs_norm_begin(data, sum(b_globals))       # the gathers then read the normalised batch
         src = self._minibatch_sources(data)
         self._minibatch_buffers(src, b_local, max(sizes))
         if self._mb_gen is None or self._mb_gen.device != dev:
@@ -765,18 +886,21 @@ class PPO(Basenn):
             self._mb_gen = torch.Generator(device=dev)
             self._mb_gen.manual_seed(self._mb_seed)
         self.last_minibatch_perms = []
-        for _ in range(self.training_iter_time):
+        for epoch in range(self.training_iter_time):
             perm = torch.randperm(b_local, generator=self._mb_gen, device=dev, dtype=torch.int32)
             self.last_minibatch_perms.append(perm)
-            for (lo, hi), b_global in zip(plan, b_globals):
+            for k, ((lo, hi), b_global) in enumerate(zip(plan, b_globals)):
                 start_time = time.time()
                 states, advs, actions, old_logps, returns, old_values = self._gather_minibatch(src, perm[lo:hi])
                 self.backward_only(states, advs, actions, old_logps, returns, b_global, minibatch=True, old_values=old_values)
                 if self._dp_world > 1:
                     self._allreduce_grads()
                 loss_log = self._step_and_log(start_time)
+                stop = self._kl_stop(loss_log)
+                if self.obs_rms is not None and (stop or (epoch == self.training_iter_time - 1 and k == m - 1)):
+                    self._obs_norm_end()
                 yield loss_log, self.update_time, True
-                if self._kl_stop(loss_log):
+                if stop:
                     return
 
     def add_critic(self, critic):

@@ -200,6 +200,23 @@ int ddrl_ppo_loss_gaussian_v(const float* mu, int ld, const float* log_std, cons
 int ddrl_adv_moments(const float* adv, int n, double* m3, void* stream);
 int ddrl_adv_normalize(const float* adv, int n, const double* m3, float eps, float* out, void* stream);
 
+/* ---- running observation normalisation (non-reference option NORM_OBS) ---------------------
+ * ddrl_obs_moments: sums[0..D) = column sums of d = x - shift and sums[D..2D) = column sums of d^2, in fp64, over the row-major
+ * fp32 x [B, D] (shift, sums: DEVICE doubles).  Rows are cut into fixed chunks whose partials go to `ws` (at least
+ * ddrl_obs_moments_ws_bytes(B, D) bytes; 0 when one chunk covers B, and ws may then be NULL), then a second launch adds them in
+ * chunk order: the result depends on (B, D) only, so it is bit-reproducible run to run, rank to rank and device to device.
+ * ddrl_obs_rms_update: Chan's merge of the batch {n, mean = shift + S1/n, var = S2/n - (S1/n)^2} into the running {mean [D],
+ * var [D], count [1]} (fp64, DEVICE; shift = the running mean the sums were taken around), then the applied form
+ * mean32 = fp32(mean), scale32 = fp32(1 / sqrt(var + 1e-8)); n = 0 rewrites only the applied form (sums may be NULL).
+ * ddrl_obs_normalize: out = min(max((x - mean32) * scale32, -clip), clip) per column, each operation rounded on its own; clip <= 0
+ * means no clamp.  out may be x. */
+int64_t ddrl_obs_moments_ws_bytes(int B, int D);
+int ddrl_obs_moments(const float* x, int B, int D, const double* shift, double* sums, void* ws, int64_t ws_bytes, void* stream);
+int ddrl_obs_rms_update(double* mean, double* var, double* count, const double* sums, double n, int D, float* mean32,
+                        float* scale32, void* stream);
+int ddrl_obs_normalize(const float* x, int B, int D, const float* mean32, const float* scale32, float clip, float* out,
+                       void* stream);
+
 /* Value loss of ONE extra critic head (nn/ppo.py:97-104: rndv_loss / gailv_loss = vlossf(data.values[k], values[k])):
  * dv[b] = d(loss)/d(v[b]) (times v_coef when shared, ppo.py:108), loss_sums[1] += contribution scaled by inv_B_global. */
 int ddrl_value_loss(const float* returns, const float* v, int B, float inv_B_global, const ddrl_ppo_hparams* hp,
