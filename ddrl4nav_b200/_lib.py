@@ -72,12 +72,17 @@ SIGNATURES = {
                                         _P]),
     "ddrl_ppo_loss_gaussian_v": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P, _P,
                                      _P, _P]),
-    "ddrl_adv_moments": (_I, [_P, _I, _P, _P]),
+    "ddrl_ppo_loss_categorical_vn": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P,
+                                          _P, _P, _P]),
+    "ddrl_ppo_loss_gaussian_vn": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P,
+                                       _P, _P, _P, _P]),
+    "ddrl_adv_moments":(_I, [_P, _I, _P, _P]),
     "ddrl_adv_normalize": (_I, [_P, _I, _P, _F, _P, _P]),
     "ddrl_obs_moments_ws_bytes": (_L, [_I, _I]),
     "ddrl_obs_moments": (_I, [_P, _I, _I, _P, _P, _P, _L, _P]),
     "ddrl_obs_rms_update": (_I, [_P, _P, _P, _P, C.c_double, _I, _P, _P, _P]),
     "ddrl_obs_normalize": (_I, [_P, _I, _I, _P, _P, _F, _P, _P]),
+    "ddrl_value_norm_update": (_I, [_P, _P, _P, _P, C.c_double, _P, _P, _P, _I, _P]),
     "ddrl_value_loss": (_I, [_P, _P, _I, _F, C.POINTER(PPOHparams), _I, _P, _P, _P]),
     "ddrl_clip_adam": (_I, [_P, _P, _P, _P, _L, C.POINTER(_L), C.POINTER(_F), _I, _I, C.POINTER(PPOHparams), _P, _P]),
     "ddrl_gemm_f32": (_I, [_I, _I, _I, _I, _I, _P, _I, _P, _I, _P, _I, _P, _I, _I, _P]),
@@ -92,6 +97,7 @@ SIGNATURES = {
     "ddrl_net_set_extra_critics": (_I, [_P, _I, C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_I)]),
     "ddrl_net_num_obs": (_I, [_P]),
     "ddrl_net_obs_elems": (_L, [_P, _I]),
+    "ddrl_net_set_value_norm": (_I, [_P, _P]),
     "ddrl_net_forward": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P, _P, _P, _P]),
     "ddrl_net_encode": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P]),
     "ddrl_net_backward": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _I, _P]),

@@ -111,6 +111,9 @@ struct ddrl_net {
   struct ExtraCritic { const float *w, *b; float *dw, *db; int in_loss; };
   std::vector<ExtraCritic> extra;
   float *vout_x = nullptr, *dv_x = nullptr;    // [kMaxExtra, MB]
+  // NORM_VALUE (ddrl_net_set_value_norm): device {mean32, scale32, sigma32}; critic 0 learns normalised targets and the
+  // forward pass returns its values denormalised.  Null: off.
+  const float* value_norm = nullptr;
   char* packed_base = nullptr;   // packed weights + packed grads arena
   char* split_base = nullptr;    // tc2 engine: [hi mirror of the packed arena | lo mirror]
   size_t packed_bytes = 0, packed_grad_off = 0, packed_grad_bytes = 0;
@@ -1653,6 +1656,21 @@ extern "C" int64_t ddrl_net_obs_elems(const ddrl_net* n, int slot) {
 }
 extern "C" int64_t ddrl_net_workspace_bytes(const ddrl_net* n) { return n ? (int64_t)(n->ws.cap + n->packed_bytes) : 0; }
 
+namespace ddrl {
+// NORM_VALUE: critic 0's values in reward units, v * sigma32 + mean32 with two roundings (no fma), as torch computes it
+__global__ void __launch_bounds__(256) value_denorm_kernel(const float* __restrict__ v, int n, const float* __restrict__ applied,
+                                                           float* __restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = __fadd_rn(__fmul_rn(v[i], applied[2]), applied[0]);
+}
+}  // namespace ddrl
+
+extern "C" int ddrl_net_set_value_norm(ddrl_net* n, const float* applied) {
+  if (!n) return DDRL_E_ARG;
+  n->value_norm = applied;
+  return DDRL_OK;
+}
+
 extern "C" int ddrl_net_forward(ddrl_net* n, const float* const* obs, int n_obs, int B, const float* draw, float* actions,
                                 float* logp, float* values, float* pi_out, void* stream) {
   if (!n || B < 0) return DDRL_E_ARG;
@@ -1677,7 +1695,12 @@ extern "C" int ddrl_net_forward(ddrl_net* n, const float* const* obs, int n_obs,
       TRY(ddrl_gaussian_head(n->logits, n->ldA, ls, draw ? draw + r0 * A : nullptr, mb, A, actions + r0 * A, logp + r0, s));
       if (pi_out) TRY(copy2d(n->logits, n->ldA, pi_out + r0 * A, A, mb, A, s));
     }
-    DDRL_CUDA(cudaMemcpyAsync(values + r0, n->vout, sizeof(float) * mb, cudaMemcpyDeviceToDevice, s));
+    if (n->value_norm) {
+      value_denorm_kernel<<<ceil_div(mb, 256), 256, 0, s>>>(n->vout, mb, n->value_norm, values + r0);
+      DDRL_LAUNCHED("value_denorm_kernel");
+    } else {
+      DDRL_CUDA(cudaMemcpyAsync(values + r0, n->vout, sizeof(float) * mb, cudaMemcpyDeviceToDevice, s));
+    }
     for (size_t k = 0; k < n->extra.size(); ++k)     // values is [1 + extras, B]
       DDRL_CUDA(cudaMemcpyAsync(values + (k + 1) * (size_t)B + r0, n->vout_x + k * (size_t)n->MB, sizeof(float) * mb,
                                 cudaMemcpyDeviceToDevice, s));
@@ -1730,14 +1753,14 @@ static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int 
     amax_new_pass(n, s, reuse_obs);
     TRY(forward_chunk(n, obs, r0, mb, true, s, reuse_obs));
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
-      TRY(ddrl_ppo_loss_categorical_v(n->logits, n->ldA, actions + r0, old_logp + r0, adv + r0, returns + r0, n->vout, mb, A,
-                                      invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
-                                      old_values ? old_values + r0 : nullptr, stats, s));
+      TRY(ddrl_ppo_loss_categorical_vn(n->logits, n->ldA, actions + r0, old_logp + r0, adv + r0, returns + r0, n->vout, mb, A,
+                                       invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
+                                       old_values ? old_values + r0 : nullptr, stats, n->value_norm, s));
     } else {
-      TRY(ddrl_ppo_loss_gaussian_v(n->logits, n->ldA, n->params + n->T[n->t_logstd].offset, actions + r0 * A, old_logp + r0,
-                                   adv + r0, returns + r0, n->vout, mb, A, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv,
-                                   n->grads + n->T[n->t_logstd].offset, loss_sums, old_values ? old_values + r0 : nullptr, stats,
-                                   s));
+      TRY(ddrl_ppo_loss_gaussian_vn(n->logits, n->ldA, n->params + n->T[n->t_logstd].offset, actions + r0 * A, old_logp + r0,
+                                    adv + r0, returns + r0, n->vout, mb, A, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv,
+                                    n->grads + n->T[n->t_logstd].offset, loss_sums, old_values ? old_values + r0 : nullptr, stats,
+                                    n->value_norm, s));
     }
     // heads backward (nn/actor.py:91 actor_linear, nn/critic.py:21 critic_linear)
     TRY(skinny_wgrad(n->dlogits, n->ldA, ta.h, F, mb, A, F, n->grads + n->T[n->t_aw].offset, n->grads + n->T[n->t_ab].offset, s));
@@ -1783,7 +1806,7 @@ static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_
   TRY(check_obs(n, obs, n_obs));
   if (!actions || !old_logp || !adv || !returns) return DDRL_E_ARG;
   const std::string key = graph_key("bwd", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, actions, old_logp,
-                                            adv, returns, old_values, n->params, n->grads, n->ws.base},
+                                            adv, returns, old_values, n->value_norm, n->params, n->grads, n->ws.base},
                                     {B_local, B_global}, hp, sizeof(*hp));
   auto launch_seg = [&](ddrl_net::GraphEntry* e, int k) {
     const int pre = (int)e->pre_execs.size();
@@ -1839,7 +1862,7 @@ extern "C" int ddrl_net_backward_segment(ddrl_net* n, const float* const* obs, i
                                          const float* actions, const float* old_logp, const float* adv, const float* returns,
                                          const ddrl_ppo_hparams* hp, int obs_unchanged, int segment, int* n_segments,
                                          void* stream) {
-  if (segment < 0 || !n_segments) return DDRL_E_ARG;
+  if (segment < 0 || !n_segments || (n && n->value_norm)) return DDRL_E_ARG;
   return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, nullptr, hp, obs_unchanged, segment,
                        n_segments, (cudaStream_t)stream);
 }
@@ -1869,7 +1892,8 @@ extern "C" int ddrl_net_backward_minibatch_v(ddrl_net* n, const float* const* ob
   };
   if (B_local > n->MB || !n->extra.empty() || !graphs_enabled(n) || n->mb_graphs_off) return body(s);
   const std::string key = graph_key("bwd_mb", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, actions,
-                                               old_logp, adv, returns, old_values, n->params, n->grads, n->ws.base},
+                                               old_logp, adv, returns, old_values, n->value_norm, n->params, n->grads,
+                                               n->ws.base},
                                     {B_local, B_global}, hp, sizeof(*hp));
   if (std::find(n->mb_seen.begin(), n->mb_seen.end(), key) == n->mb_seen.end()) {
     if (n->mb_seen.size() >= 16) n->mb_seen.erase(n->mb_seen.begin());

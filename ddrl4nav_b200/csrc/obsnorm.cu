@@ -4,6 +4,10 @@
 //   ddrl_obs_rms_update   Chan's parallel merge of one batch into the running {mean, var, count}, then the applied form
 //                         mean32 = fp32(mean), scale32 = fp32(1 / sqrt(var + 1e-8))
 //   ddrl_obs_normalize    out = min(max((x - mean32) * scale32, -clip), clip)
+//   ddrl_value_norm_update  the same merge for critic 0's return targets (non-reference option NORM_VALUE, one column), the
+//                         applied form {mean32, scale32, sigma32 = fp32(sqrt(var + 1e-8))}, and the PopArt rescale of critic
+//                         0's head that keeps its unnormalised outputs: W' = W sigma_old / sigma_new,
+//                         b' = (sigma_old b + mean_old - mean_new) / sigma_new
 //
 // The statistics must be the same bits on every data-parallel rank and in every predictor, so the moments use a reduction
 // order that depends on (B, D) only: rows are cut into fixed chunks of kMomChunkRows, each block sums one chunk of one column
@@ -25,6 +29,7 @@ constexpr int kMomUnroll = 4;
 constexpr int kNormThreads = 256;
 constexpr int kNormUnroll = 4;
 constexpr int kRmsThreads = 1024;
+constexpr int kValueNormThreads = 512;               // one thread per weight of a 512-wide critic head
 
 inline int64_t obs_moment_chunks(int B) { return B > 0 ? ceil_div64(B, kMomChunkRows) : 0; }
 
@@ -107,6 +112,15 @@ __global__ void __launch_bounds__(256) obs_moments_reduce_kernel(const double* _
   }
 }
 
+// Chan's merge of one column's batch of n rows, given as the sums s1 = sum d and s2 = sum d^2 of d = x - m, into the running
+// (m, v) of count c; tot = c + n.  Shared by the observation and the value-target statistics.
+__device__ __forceinline__ void rms_merge(double& m, double& v, double c, double n, double tot, double s1, double s2) {
+  const double delta = s1 / n;                                   // batch mean - running mean (the sums are shifted by it)
+  const double bvar = fmax(s2 / n - delta * delta, 0.0);         // population variance of the batch
+  m = m + delta * n / tot;
+  v = (v * c + bvar * n + delta * delta * c * n / tot) / tot;
+}
+
 // ONE block: every thread reads the count before thread 0 rewrites it
 __global__ void __launch_bounds__(kRmsThreads) obs_rms_update_kernel(double* __restrict__ mean, double* __restrict__ var,
                                                                      double* __restrict__ count, const double* __restrict__ sums,
@@ -117,10 +131,7 @@ __global__ void __launch_bounds__(kRmsThreads) obs_rms_update_kernel(double* __r
   for (int j = threadIdx.x; j < D; j += blockDim.x) {
     double m = mean[j], v = var[j];
     if (n > 0.0) {
-      const double delta = sums[j] / n;                            // batch mean - running mean (the sums are shifted by it)
-      const double bvar = fmax(sums[D + j] / n - delta * delta, 0.0);   // population variance of the batch
-      m = m + delta * n / tot;
-      v = (v * c + bvar * n + delta * delta * c * n / tot) / tot;
+      rms_merge(m, v, c, n, tot, sums[j], sums[D + j]);
       mean[j] = m;
       var[j] = v;
     }
@@ -129,6 +140,35 @@ __global__ void __launch_bounds__(kRmsThreads) obs_rms_update_kernel(double* __r
   }
   __syncthreads();
   if (n > 0.0 && threadIdx.x == 0) *count = tot;
+}
+
+// NORM_VALUE, ONE block: every thread merges the single column redundantly (same bits), rescales its share of the head's
+// weights, and the threads wait for each other before thread 0 rewrites the state.  The head arithmetic and the applied form
+// use the correctly rounded intrinsics (no contraction into fma), so torch's float64 reproduces them to the bit.
+__global__ void __launch_bounds__(kValueNormThreads) value_norm_update_kernel(double* __restrict__ mean, double* __restrict__ var,
+                                                                              double* __restrict__ count,
+                                                                              const double* __restrict__ sums, double n,
+                                                                              float* __restrict__ applied, float* __restrict__ w,
+                                                                              float* __restrict__ b, int F) {
+  const double c = *count, m_old = *mean, v_old = *var;
+  double m = m_old, v = v_old;
+  if (n > 0.0) rms_merge(m, v, c, n, c + n, sums[0], sums[1]);
+  const double s_old = __dsqrt_rn(__dadd_rn(v_old, 1e-8)), s_new = __dsqrt_rn(__dadd_rn(v, 1e-8));
+  const bool rescale = n > 0.0 && w;
+  if (rescale)
+    for (int j = threadIdx.x; j < F; j += blockDim.x) w[j] = (float)__ddiv_rn(__dmul_rn((double)w[j], s_old), s_new);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    if (rescale) *b = (float)__ddiv_rn(__dsub_rn(__dadd_rn(__dmul_rn(s_old, (double)*b), m_old), m), s_new);
+    if (n > 0.0) {
+      *mean = m;
+      *var = v;
+      *count = c + n;
+    }
+    applied[0] = (float)m;
+    applied[1] = (float)__ddiv_rn(1.0, s_new);
+    applied[2] = (float)s_new;
+  }
 }
 
 // grid (column groups, row stripes); each thread keeps its columns' mean / scale in registers and walks rows y, y + gridDim.y, ...
@@ -225,6 +265,16 @@ extern "C" int ddrl_obs_rms_update(double* mean, double* var, double* count, con
   prof_work(8.0 * 5 * D);
   obs_rms_update_kernel<<<1, kRmsThreads, 0, (cudaStream_t)stream>>>(mean, var, count, sums, n, D, mean32, scale32);
   DDRL_LAUNCHED("obs_rms_update_kernel");
+  return DDRL_OK;
+}
+
+extern "C" int ddrl_value_norm_update(double* mean, double* var, double* count, const double* sums, double n, float* applied,
+                                      float* head_w, float* head_b, int F, void* stream) {
+  if (!mean || !var || !count || !applied || !(n >= 0.0) || (n > 0.0 && !sums)) return DDRL_E_ARG;
+  if ((head_w == nullptr) != (head_b == nullptr) || (head_w && F < 1)) return DDRL_E_ARG;
+  prof_work(8.0 * 5 + (head_w ? 8.0 * F : 0.0));
+  value_norm_update_kernel<<<1, kValueNormThreads, 0, (cudaStream_t)stream>>>(mean, var, count, sums, n, applied, head_w, head_b, F);
+  DDRL_LAUNCHED("value_norm_update_kernel");
   return DDRL_OK;
 }
 

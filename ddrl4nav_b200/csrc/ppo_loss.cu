@@ -19,6 +19,8 @@
 //          (clamp passes the gradient on the closed interval, max splits ties 1/2-1/2 as torch.max does).
 //   stats: stats[0] += inv_B*((r - 1) - log r) (approx KL), stats[1] += inv_B*[|r - 1| > ppo_clip] (clip fraction), through
 //          the same ordered / atomic adds as the loss sums.
+//   value_norm (in LossParams): critic 0 learns normalised targets R~ = (R - mean32) * scale32, and old_v is normalised the same
+//          way, each operation rounded on its own; the extra critics' value_loss_kernel never normalises.
 #include "common.cuh"
 
 namespace ddrl {
@@ -31,6 +33,7 @@ constexpr int kMaxAL = 64;
 struct LossParams {
   float ppo_clip, dual_clip, v_coef, ent_coef, inv_B, value_clip;
   int smooth_l1, shared;
+  const float* value_norm;        // NORM_VALUE: device {mean32, scale32, sigma32} of critic 0's targets, or null
 };
 
 // d(term)/d(ratio) of term = A>0 ? s : max(s, dual*A), s = min(ratio*A, clamp(ratio)*A); also returns term
@@ -63,13 +66,20 @@ __device__ __forceinline__ float value_loss(float R, float v, int smooth_l1, flo
   return az - 0.5f;
 }
 
-// value loss of critic 0 and its d/dv, clipped around old_v when old_v is given (c = clip width)
+// value loss of critic 0 and its d/dv, clipped around old_v when old_v is given (c = clip width); with value_norm the target and
+// the old value are normalised first
 __device__ __forceinline__ float value_loss_clipped(float R, float v, const float* __restrict__ old_v, int b, float c,
-                                                    int smooth_l1, float* dl_dv) {
+                                                    int smooth_l1, const float* __restrict__ value_norm, float* dl_dv) {
+  float mean32 = 0.f, scale32 = 0.f;
+  if (value_norm) {
+    mean32 = value_norm[0];
+    scale32 = value_norm[1];
+    R = __fmul_rn(__fsub_rn(R, mean32), scale32);
+  }
   float dl;
   const float lu = value_loss(R, v, smooth_l1, &dl);
   if (!old_v) { *dl_dv = dl; return lu; }
-  const float vo = old_v[b];
+  const float vo = value_norm ? __fmul_rn(__fsub_rn(old_v[b], mean32), scale32) : old_v[b];
   const float d = v - vo;
   const float vc = vo + fminf(fmaxf(d, -c), c);
   float dlc;
@@ -139,7 +149,7 @@ __global__ void __launch_bounds__(128) ppo_loss_categorical_kernel(
     float* dx = dlogits + (size_t)b * ld_d;
     for (int j = 0; j < A; ++j) dx[j] = p[j] * (gq[j] - dot_p);
     float dl;
-    l_v = value_loss_clipped(returns[b], v[b], old_v, b, hp.value_clip, hp.smooth_l1, &dl) * hp.inv_B;
+    l_v = value_loss_clipped(returns[b], v[b], old_v, b, hp.value_clip, hp.smooth_l1, hp.value_norm, &dl) * hp.inv_B;
     dv[b] = dl * hp.inv_B * (hp.shared ? hp.v_coef : 1.f);
   }
   l_actor = block_sum(l_actor, scratch);
@@ -204,7 +214,7 @@ __global__ void __launch_bounds__(128) ppo_loss_gaussian_kernel(
       if (j < 8) dls[j] = g;
     }
     float dl;
-    l_v = value_loss_clipped(returns[b], v[b], old_v, b, hp.value_clip, hp.smooth_l1, &dl) * hp.inv_B;
+    l_v = value_loss_clipped(returns[b], v[b], old_v, b, hp.value_clip, hp.smooth_l1, hp.value_norm, &dl) * hp.inv_B;
     dv[b] = dl * hp.inv_B * (hp.shared ? hp.v_coef : 1.f);
   }
   l_actor = block_sum(l_actor, scratch);
@@ -249,10 +259,10 @@ __global__ void __launch_bounds__(128) value_loss_kernel(const float* __restrict
   }
 }
 
-static LossParams make_params(const ddrl_ppo_hparams* hp, float inv_B, int shared) {
+static LossParams make_params(const ddrl_ppo_hparams* hp, float inv_B, int shared, const float* value_norm = nullptr) {
   LossParams p;
   p.ppo_clip = hp->ppo_clip; p.dual_clip = hp->dual_clip; p.v_coef = hp->v_coef; p.ent_coef = hp->ent_coef;
-  p.inv_B = inv_B; p.value_clip = hp->value_clip; p.smooth_l1 = hp->smooth_l1; p.shared = shared;
+  p.inv_B = inv_B; p.value_clip = hp->value_clip; p.smooth_l1 = hp->smooth_l1; p.shared = shared; p.value_norm = value_norm;
   return p;
 }
 
@@ -265,21 +275,30 @@ static bool value_clip_args_ok(const ddrl_ppo_hparams* hp, const float* old_valu
   return old_values ? hp->value_clip > 0.f : !(hp->value_clip > 0.f);
 }
 
-extern "C" int ddrl_ppo_loss_categorical_v(const float* logits, int ld, const float* actions, const float* old_logp,
-                                           const float* adv, const float* returns, const float* v, int B, int A,
-                                           float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dlogits,
-                                           int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
-                                           void* stream) {
+extern "C" int ddrl_ppo_loss_categorical_vn(const float* logits, int ld, const float* actions, const float* old_logp,
+                                            const float* adv, const float* returns, const float* v, int B, int A,
+                                            float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dlogits,
+                                            int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
+                                            const float* value_norm, void* stream) {
   if (B < 0 || A < 1 || A > kMaxAL || ld < A || ld_d < A || !hp) return DDRL_E_ARG;
   if (!value_clip_args_ok(hp, old_values)) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!logits || !actions || !old_logp || !adv || !returns || !v || !dlogits || !dv || !loss_sums) return DDRL_E_ARG;
   ppo_loss_categorical_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(
-      logits, ld, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared), dlogits, ld_d, dv,
-      loss_sums, old_values, stats, det_seq(1));
+      logits, ld, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared, value_norm), dlogits, ld_d,
+      dv, loss_sums, old_values, stats, det_seq(1));
   prof_work((8.0 * A + 24.0 + (old_values ? 4.0 : 0.0)) * B);
   DDRL_LAUNCHED("ppo_loss_categorical_kernel");
   return DDRL_OK;
+}
+
+extern "C" int ddrl_ppo_loss_categorical_v(const float* logits, int ld, const float* actions, const float* old_logp,
+                                           const float* adv, const float* returns, const float* v, int B, int A,
+                                           float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dlogits,
+                                           int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
+                                           void* stream) {
+  return ddrl_ppo_loss_categorical_vn(logits, ld, actions, old_logp, adv, returns, v, B, A, inv_B_global, hp, shared, dlogits,
+                                      ld_d, dv, loss_sums, old_values, stats, nullptr, stream);
 }
 
 extern "C" int ddrl_ppo_loss_categorical(const float* logits, int ld, const float* actions, const float* old_logp,
@@ -302,22 +321,31 @@ extern "C" int ddrl_value_loss(const float* returns, const float* v, int B, floa
   return DDRL_OK;
 }
 
-extern "C" int ddrl_ppo_loss_gaussian_v(const float* mu, int ld, const float* log_std, const float* actions,
-                                        const float* old_logp, const float* adv, const float* returns, const float* v,
-                                        int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
-                                        float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums,
-                                        const float* old_values, float* stats, void* stream) {
+extern "C" int ddrl_ppo_loss_gaussian_vn(const float* mu, int ld, const float* log_std, const float* actions,
+                                         const float* old_logp, const float* adv, const float* returns, const float* v,
+                                         int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                                         float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums,
+                                         const float* old_values, float* stats, const float* value_norm, void* stream) {
   if (B < 0 || A < 1 || A > 8 || ld < A || ld_d < A || !hp) return DDRL_E_ARG;
   if (!value_clip_args_ok(hp, old_values)) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!mu || !log_std || !actions || !old_logp || !adv || !returns || !v || !dmu || !dv || !dlog_std || !loss_sums)
     return DDRL_E_ARG;
   ppo_loss_gaussian_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(
-      mu, ld, log_std, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared), dmu, ld_d, dv,
-      dlog_std, loss_sums, old_values, stats, det_seq(1));
+      mu, ld, log_std, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared, value_norm), dmu, ld_d,
+      dv, dlog_std, loss_sums, old_values, stats, det_seq(1));
   prof_work((12.0 * A + 20.0 + (old_values ? 4.0 : 0.0)) * B);
   DDRL_LAUNCHED("ppo_loss_gaussian_kernel");
   return DDRL_OK;
+}
+
+extern "C" int ddrl_ppo_loss_gaussian_v(const float* mu, int ld, const float* log_std, const float* actions,
+                                        const float* old_logp, const float* adv, const float* returns, const float* v,
+                                        int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                                        float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums,
+                                        const float* old_values, float* stats, void* stream) {
+  return ddrl_ppo_loss_gaussian_vn(mu, ld, log_std, actions, old_logp, adv, returns, v, B, A, inv_B_global, hp, shared, dmu,
+                                   ld_d, dv, dlog_std, loss_sums, old_values, stats, nullptr, stream);
 }
 
 extern "C" int ddrl_ppo_loss_gaussian(const float* mu, int ld, const float* log_std, const float* actions,

@@ -77,7 +77,9 @@ def global_moments(m3: torch.Tensor, group=None) -> torch.Tensor:
 def global_obs_sums(sums: torch.Tensor, group=None) -> torch.Tensor:
     """In-place sum over ranks of the float64 observation moments of every normalised slot, concatenated into ONE buffer
     (kernels.obs_moments, NORM_OBS): every rank shifts by the same running mean, so the sums add, and every rank then merges
-    the same global batch into its statistics.  One collective per learn call."""
+    the same global batch into its statistics.  With NORM_VALUE the two sums of critic 0's return targets follow the
+    observation sums in the same buffer (nn/obs_rms.share_sums), or are the whole buffer without NORM_OBS.  One collective per
+    learn call."""
     import torch.distributed as dist
     _, ws = world(group)
     if ws > 1:

@@ -338,6 +338,32 @@ def obs_rms_update(mean: torch.Tensor, var: torch.Tensor, count: torch.Tensor, s
                                           ptr(mean32), ptr(scale32), current_stream()), "ddrl_obs_rms_update")
 
 
+def value_norm_update(mean: torch.Tensor, var: torch.Tensor, count: torch.Tensor, sums: Optional[torch.Tensor], n: float,
+                      applied: torch.Tensor, head_w: Optional[torch.Tensor] = None, head_b: Optional[torch.Tensor] = None) -> None:
+    """NORM_VALUE (ddrl_value_norm_update, one launch): merges the batch of `n` return targets whose moments (obs_moments with
+    D = 1 around `mean`) are `sums` into the float64 [1] {mean, var, count} in place, writes applied [3] = {mean32, scale32,
+    sigma32}, and, given critic 0's head (fp32 weight [F] and bias [1], e.g. views into the flat parameter buffer), rescales it
+    in place so that its unnormalised outputs are kept.  n = 0: the applied form only."""
+    dev = mean.device
+    require_cuda(mean)
+    for t, what in ((mean, "mean"), (var, "var"), (count, "count")):
+        _f64_vec(t, 1, dev, "value_norm_update: " + what)
+    if n > 0:
+        _f64_vec(sums, 2, dev, "value_norm_update: sums")
+    if applied.dtype != torch.float32 or applied.numel() != 3 or not applied.is_contiguous() or applied.device != dev:
+        raise DDRLError("value_norm_update: applied must be a contiguous fp32 [3] tensor on %s" % dev)
+    if (head_w is None) != (head_b is None):
+        raise DDRLError("value_norm_update: give both head_w and head_b, or neither")
+    F = 0
+    if head_w is not None:
+        for t, k, what in ((head_w, head_w.numel(), "head_w"), (head_b, 1, "head_b")):
+            if t.dtype != torch.float32 or t.numel() != k or k < 1 or not t.is_contiguous() or t.device != dev:
+                raise DDRLError("value_norm_update: %s must be a contiguous fp32 tensor on %s (bias: one element)" % (what, dev))
+        F = head_w.numel()
+    check(_lib.load().ddrl_value_norm_update(ptr(mean), ptr(var), ptr(count), ptr(sums) if n > 0 else None, float(n), ptr(applied),
+                                             ptr(head_w), ptr(head_b), F, current_stream()), "ddrl_value_norm_update")
+
+
 def obs_normalize(x: torch.Tensor, mean32: torch.Tensor, scale32: torch.Tensor, clip: Optional[float],
                   out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """clamp((x - mean32) * scale32, -clip, clip) per column of x read as [B, D] (D = mean32.numel()); clip None: no clamp

@@ -86,8 +86,11 @@ class ObsRMS(torch.nn.Module):
         key = self._key()
         if key != self._applied:
             for s in self.slots:
-                kernels.obs_rms_update(*self.state(s), None, 0.0, *self.applied(s))
+                self._rewrite_applied(s)
             self._applied = key
+
+    def _rewrite_applied(self, s):
+        kernels.obs_rms_update(*self.state(s), None, 0.0, *self.applied(s))
 
     def normalize(self, s, x, out):
         mean32, scale32 = self.applied(s)
@@ -146,3 +149,67 @@ class ObsRMS(torch.nn.Module):
                 a_mean.copy_(m32)
                 a_scale.copy_(s32)
         self._applied = self._key()
+
+
+class ValueRMS(ObsRMS):
+    """Running statistics of critic 0's return targets (non-reference option NORM_VALUE of ``PPO``, PopArt): float64 buffers
+    ``mean``, ``var`` and ``count`` of shape [1] with the same gym conventions, and the non-persistent fp32 applied form
+    ``applied`` [3] = {mean32, scale32 = fp32(1 / sigma), sigma32 = fp32(sigma)}, sigma = sqrt(var + 1e-8).  Critic 0 learns
+    (R - mean32) * scale32 and the Forward module returns its values as v * sigma32 + mean32.  One column of ObsRMS: the
+    moments, the workspace and the refresh by buffer version are ObsRMS's; the merge also rescales the head
+    (kernels.value_norm_update)."""
+
+    def __init__(self):
+        super().__init__((0,), None)
+        self.register_buffer("mean", torch.zeros(1, dtype=torch.float64))
+        self.register_buffer("var", torch.ones(1, dtype=torch.float64))
+        self.register_buffer("count", torch.full((1,), 1e-4, dtype=torch.float64))
+
+    def state(self, s=0):
+        return self.mean, self.var, self.count
+
+    def applied(self, s=0):
+        return self.applied32
+
+    def bind(self, dev):
+        """Moves the statistics to `dev` and creates the applied form and the moment sums there."""
+        for name in ("mean", "var", "count"):
+            self.register_buffer(name, getattr(self, name).to(device=dev, dtype=torch.float64).contiguous())
+        self.register_buffer("applied32", torch.empty(3, dtype=torch.float32, device=dev), persistent=False)
+        self.slots, self.dims = (0,), {0: 1}
+        self.sums = torch.zeros(2, dtype=torch.float64, device=dev)
+        self._ws = None
+        self._applied = None
+
+    def _rewrite_applied(self, s):
+        kernels.value_norm_update(*self.state(), None, 0.0, self.applied32)
+
+    def merge(self, n, head_w, head_b):
+        """Folds the `n` targets whose moments are in self.sums into the statistics, rewrites the applied form and rescales
+        critic 0's head (head_w [F], head_b [1]) in place so that its unnormalised outputs are kept."""
+        kernels.value_norm_update(*self.state(), self.sums, float(n), self.applied32, head_w, head_b)
+
+    def records(self):
+        """[mean32, scale32, sigma32, count] as ONE fp32 array (one device-to-host copy)."""
+        self.refresh()
+        return [torch.cat([self.applied32, self.count.float()]).cpu().numpy()]
+
+    def load_records(self, rec):
+        """Sets the applied form bit-exactly from the record [mean32, scale32, sigma32, count], and the float64 state to
+        (mean32, sigma32^2 - 1e-8, count): an approximation of the learner's state, enough to act with."""
+        r = torch.from_numpy(np.ascontiguousarray(rec, dtype=np.float32)).to(self.mean.device)
+        with torch.no_grad():
+            self.applied32.copy_(r[:3])
+            self.mean.copy_(r[0:1].double())
+            self.var.copy_(r[2:3].double() ** 2 - 1e-8)
+            self.count.copy_(r[3:4].double())
+        self._applied = self._key()
+
+
+def share_sums(obs_rms, value_rms):
+    """Points the moment sums of both statistics into ONE float64 buffer, the observation sums followed by the two value sums,
+    so that a data-parallel learner sums both over its ranks with one collective; returns that buffer."""
+    n = obs_rms.sums.numel()
+    buf = torch.zeros(n + 2, dtype=torch.float64, device=obs_rms.sums.device)
+    obs_rms.sums, value_rms.sums = buf[:n], buf[n:]
+    return buf

@@ -30,7 +30,7 @@ from torch.distributions.normal import Normal
 from .. import _lib, dist, kernels
 from .._lib import DDRLError, NetDesc, check, current_stream, ptr
 from .base import Basenn
-from .obs_rms import ObsRMS
+from .obs_rms import ObsRMS, ValueRMS, share_sums
 
 
 def _on_device(fn):
@@ -108,6 +108,11 @@ class PPO(Basenn):
         self._obs_act = {}              # NORM_OBS: per slot, the act / encode scratch (grows with B)
         self._obs_learn = {}            # NORM_OBS: per slot, the learner's persistent normalised batch
         self._obs_n = 0                 # NORM_OBS: rows of the global batch of the current learn call
+        # value-target normalisation (non-reference, off by default; PopArt): float64 statistics of critic 0's return targets in
+        # the submodule value_rms (state_dict keys value_rms.{mean,var,count}); critic 0 learns normalised targets and act /
+        # forward return its values denormalised
+        self.value_rms = ValueRMS() if _flag_option(config_nn, "NORM_VALUE") else None
+        self._norm_sums = None          # NORM_VALUE: the float64 moment sums a data-parallel learner all-reduces (+ NORM_OBS's)
         self.hp = kernels.make_hparams(
             ppo_clip=_cfg(config_nn, "PPO_CLIP", 0.2), dual_clip=_cfg(config_nn, "DUEL_PPO_CLIP", 3),
             v_coef=_cfg(config_nn, "V_LOSS_THETA", 1.0), ent_coef=_cfg(config_nn, "ENTROPY_LOSS_THETA", 0.05),
@@ -276,6 +281,10 @@ class PPO(Basenn):
             except DDRLError:
                 self._destroy()
                 raise
+        if self.value_rms is not None:
+            self.value_rms.bind(dev)
+            self._norm_sums = self.value_rms.sums if self.obs_rms is None else share_sums(self.obs_rms, self.value_rms)
+            check(lib.ddrl_net_set_value_norm(h, ptr(self.value_rms.applied32)), "ddrl_net_set_value_norm")
         nt = lib.ddrl_net_num_tensors(h)
         P = lib.ddrl_net_num_params(h)
         if nt != len(plist):
@@ -341,18 +350,33 @@ class PPO(Basenn):
 
     @_on_device
     def _state_records(self):
-        """NORM_OBS: per normalised slot, in slot order, the records mean32 [D], scale32 [D] and count [1] after the
-        parameters, so that a predictor loading the blob acts with exactly the learner's applied form."""
-        if self.obs_rms is None:
+        """After the parameters, so that a predictor loading the blob acts with exactly the learner's applied forms:
+        NORM_OBS: per normalised slot, in slot order, the records mean32 [D], scale32 [D] and count [1];
+        NORM_VALUE: then one record [4] = {mean32, scale32, sigma32, count}."""
+        if self.obs_rms is None and self.value_rms is None:
             return []
         self._ensure_engine()
-        return self.obs_rms.records()
+        recs = self.obs_rms.records() if self.obs_rms is not None else []
+        return recs + (self.value_rms.records() if self.value_rms is not None else [])
 
     @_on_device
     def _load_state_records(self, view):
-        if self.obs_rms is None:
+        if self.obs_rms is None and self.value_rms is None:
             return
         self._ensure_engine()
+        index = self._load_obs_records(view) if self.obs_rms is not None else 0
+        if self.value_rms is not None:
+            try:
+                wb, _ = self._decode_wb(view[index:])
+            except (struct.error, ValueError):
+                wb = None
+            if wb is None or wb.shape != (4,):
+                raise DDRLError("model blob has no NORM_VALUE record [4] after the parameters%s (written by a net without "
+                                "NORM_VALUE?)" % (" and the NORM_OBS records" if self.obs_rms is not None else ""))
+            self.value_rms.load_records(wb)
+
+    def _load_obs_records(self, view):
+        """Reads the NORM_OBS records at the start of `view`; returns the bytes they take."""
         rms, recs, index = self.obs_rms, [], 0
         for s in rms.slots:
             got = []
@@ -368,6 +392,7 @@ class PPO(Basenn):
                 index += used
             recs.append(got)
         rms.load_records(recs)
+        return index
 
     def flat_grads(self):
         """View of the flat gradient buffer (reference parameter order) of the last backward."""
@@ -430,6 +455,8 @@ class PPO(Basenn):
         lib = _lib.load()
         if self.obs_rms is not None:
             states = self._normalized_obs(states, self._obs_act)
+        if self.value_rms is not None:
+            self.value_rms.refresh()
         keep, arr, n_obs, B = self._obs_ptrs(states)
         dev = self._flat.device
         A = self.actor.actor_linear.out_features
@@ -581,6 +608,8 @@ class PPO(Basenn):
         This is the engine-level pass: with NORM_OBS it takes `states` as given, so they must already be normalised."""
         self._ensure_engine()
         lib = _lib.load()
+        if self.value_rms is not None:
+            self.value_rms.refresh()
         args, held, B = self._bwd_args(states, advs, actions, old_logps, returns, b_global, obs_unchanged, minibatch)
         keep, rows = held[0], held[-1]
         dev = self._flat.device
@@ -694,7 +723,9 @@ class PPO(Basenn):
         PPO_STATS adds ApproxKL and ClipFrac to every dict; with TARGET_KL the call ends after the first step whose ApproxKL
         exceeds the target (that step is applied and yielded).
         NORM_OBS: every step sees the observations normalised with the statistics held when the call started (those the
-        Forward module acted with); the call's batch is folded into the statistics once, before the final step's yield."""
+        Forward module acted with); the call's batch is folded into the statistics once, before the final step's yield.
+        NORM_VALUE: the call's return targets are folded into critic 0's target statistics once, at the start, and the head
+        is rescaled to keep its outputs; every step then learns the targets normalised with the new statistics (PopArt)."""
         if self.mini_batch_num > 1:
             yield from self._learn_minibatch(data)
             return
@@ -705,14 +736,16 @@ class PPO(Basenn):
             b_global = dist.global_rows(b_local, self._flat.device, self._dp_group)
         if self.obs_rms is not None:
             data = self._obs_norm_begin(data, b_global)
-        options = self.norm_adv or self.value_clip is not None or self.ppo_stats
+        if self.value_rms is not None:
+            self._value_norm_begin(data, b_global)
+        options = self.norm_adv or self.value_clip is not None or self.ppo_stats or self.value_rms is not None
         advs, old_values = self._full_batch_inputs(data) if options else (data.advs, None)
         for it in range(self.training_iter_time):
             start_time = time.time()
             if self._dp_world > 1 and not options:
                 self._backward_allreduce(data, b_global, obs_unchanged=it > 0)
             else:
-                # the options take the whole (not the segmented) backward, as extra critics do
+                # the options (and NORM_VALUE) take the whole (not the segmented) backward, as extra critics do
                 self.backward_only(data.states, advs, data.actions, data.old_logps, data.values, b_global,
                                    obs_unchanged=it > 0, old_values=old_values)
                 if self._dp_world > 1:
@@ -740,7 +773,7 @@ class PPO(Basenn):
                 raw[s] = t.to(device=self._flat.device, dtype=torch.float32).contiguous()
         states = self._normalized_obs([raw.get(i, x) for i, x in enumerate(data.states)], self._obs_learn)
         rms.moments(raw)
-        if self._dp_world > 1:
+        if self._dp_world > 1 and self.value_rms is None:        # with NORM_VALUE its collective carries these sums too
             dist.global_obs_sums(rms.sums, self._dp_group)
         self._obs_n = n_global
         out = copy.copy(data)
@@ -750,6 +783,25 @@ class PPO(Basenn):
     @_on_device
     def _obs_norm_end(self):
         self.obs_rms.merge(self._obs_n)
+
+    @_on_device
+    def _value_norm_begin(self, data, n_global):
+        """NORM_VALUE at the start of a learn call: the moments of critic 0's return targets (data.values[0]) around the
+        running mean, summed over the ranks of a data-parallel learner (one collective, shared with NORM_OBS's sums), folded
+        into the statistics, and critic 0's head rescaled in the flat parameter buffer so that its unnormalised outputs are
+        kept.  Every rank merges the same global sums and rescales the same replicated head: the replicas stay identical.
+        The engine reads the head from the flat buffer only, so no re-preparation follows."""
+        self._ensure_engine()
+        self.value_rms.refresh()
+        values = data.values if torch.is_tensor(data.values) else torch.as_tensor(np.asarray(data.values))
+        values = values.to(device=self._flat.device, dtype=torch.float32)
+        self.value_rms.moments({0: (values if values.dim() == 2 else values.view(1, -1))[0].contiguous()})
+        if self._dp_world > 1:
+            dist.global_obs_sums(self._norm_sums, self._dp_group)
+        off = dict(zip((n for n, _ in self.named_parameters()), self._offsets))
+        w, b = (self._flat[off["critic.critic_linear." + k]:][:p.numel()]
+                for k, p in (("weight", self.critic.critic_linear.weight), ("bias", self.critic.critic_linear.bias)))
+        self.value_rms.merge(n_global, w, b)
 
     def _step_and_log(self, start_time):
         """clip+Adam, then the loss dict of the step from ONE D2H copy (reference: four .item())."""
@@ -878,6 +930,8 @@ class PPO(Basenn):
         b_globals = dist.global_chunk_rows(sizes, dev, self._dp_group) if self._dp_world > 1 else sizes
         if self.obs_rms is not None:
             data = self._obs_norm_begin(data, sum(b_globals))       # the gathers then read the normalised batch
+        if self.value_rms is not None:
+            self._value_norm_begin(data, sum(b_globals))
         src = self._minibatch_sources(data)
         self._minibatch_buffers(src, b_local, max(sizes))
         if self._mb_gen is None or self._mb_gen.device != dev:

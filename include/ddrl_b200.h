@@ -190,6 +190,19 @@ int ddrl_ppo_loss_gaussian_v(const float* mu, int ld, const float* log_std, cons
                              int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
                              float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums, const float* old_values,
                              float* stats, void* stream);
+/* The same with value_norm (non-reference option NORM_VALUE): DEVICE {mean32, scale32, sigma32} or NULL.  When given, critic 0
+ * learns the normalised target (returns[b] - mean32) * scale32 and, with old_values, clips around (old_values[b] - mean32) *
+ * scale32, each operation rounded on its own; loss_sums[1] is then in normalised units.  NULL: the _v calls above. */
+int ddrl_ppo_loss_categorical_vn(const float* logits, int ld, const float* actions, const float* old_logp,
+                                 const float* adv, const float* returns, const float* v, int B, int A,
+                                 float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                                 float* dlogits, int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
+                                 const float* value_norm, void* stream);
+int ddrl_ppo_loss_gaussian_vn(const float* mu, int ld, const float* log_std, const float* actions,
+                              const float* old_logp, const float* adv, const float* returns, const float* v,
+                              int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                              float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums, const float* old_values,
+                              float* stats, const float* value_norm, void* stream);
 
 /* ---- advantage normalisation (non-reference option NORM_ADV) -------------------------------
  * ddrl_adv_moments: m3[0..2] = {n, sum a, sum a^2} of adv[0..n) in fp64 (m3: DEVICE, 3 doubles); a data-parallel learner sums
@@ -216,6 +229,15 @@ int ddrl_obs_rms_update(double* mean, double* var, double* count, const double* 
                         float* scale32, void* stream);
 int ddrl_obs_normalize(const float* x, int B, int D, const float* mean32, const float* scale32, float clip, float* out,
                        void* stream);
+
+/* ---- value-target normalisation (non-reference option NORM_VALUE, PopArt) ------------------
+ * ONE launch: the merge of ddrl_obs_rms_update for one column (critic 0's return targets; sums = ddrl_obs_moments with D = 1
+ * around *mean), then the applied form applied[0..3) = {fp32(mean), fp32(1 / sigma), fp32(sigma)}, sigma = sqrt(var + 1e-8)
+ * in fp64, and -- when head_w [F] and head_b [1] (device fp32, critic 0's head) are given and n > 0 -- the rescale that keeps
+ * the head's unnormalised outputs: w' = fp32(w * sigma_old / sigma_new), b' = fp32((sigma_old * b + mean_old - mean_new) /
+ * sigma_new), in fp64 with every operation correctly rounded (no fma).  n = 0 rewrites only the applied form (sums may be NULL). */
+int ddrl_value_norm_update(double* mean, double* var, double* count, const double* sums, double n, float* applied,
+                           float* head_w, float* head_b, int F, void* stream);
 
 /* Value loss of ONE extra critic head (nn/ppo.py:97-104: rndv_loss / gailv_loss = vlossf(data.values[k], values[k])):
  * dv[b] = d(loss)/d(v[b]) (times v_coef when shared, ppo.py:108), loss_sums[1] += contribution scaled by inv_B_global. */
@@ -284,6 +306,10 @@ int ddrl_net_bind(ddrl_net* net, float* params, float* grads, float* adam_m, flo
  * with its own encoder is a net of its own -- ddrl4nav_b200/nn/ppo.py builds one).  count = 0 clears. */
 int ddrl_net_set_extra_critics(ddrl_net* net, int count, const float* const* w, const float* const* b,
                                float* const* dw, float* const* db, const int* in_loss);
+/* NORM_VALUE: applied = DEVICE {mean32, scale32, sigma32} (ddrl_value_norm_update), read at every launch, or NULL (off).
+ * While set, the backward passes normalise critic 0's targets (ddrl_ppo_loss_*_vn), ddrl_net_forward returns critic 0's
+ * values as v * sigma32 + mean32 (two roundings), and ddrl_net_backward_segment returns DDRL_E_ARG. */
+int ddrl_net_set_value_norm(ddrl_net* net, const float* applied);
 /* tell the net the flat params were changed behind its back (load_state_dict, updatenn_by_redis) */
 int ddrl_net_params_changed(ddrl_net* net);
 /* number of observation slots and per-sample element count of each (for argument checking) */
