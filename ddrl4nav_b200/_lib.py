@@ -76,6 +76,12 @@ SIGNATURES = {
                                           _P, _P, _P]),
     "ddrl_ppo_loss_gaussian_vn": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P,
                                        _P, _P, _P, _P]),
+    "ddrl_ppo_loss_categorical_dc": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P,
+                                          _P, _P, _P, _F, _P]),
+    "ddrl_ppo_loss_gaussian_dc": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P,
+                                       _P, _P, _P, _P, _F, _P]),
+    "ddrl_logp_actions_categorical": (_I, [_P, _I, _P, _I, _I, _P, _P]),
+    "ddrl_logp_actions_gaussian": (_I, [_P, _I, _P, _P, _I, _I, _P, _P]),
     "ddrl_adv_moments":(_I, [_P, _I, _P, _P]),
     "ddrl_adv_normalize": (_I, [_P, _I, _P, _F, _P, _P]),
     "ddrl_obs_moments_ws_bytes": (_L, [_I, _I]),
@@ -99,13 +105,17 @@ SIGNATURES = {
     "ddrl_net_obs_elems": (_L, [_P, _I]),
     "ddrl_net_set_value_norm": (_I, [_P, _P]),
     "ddrl_net_forward": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P, _P, _P, _P]),
+    "ddrl_net_log_prob": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P]),
     "ddrl_net_encode": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P]),
     "ddrl_net_backward": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _I, _P]),
     "ddrl_net_backward_v": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, _P, C.POINTER(PPOHparams), _I, _P]),
+    "ddrl_net_backward_dc": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, _P, _P, _F, C.POINTER(PPOHparams), _I, _P]),
     "ddrl_net_backward_segment": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _I, _I, C.POINTER(_I), _P]),
     "ddrl_net_tensor_segment": (_I, [_P, _I]),
     "ddrl_net_backward_minibatch": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, C.POINTER(PPOHparams), _P]),
     "ddrl_net_backward_minibatch_v": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, _P, C.POINTER(PPOHparams), _P]),
+    "ddrl_net_backward_minibatch_dc": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P, _P, _P, _P, _P, _F, C.POINTER(PPOHparams),
+                                            _P]),
     "ddrl_gather_rows": (_I, [_P, _I, C.POINTER(GatherJob), _I, _P]),
     "ddrl_set_deterministic": (_I, [_I]),
     "ddrl_peer_allreduce_flag_bytes": (_I, []),

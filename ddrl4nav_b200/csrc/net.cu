@@ -114,6 +114,9 @@ struct ddrl_net {
   // NORM_VALUE (ddrl_net_set_value_norm): device {mean32, scale32, sigma32}; critic 0 learns normalised targets and the
   // forward pass returns its values denormalised.  Null: off.
   const float* value_norm = nullptr;
+  // DECOUPLED_PPO with hp->ppo_stats: the last backward pass took proximal log-probs, so its loss tail holds the behaviour KL
+  // in slot P+5 and ddrl_net_clip_adam reports it as loss4_out[6]
+  bool behaviour_kl = false;
   char* packed_base = nullptr;   // packed weights + packed grads arena
   char* split_base = nullptr;    // tc2 engine: [hi mirror of the packed arena | lo mirror]
   size_t packed_bytes = 0, packed_grad_off = 0, packed_grad_bytes = 0;
@@ -1730,19 +1733,49 @@ extern "C" int ddrl_net_encode(ddrl_net* n, const float* const* obs, int n_obs, 
   return DDRL_OK;
 }
 
+// DECOUPLED_PPO pre-pass: the training forward of the backward pass (same workspace, same lowering), then the loss kernels'
+// log-prob of the taken actions, so that a full-batch call within one micro-batch sees r == 1 exactly at its first step
+extern "C" int ddrl_net_log_prob(ddrl_net* n, const float* const* obs, int n_obs, int B, const float* actions, float* out_logp,
+                                 void* stream) {
+  if (!n || B < 0) return DDRL_E_ARG;
+  if (!n->params) return DDRL_E_STATE;
+  if (B == 0) return DDRL_OK;
+  TRY(check_obs(n, obs, n_obs));
+  if (!actions || !out_logp) return DDRL_E_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  TRY(ensure_workspace(n, B, true));     // the backward's workspace: no reallocation, so its graph keys hold
+  if (n->dirty) TRY(repack(n, s));
+  n->cols_obs0 = nullptr;                // the staged observations belong to no backward call now
+  n->cols_rows = -1;
+  const int A = n->d.act_dim;
+  for (long long r0 = 0; r0 < B; r0 += n->MB) {
+    const int mb = (int)std::min<long long>(n->MB, B - r0);
+    amax_new_pass(n, s, false);
+    TRY(forward_chunk(n, obs, r0, mb, true, s));
+    if (n->d.dist == DDRL_DIST_CATEGORICAL) {
+      TRY(ddrl_logp_actions_categorical(n->logits, n->ldA, actions + r0, mb, A, out_logp + r0, s));
+    } else {
+      TRY(ddrl_logp_actions_gaussian(n->logits, n->ldA, n->params + n->T[n->t_logstd].offset, actions + r0 * A, mb, A,
+                                     out_logp + r0, s));
+    }
+  }
+  return DDRL_OK;
+}
+
 namespace ddrl {
 // zero the gradients, then per micro-batch: forward (act = data.actions), fused loss, heads and encoders backward; finally
 // the packed weight gradients are un-permuted into the reference layout
 static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int B_global, const float* actions,
                          const float* old_logp, const float* adv, const float* returns, const float* old_values,
-                         const ddrl_ppo_hparams* hp, bool reuse_obs, cudaStream_t s) {
+                         const float* prox_logp, float is_clip, const ddrl_ppo_hparams* hp, bool reuse_obs, cudaStream_t s) {
   // zero the flat grads (+ loss tail) and the packed grads: everything below accumulates
   DDRL_CUDA(cudaMemsetAsync(n->grads, 0, sizeof(float) * (size_t)(n->P + 8), s));
   if (n->packed_base) DDRL_CUDA(cudaMemsetAsync(n->packed_base + n->packed_grad_off, 0, n->packed_grad_bytes, s));
   const int A = n->d.act_dim, F = n->d.feat;
   const float invB = 1.0f / (float)B_global;
   float* loss_sums = n->grads + n->P;
-  float* stats = hp->ppo_stats ? loss_sums + 3 : nullptr;      // {approx KL, clip fraction} sums in tail slots 3 and 4
+  // {approx KL, clip fraction} sums in tail slots 3 and 4 (+ the behaviour KL in slot 5 with prox_logp)
+  float* stats = hp->ppo_stats ? loss_sums + 3 : nullptr;
   Tower& ta = n->towers[0];
   Tower& tc = n->towers[n->d.shared ? 0 : 1];
   float* aw = n->params + n->T[n->t_aw].offset;
@@ -1753,14 +1786,15 @@ static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int 
     amax_new_pass(n, s, reuse_obs);
     TRY(forward_chunk(n, obs, r0, mb, true, s, reuse_obs));
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
-      TRY(ddrl_ppo_loss_categorical_vn(n->logits, n->ldA, actions + r0, old_logp + r0, adv + r0, returns + r0, n->vout, mb, A,
+      TRY(ddrl_ppo_loss_categorical_dc(n->logits, n->ldA, actions + r0, old_logp + r0, adv + r0, returns + r0, n->vout, mb, A,
                                        invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
-                                       old_values ? old_values + r0 : nullptr, stats, n->value_norm, s));
+                                       old_values ? old_values + r0 : nullptr, stats, n->value_norm,
+                                       prox_logp ? prox_logp + r0 : nullptr, is_clip, s));
     } else {
-      TRY(ddrl_ppo_loss_gaussian_vn(n->logits, n->ldA, n->params + n->T[n->t_logstd].offset, actions + r0 * A, old_logp + r0,
+      TRY(ddrl_ppo_loss_gaussian_dc(n->logits, n->ldA, n->params + n->T[n->t_logstd].offset, actions + r0 * A, old_logp + r0,
                                     adv + r0, returns + r0, n->vout, mb, A, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv,
                                     n->grads + n->T[n->t_logstd].offset, loss_sums, old_values ? old_values + r0 : nullptr, stats,
-                                    n->value_norm, s));
+                                    n->value_norm, prox_logp ? prox_logp + r0 : nullptr, is_clip, s));
     }
     // heads backward (nn/actor.py:91 actor_linear, nn/critic.py:21 critic_linear)
     TRY(skinny_wgrad(n->dlogits, n->ldA, ta.h, F, mb, A, F, n->grads + n->T[n->t_aw].offset, n->grads + n->T[n->t_ab].offset, s));
@@ -1790,12 +1824,22 @@ static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int 
 
 // seg < 0: the whole pass.  seg >= 0: segment `seg` only (seg 0 validates, prepares and -- when the pass is not replayable as
 // a graph chain -- runs everything and reports one segment).
+// the truncation of the behaviour weight as a graph-key integer (its bits)
+static long long is_clip_key(float is_clip) {
+  uint32_t u;
+  memcpy(&u, &is_clip, sizeof(u));
+  return (long long)u;
+}
+
 static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global, const float* actions,
                          const float* old_logp, const float* adv, const float* returns, const float* old_values,
-                         const ddrl_ppo_hparams* hp, int obs_unchanged, int seg, int* nseg_out, cudaStream_t s) {
+                         const float* prox_logp, float is_clip, const ddrl_ppo_hparams* hp, int obs_unchanged, int seg,
+                         int* nseg_out, cudaStream_t s) {
   if (!n || !hp || B_local < 0 || B_global < B_local || B_global < 1) return DDRL_E_ARG;
   if (B_local > 0 && !value_clip_ok(hp, old_values)) return DDRL_E_ARG;
   if (!n->params || !n->grads) return DDRL_E_STATE;
+  if (!prox_logp) is_clip = 0.f;
+  n->behaviour_kl = prox_logp && hp->ppo_stats;
   if (nseg_out) *nseg_out = 1;
   if (B_local == 0) {
     if (seg > 0) return DDRL_E_ARG;
@@ -1806,8 +1850,8 @@ static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_
   TRY(check_obs(n, obs, n_obs));
   if (!actions || !old_logp || !adv || !returns) return DDRL_E_ARG;
   const std::string key = graph_key("bwd", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, actions, old_logp,
-                                            adv, returns, old_values, n->value_norm, n->params, n->grads, n->ws.base},
-                                    {B_local, B_global}, hp, sizeof(*hp));
+                                            adv, returns, old_values, n->value_norm, prox_logp, n->params, n->grads, n->ws.base},
+                                    {B_local, B_global, is_clip_key(is_clip)}, hp, sizeof(*hp));
   auto launch_seg = [&](ddrl_net::GraphEntry* e, int k) {
     const int pre = (int)e->pre_execs.size();
     if (k < 0 || k > pre) return (int)DDRL_E_ARG;
@@ -1835,27 +1879,37 @@ static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_
   if (reuse_obs && n->extra.empty() && graphs_enabled(n)) {
     ddrl_net::GraphEntry* e = nullptr;
     TRY(run_graphed(n, key, s, [&](cudaStream_t cs) {
-      return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, hp, true, cs);
+      return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, prox_logp, is_clip, hp, true,
+                           cs);
     }, seg < 0 ? nullptr : &e));
     if (seg < 0 || !e) return DDRL_OK;             // launched whole / capture failed: the body already ran on the stream
     if (nseg_out) *nseg_out = (int)e->pre_execs.size() + 1;
     return launch_seg(e, 0);
   }
-  return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, hp, reuse_obs, s);
+  return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, prox_logp, is_clip, hp, reuse_obs,
+                       s);
 }
 
 extern "C" int ddrl_net_backward(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
                                  const float* actions, const float* old_logp, const float* adv, const float* returns,
                                  const ddrl_ppo_hparams* hp, int obs_unchanged, void* stream) {
-  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, nullptr, hp, obs_unchanged, -1, nullptr,
-                       (cudaStream_t)stream);
+  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, nullptr, nullptr, 0.f, hp, obs_unchanged,
+                       -1, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int ddrl_net_backward_dc(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
+                                    const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                    const float* old_values, const float* prox_logp, float is_clip, const ddrl_ppo_hparams* hp,
+                                    int obs_unchanged, void* stream) {
+  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, old_values, prox_logp, is_clip, hp,
+                       obs_unchanged, -1, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int ddrl_net_backward_v(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
                                    const float* actions, const float* old_logp, const float* adv, const float* returns,
                                    const float* old_values, const ddrl_ppo_hparams* hp, int obs_unchanged, void* stream) {
-  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, old_values, hp, obs_unchanged, -1,
-                       nullptr, (cudaStream_t)stream);
+  return ddrl_net_backward_dc(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, old_values, nullptr, 0.f, hp,
+                              obs_unchanged, stream);
 }
 
 extern "C" int ddrl_net_backward_segment(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
@@ -1863,18 +1917,21 @@ extern "C" int ddrl_net_backward_segment(ddrl_net* n, const float* const* obs, i
                                          const ddrl_ppo_hparams* hp, int obs_unchanged, int segment, int* n_segments,
                                          void* stream) {
   if (segment < 0 || !n_segments || (n && n->value_norm)) return DDRL_E_ARG;
-  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, nullptr, hp, obs_unchanged, segment,
-                       n_segments, (cudaStream_t)stream);
+  return backward_impl(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, nullptr, nullptr, 0.f, hp, obs_unchanged,
+                       segment, n_segments, (cudaStream_t)stream);
 }
 
 // One minibatch step: new rows at the addresses of an earlier call.  The observations are always restaged (reuse_obs = false),
 // so the pass depends on no staging left by an earlier call; the staged observations it leaves belong to no full-batch call.
-extern "C" int ddrl_net_backward_minibatch_v(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
-                                             const float* actions, const float* old_logp, const float* adv, const float* returns,
-                                             const float* old_values, const ddrl_ppo_hparams* hp, void* stream) {
+extern "C" int ddrl_net_backward_minibatch_dc(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
+                                              const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                              const float* old_values, const float* prox_logp, float is_clip,
+                                              const ddrl_ppo_hparams* hp, void* stream) {
   if (!n || !hp || B_local < 0 || B_global < B_local || B_global < 1) return DDRL_E_ARG;
   if (B_local > 0 && !value_clip_ok(hp, old_values)) return DDRL_E_ARG;
   if (!n->params || !n->grads) return DDRL_E_STATE;
+  if (!prox_logp) is_clip = 0.f;
+  n->behaviour_kl = prox_logp && hp->ppo_stats;
   cudaStream_t s = (cudaStream_t)stream;
   if (B_local == 0) {
     DDRL_CUDA(cudaMemsetAsync(n->grads, 0, sizeof(float) * (size_t)(n->P + 8), s));
@@ -1888,19 +1945,26 @@ extern "C" int ddrl_net_backward_minibatch_v(ddrl_net* n, const float* const* ob
   n->cols_obs0 = nullptr;            // a later ddrl_net_backward(obs_unchanged) restages
   n->cols_rows = -1;
   auto body = [&](cudaStream_t cs) {
-    return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, hp, false, cs);
+    return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, prox_logp, is_clip, hp, false, cs);
   };
   if (B_local > n->MB || !n->extra.empty() || !graphs_enabled(n) || n->mb_graphs_off) return body(s);
   const std::string key = graph_key("bwd_mb", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, actions,
-                                               old_logp, adv, returns, old_values, n->value_norm, n->params, n->grads,
+                                               old_logp, adv, returns, old_values, n->value_norm, prox_logp, n->params, n->grads,
                                                n->ws.base},
-                                    {B_local, B_global}, hp, sizeof(*hp));
+                                    {B_local, B_global, is_clip_key(is_clip)}, hp, sizeof(*hp));
   if (std::find(n->mb_seen.begin(), n->mb_seen.end(), key) == n->mb_seen.end()) {
     if (n->mb_seen.size() >= 16) n->mb_seen.erase(n->mb_seen.begin());
     n->mb_seen.push_back(key);
     return body(s);
   }
   return run_graphed(n, key, s, body, nullptr, &n->mb_graphs_off);
+}
+
+extern "C" int ddrl_net_backward_minibatch_v(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
+                                             const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                             const float* old_values, const ddrl_ppo_hparams* hp, void* stream) {
+  return ddrl_net_backward_minibatch_dc(n, obs, n_obs, B_local, B_global, actions, old_logp, adv, returns, old_values, nullptr,
+                                        0.f, hp, stream);
 }
 
 extern "C" int ddrl_net_backward_minibatch(ddrl_net* n, const float* const* obs, int n_obs, int B_local, int B_global,
@@ -1930,19 +1994,22 @@ extern "C" int ddrl_net_debug_buffer(ddrl_net* n, int tower, int idx, float* out
 }
 
 namespace ddrl {
+// stats: 0 none, 1 {approx KL, clip fraction}, 2 the same + the behaviour KL (DECOUPLED_PPO)
 __global__ void finish_losses_kernel(const float* __restrict__ sums, float v_coef, float ent_coef, int stats,
                                      float* __restrict__ out) {
   const float a = sums[0], v = sums[1], e = sums[2];
   out[0] = a + v * v_coef - e * ent_coef;      // nn/ppo.py:108
   out[1] = a; out[2] = v; out[3] = e;
   if (stats) { out[4] = sums[3]; out[5] = sums[4]; }
+  if (stats > 1) out[6] = sums[5];
 }
 }  // namespace ddrl
 
 namespace ddrl {
 static int clip_adam_body(ddrl_net* n, int step, const ddrl_ppo_hparams* hp, float* loss4_out, cudaStream_t s) {
   if (loss4_out) {
-    finish_losses_kernel<<<1, 1, 0, s>>>(n->grads + n->P, hp->v_coef, hp->ent_coef, hp->ppo_stats, loss4_out);
+    const int stats = hp->ppo_stats ? (n->behaviour_kl ? 2 : 1) : 0;
+    finish_losses_kernel<<<1, 1, 0, s>>>(n->grads + n->P, hp->v_coef, hp->ent_coef, stats, loss4_out);
     DDRL_LAUNCHED("finish_losses_kernel");
   }
   long long sb[3] = {n->seg_begin[0], n->seg_begin[1], n->seg_begin[2]};
@@ -1964,7 +2031,8 @@ extern "C" int ddrl_net_clip_adam(ddrl_net* n, int step, const ddrl_ppo_hparams*
   // step-dependent scalars of the clip+Adam node change between replays.  The first step of a net runs on the stream (it
   // also performs the one-time allocations a capture must not contain).
   if (step > 1 && !n->dirty && n->packed_base && graphs_enabled(n)) {
-    const std::string key = graph_key("adam", {loss4_out, n->params, n->grads, n->am, n->av}, {}, hp, sizeof(*hp));
+    const std::string key = graph_key("adam", {loss4_out, n->params, n->grads, n->am, n->av}, {(long long)n->behaviour_kl}, hp,
+                                      sizeof(*hp));
     ddrl_net::GraphEntry* e = nullptr;
     TRY(run_graphed(n, key, s, [&](cudaStream_t cs) { return clip_adam_body(n, step, hp, loss4_out, cs); }, &e));
     if (!e) return DDRL_OK;                       // capture failed: the body already ran on the stream

@@ -21,6 +21,10 @@
 //          the same ordered / atomic adds as the loss sums.
 //   value_norm (in LossParams): critic 0 learns normalised targets R~ = (R - mean32) * scale32, and old_v is normalised the same
 //          way, each operation rounded on its own; the extra critics' value_loss_kernel never normalises.
+//   prox (in LossParams, DECOUPLED_PPO): the ratio is taken against the proximal log-prob, r = exp(logp - prox), and the actor
+//          term and its gradient are weighted by the behaviour weight w = exp(prox - old_logp) (min(w, is_clip) when is_clip > 0):
+//          w * term(r, A) and w * dterm * r.  stats[2] += inv_B*((rho - 1) - log rho), rho = exp(prox - old_logp) untruncated.
+//          With prox null, w = 1 and every product by it is exact: the kernels compute exactly the loss without it.
 #include "common.cuh"
 
 namespace ddrl {
@@ -34,7 +38,53 @@ struct LossParams {
   float ppo_clip, dual_clip, v_coef, ent_coef, inv_B, value_clip;
   int smooth_l1, shared;
   const float* value_norm;        // NORM_VALUE: device {mean32, scale32, sigma32} of critic 0's targets, or null
+  const float* prox;              // DECOUPLED_PPO: proximal log-probs [B], or null
+  float is_clip;                  // DECOUPLED_PPO: truncation of the behaviour weight, <= 0: none
 };
+
+// log-prob of the taken action a (clamped into [0, A)) under Categorical(logits = x[0..A)): the softmax -> q = p / sum(p) ->
+// clamp(eps, 1 - eps) -> log chain of torch.  Leaves the softmax p[0..A) and s2 = sum(p) for the loss kernel's gradient.  The
+// loss kernel and logp_actions_categorical_kernel share it, so equal logits give equal log-prob bits.
+__device__ __forceinline__ float categorical_logp(const float* __restrict__ x, int A, float action, float* p, float* s2_out) {
+  float m = x[0];
+  for (int j = 1; j < A; ++j) m = fmaxf(m, x[j]);
+  float s = 0.f;
+  for (int j = 0; j < A; ++j) { p[j] = expf(x[j] - m); s += p[j]; }
+  float s2 = 0.f;
+  for (int j = 0; j < A; ++j) { p[j] = p[j] / s; s2 += p[j]; }
+  int a = (int)action;                      // Categorical.log_prob: value.long()
+  a = a < 0 ? 0 : (a >= A ? A - 1 : a);     // the reference raises on an action outside [0, A); never read out of bounds
+  const float qa = p[a] / s2;
+  const float ca = fminf(fmaxf(qa, kEpsL), 1.f - kEpsL);
+  *s2_out = s2;
+  return logf(ca);
+}
+
+// log-prob of the action row act[0..A) under Normal(mu[0..A), exp(log_std)) summed over A (normal.py log_prob); shared by the
+// Gaussian loss kernel and logp_actions_gaussian_kernel
+__device__ __forceinline__ float gaussian_logp(const float* __restrict__ mu, const float* __restrict__ log_std,
+                                               const float* __restrict__ act, int A) {
+  float lp = 0.f;
+  for (int j = 0; j < A; ++j) {
+    const float sd = expf(log_std[j]);
+    const float z = act[j] - mu[j];
+    lp += -(z * z) / (2.f * (sd * sd)) - logf(sd) - kLogSqrt2PiL;
+  }
+  return lp;
+}
+
+// DECOUPLED_PPO: log r against the proximal log-prob when it is given (else against old_logp), and the behaviour weight w
+// (1 without prox); *l_bkl = inv_B * ((rho - 1) - log rho) with rho = exp(prox - old_logp) when stats are on
+__device__ __forceinline__ float decoupled_log_ratio(float logp, const float* __restrict__ old_logp, int b, const LossParams& hp,
+                                                     bool stats, float* w, float* l_bkl) {
+  if (!hp.prox) { *w = 1.f; return logp - old_logp[b]; }
+  const float pl = hp.prox[b];
+  const float log_rho = pl - old_logp[b];
+  const float rho = expf(log_rho);
+  *w = hp.is_clip > 0.f ? fminf(rho, hp.is_clip) : rho;
+  if (stats) *l_bkl = ((rho - 1.f) - log_rho) * hp.inv_B;
+  return logp - pl;
+}
 
 // d(term)/d(ratio) of term = A>0 ? s : max(s, dual*A), s = min(ratio*A, clamp(ratio)*A); also returns term
 __device__ __forceinline__ float surrogate(float ratio, float A, const LossParams& hp, float* dterm_dratio) {
@@ -100,33 +150,26 @@ __global__ void __launch_bounds__(128) ppo_loss_categorical_kernel(
     const float* __restrict__ old_v, float* __restrict__ stats, DetSeq det) {
   __shared__ float scratch[32];
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  float l_actor = 0.f, l_v = 0.f, l_ent = 0.f, l_kl = 0.f, l_cf = 0.f;
+  float l_actor = 0.f, l_v = 0.f, l_ent = 0.f, l_kl = 0.f, l_cf = 0.f, l_bkl = 0.f;
   if (b < B) {
     const float* x = logits + (size_t)b * ld;
     float p[kMaxAL];
-    float m = x[0];
-    for (int j = 1; j < A; ++j) m = fmaxf(m, x[j]);
-    float s = 0.f;
-    for (int j = 0; j < A; ++j) { p[j] = expf(x[j] - m); s += p[j]; }
-    float s2 = 0.f;
-    for (int j = 0; j < A; ++j) { p[j] = p[j] / s; s2 += p[j]; }
-    int a = (int)actions[b];                  // Categorical.log_prob: value.long()
-    a = a < 0 ? 0 : (a >= A ? A - 1 : a);     // the reference raises on an action outside [0, A); never read out of bounds
+    float s2;
+    const float logp = categorical_logp(x, A, actions[b], p, &s2);      // log-prob of the taken action
+    int a = (int)actions[b];
+    a = a < 0 ? 0 : (a >= A ? A - 1 : a);
     const float Ai = adv[b];
-    // log-prob of the taken action
-    const float qa = p[a] / s2;
-    const float ca = fminf(fmaxf(qa, kEpsL), 1.f - kEpsL);
-    const float logp = logf(ca);
-    const float log_ratio = logp - old_logp[b];
+    float w;
+    const float log_ratio = decoupled_log_ratio(logp, old_logp, b, hp, stats != nullptr, &w, &l_bkl);
     const float ratio = expf(log_ratio);
     float dterm;
     const float term = surrogate(ratio, Ai, hp, &dterm);
-    l_actor = -term * hp.inv_B;
+    l_actor = -(w * term) * hp.inv_B;
     if (stats) {
       l_kl = ((ratio - 1.f) - log_ratio) * hp.inv_B;
       l_cf = fabsf(ratio - 1.f) > hp.ppo_clip ? hp.inv_B : 0.f;
     }
-    const float w_lp = -hp.inv_B * dterm * ratio;                       // dLoss/dlogp
+    const float w_lp = -hp.inv_B * (w * dterm) * ratio;                 // dLoss/dlogp
     const float w_ent = hp.shared ? -hp.ent_coef * hp.inv_B : 0.f;      // dLoss/dH_b
     // gradient wrt q (normalised probs): gq_j
     float H = 0.f, dot_q = 0.f;
@@ -158,6 +201,7 @@ __global__ void __launch_bounds__(128) ppo_loss_categorical_kernel(
   if (stats) {
     l_kl = block_sum(l_kl, scratch);
     l_cf = block_sum(l_cf, scratch);
+    if (hp.prox) l_bkl = block_sum(l_bkl, scratch);
   }
   if (threadIdx.x == 0) {
     if (det.ctr) det_enter(det.ctr, blockIdx.x);         // deterministic mode: the blocks add in block order
@@ -167,6 +211,7 @@ __global__ void __launch_bounds__(128) ppo_loss_categorical_kernel(
     if (stats) {
       det_add(det.ctr != nullptr, stats + 0, l_kl);
       det_add(det.ctr != nullptr, stats + 1, l_cf);
+      if (hp.prox) det_add(det.ctr != nullptr, stats + 2, l_bkl);
     }
     if (det.ctr) det_leave(det.ctr, blockIdx.x, gridDim.x);
   }
@@ -180,30 +225,27 @@ __global__ void __launch_bounds__(128) ppo_loss_gaussian_kernel(
     float* __restrict__ stats, DetSeq det) {
   __shared__ float scratch[32];
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  float l_actor = 0.f, l_v = 0.f, l_ent = 0.f, l_kl = 0.f, l_cf = 0.f;
+  float l_actor = 0.f, l_v = 0.f, l_ent = 0.f, l_kl = 0.f, l_cf = 0.f, l_bkl = 0.f;
   float dls[8];
 #pragma unroll
   for (int j = 0; j < 8; ++j) dls[j] = 0.f;
   if (b < B) {
-    float lp = 0.f, H = 0.f;
-    for (int j = 0; j < A; ++j) {
-      const float sd = expf(log_std[j]);
-      const float z = actions[(size_t)b * A + j] - mu[(size_t)b * ld + j];
-      lp += -(z * z) / (2.f * (sd * sd)) - logf(sd) - kLogSqrt2PiL;
-      H += 0.5f + kLogSqrt2PiL + logf(sd);      // normal.py:114-115
-    }
+    const float lp = gaussian_logp(mu + (size_t)b * ld, log_std, actions + (size_t)b * A, A);
+    float H = 0.f;
+    for (int j = 0; j < A; ++j) H += 0.5f + kLogSqrt2PiL + logf(expf(log_std[j]));      // normal.py:114-115
     const float Ai = adv[b];
-    const float log_ratio = lp - old_logp[b];
+    float w;
+    const float log_ratio = decoupled_log_ratio(lp, old_logp, b, hp, stats != nullptr, &w, &l_bkl);
     const float ratio = expf(log_ratio);
     float dterm;
     const float term = surrogate(ratio, Ai, hp, &dterm);
-    l_actor = -term * hp.inv_B;
+    l_actor = -(w * term) * hp.inv_B;
     if (stats) {
       l_kl = ((ratio - 1.f) - log_ratio) * hp.inv_B;
       l_cf = fabsf(ratio - 1.f) > hp.ppo_clip ? hp.inv_B : 0.f;
     }
     l_ent = H * hp.inv_B / (float)A;            // mean over all [B,A] elements
-    const float w_lp = -hp.inv_B * dterm * ratio;
+    const float w_lp = -hp.inv_B * (w * dterm) * ratio;
     for (int j = 0; j < A; ++j) {
       const float sd = expf(log_std[j]);
       const float var = sd * sd;
@@ -223,6 +265,7 @@ __global__ void __launch_bounds__(128) ppo_loss_gaussian_kernel(
   if (stats) {
     l_kl = block_sum(l_kl, scratch);
     l_cf = block_sum(l_cf, scratch);
+    if (hp.prox) l_bkl = block_sum(l_bkl, scratch);
   }
   float tls[8];
   for (int j = 0; j < A && j < 8; ++j) tls[j] = block_sum(dls[j], scratch);
@@ -234,6 +277,7 @@ __global__ void __launch_bounds__(128) ppo_loss_gaussian_kernel(
     if (stats) {
       det_add(det.ctr != nullptr, stats + 0, l_kl);
       det_add(det.ctr != nullptr, stats + 1, l_cf);
+      if (hp.prox) det_add(det.ctr != nullptr, stats + 2, l_bkl);
     }
     for (int j = 0; j < A && j < 8; ++j) det_add(det.ctr != nullptr, dlog_std + j, tls[j]);
     if (det.ctr) det_leave(det.ctr, blockIdx.x, gridDim.x);
@@ -259,10 +303,32 @@ __global__ void __launch_bounds__(128) value_loss_kernel(const float* __restrict
   }
 }
 
-static LossParams make_params(const ddrl_ppo_hparams* hp, float inv_B, int shared, const float* value_norm = nullptr) {
+// DECOUPLED_PPO pre-pass: out_logp[b] = log-prob of the taken action, bit-equal to the loss kernels' on the same logits / means
+__global__ void __launch_bounds__(128) logp_actions_categorical_kernel(const float* __restrict__ logits, int ld,
+                                                                       const float* __restrict__ actions, int B, int A,
+                                                                       float* __restrict__ out_logp) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  float p[kMaxAL];
+  float s2;
+  out_logp[b] = categorical_logp(logits + (size_t)b * ld, A, actions[b], p, &s2);
+}
+
+__global__ void __launch_bounds__(128) logp_actions_gaussian_kernel(const float* __restrict__ mu, int ld,
+                                                                    const float* __restrict__ log_std,
+                                                                    const float* __restrict__ actions, int B, int A,
+                                                                    float* __restrict__ out_logp) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  out_logp[b] = gaussian_logp(mu + (size_t)b * ld, log_std, actions + (size_t)b * A, A);
+}
+
+static LossParams make_params(const ddrl_ppo_hparams* hp, float inv_B, int shared, const float* value_norm = nullptr,
+                              const float* prox = nullptr, float is_clip = 0.f) {
   LossParams p;
   p.ppo_clip = hp->ppo_clip; p.dual_clip = hp->dual_clip; p.v_coef = hp->v_coef; p.ent_coef = hp->ent_coef;
   p.inv_B = inv_B; p.value_clip = hp->value_clip; p.smooth_l1 = hp->smooth_l1; p.shared = shared; p.value_norm = value_norm;
+  p.prox = prox; p.is_clip = prox ? is_clip : 0.f;
   return p;
 }
 
@@ -275,21 +341,30 @@ static bool value_clip_args_ok(const ddrl_ppo_hparams* hp, const float* old_valu
   return old_values ? hp->value_clip > 0.f : !(hp->value_clip > 0.f);
 }
 
-extern "C" int ddrl_ppo_loss_categorical_vn(const float* logits, int ld, const float* actions, const float* old_logp,
+extern "C" int ddrl_ppo_loss_categorical_dc(const float* logits, int ld, const float* actions, const float* old_logp,
                                             const float* adv, const float* returns, const float* v, int B, int A,
                                             float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dlogits,
                                             int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
-                                            const float* value_norm, void* stream) {
+                                            const float* value_norm, const float* prox_logp, float is_clip, void* stream) {
   if (B < 0 || A < 1 || A > kMaxAL || ld < A || ld_d < A || !hp) return DDRL_E_ARG;
   if (!value_clip_args_ok(hp, old_values)) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!logits || !actions || !old_logp || !adv || !returns || !v || !dlogits || !dv || !loss_sums) return DDRL_E_ARG;
   ppo_loss_categorical_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(
-      logits, ld, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared, value_norm), dlogits, ld_d,
-      dv, loss_sums, old_values, stats, det_seq(1));
-  prof_work((8.0 * A + 24.0 + (old_values ? 4.0 : 0.0)) * B);
+      logits, ld, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared, value_norm, prox_logp, is_clip),
+      dlogits, ld_d, dv, loss_sums, old_values, stats, det_seq(1));
+  prof_work((8.0 * A + 24.0 + (old_values ? 4.0 : 0.0) + (prox_logp ? 4.0 : 0.0)) * B);
   DDRL_LAUNCHED("ppo_loss_categorical_kernel");
   return DDRL_OK;
+}
+
+extern "C" int ddrl_ppo_loss_categorical_vn(const float* logits, int ld, const float* actions, const float* old_logp,
+                                            const float* adv, const float* returns, const float* v, int B, int A,
+                                            float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dlogits,
+                                            int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
+                                            const float* value_norm, void* stream) {
+  return ddrl_ppo_loss_categorical_dc(logits, ld, actions, old_logp, adv, returns, v, B, A, inv_B_global, hp, shared, dlogits,
+                                      ld_d, dv, loss_sums, old_values, stats, value_norm, nullptr, 0.f, stream);
 }
 
 extern "C" int ddrl_ppo_loss_categorical_v(const float* logits, int ld, const float* actions, const float* old_logp,
@@ -321,21 +396,53 @@ extern "C" int ddrl_value_loss(const float* returns, const float* v, int B, floa
   return DDRL_OK;
 }
 
-extern "C" int ddrl_ppo_loss_gaussian_vn(const float* mu, int ld, const float* log_std, const float* actions,
+extern "C" int ddrl_ppo_loss_gaussian_dc(const float* mu, int ld, const float* log_std, const float* actions,
                                          const float* old_logp, const float* adv, const float* returns, const float* v,
                                          int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
                                          float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums,
-                                         const float* old_values, float* stats, const float* value_norm, void* stream) {
+                                         const float* old_values, float* stats, const float* value_norm,
+                                         const float* prox_logp, float is_clip, void* stream) {
   if (B < 0 || A < 1 || A > 8 || ld < A || ld_d < A || !hp) return DDRL_E_ARG;
   if (!value_clip_args_ok(hp, old_values)) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!mu || !log_std || !actions || !old_logp || !adv || !returns || !v || !dmu || !dv || !dlog_std || !loss_sums)
     return DDRL_E_ARG;
   ppo_loss_gaussian_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(
-      mu, ld, log_std, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared, value_norm), dmu, ld_d,
-      dv, dlog_std, loss_sums, old_values, stats, det_seq(1));
-  prof_work((12.0 * A + 20.0 + (old_values ? 4.0 : 0.0)) * B);
+      mu, ld, log_std, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared, value_norm, prox_logp, is_clip),
+      dmu, ld_d, dv, dlog_std, loss_sums, old_values, stats, det_seq(1));
+  prof_work((12.0 * A + 20.0 + (old_values ? 4.0 : 0.0) + (prox_logp ? 4.0 : 0.0)) * B);
   DDRL_LAUNCHED("ppo_loss_gaussian_kernel");
+  return DDRL_OK;
+}
+
+extern "C" int ddrl_ppo_loss_gaussian_vn(const float* mu, int ld, const float* log_std, const float* actions,
+                                         const float* old_logp, const float* adv, const float* returns, const float* v,
+                                         int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                                         float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums,
+                                         const float* old_values, float* stats, const float* value_norm, void* stream) {
+  return ddrl_ppo_loss_gaussian_dc(mu, ld, log_std, actions, old_logp, adv, returns, v, B, A, inv_B_global, hp, shared, dmu,
+                                   ld_d, dv, dlog_std, loss_sums, old_values, stats, value_norm, nullptr, 0.f, stream);
+}
+
+extern "C" int ddrl_logp_actions_categorical(const float* logits, int ld, const float* actions, int B, int A, float* out_logp,
+                                             void* stream) {
+  if (B < 0 || A < 1 || A > kMaxAL || ld < A) return DDRL_E_ARG;
+  if (B == 0) return DDRL_OK;
+  if (!logits || !actions || !out_logp) return DDRL_E_ARG;
+  logp_actions_categorical_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, actions, B, A, out_logp);
+  prof_work((4.0 * A + 8.0) * B);
+  DDRL_LAUNCHED("logp_actions_categorical_kernel");
+  return DDRL_OK;
+}
+
+extern "C" int ddrl_logp_actions_gaussian(const float* mu, int ld, const float* log_std, const float* actions, int B, int A,
+                                          float* out_logp, void* stream) {
+  if (B < 0 || A < 1 || A > 8 || ld < A) return DDRL_E_ARG;
+  if (B == 0) return DDRL_OK;
+  if (!mu || !log_std || !actions || !out_logp) return DDRL_E_ARG;
+  logp_actions_gaussian_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(mu, ld, log_std, actions, B, A, out_logp);
+  prof_work((8.0 * A + 4.0) * B);
+  DDRL_LAUNCHED("logp_actions_gaussian_kernel");
   return DDRL_OK;
 }
 

@@ -57,7 +57,8 @@ def global_chunk_rows(chunk_rows, device, group=None):
 
 def allreduce_grads(flat_grads_with_tail: torch.Tensor, n_params: int, group=None, tail: int = 4) -> None:
     """In-place sum over ranks of grads[0 : P+tail]: P parameters + the loss sums {actor, v, entropy, -} (tail 4), or
-    {actor, v, entropy, approx KL, clip fraction} (tail 5, PPO_STATS)."""
+    {actor, v, entropy, approx KL, clip fraction} (tail 5, PPO_STATS), + the behaviour KL (tail 6, PPO_STATS with
+    DECOUPLED_PPO)."""
     import torch.distributed as dist
     _, ws = world(group)
     if ws > 1:

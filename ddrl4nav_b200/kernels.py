@@ -158,6 +158,75 @@ def ppo_loss_gaussian(mu, log_std, actions, old_logp, adv, returns, v, hp: PPOHp
     return dmu, dv, dls, sums
 
 
+def ppo_loss_categorical_dc(logits, actions, old_logp, adv, returns, v, hp: PPOHparams, shared: bool, prox_logp=None,
+                            is_clip: Optional[float] = None, b_global: Optional[int] = None):
+    """The decoupled loss (ddrl_ppo_loss_categorical_dc) with the statistics on -> (dlogits [B,A], dv [B], sums [8]):
+    sums[0..3) = {actor, v, entropy}, sums[3..6) = {approx KL, clip fraction, behaviour KL}.  prox_logp None: plain PPO."""
+    lib = _lib.load()
+    logits, actions, old_logp, adv, returns, v = map(_f32c, (logits, actions, old_logp, adv, returns, v))
+    prox_logp = None if prox_logp is None else _f32c(prox_logp)
+    B, A = logits.shape
+    dlogits = torch.empty_like(logits)
+    dv = torch.empty(B, dtype=torch.float32, device=logits.device)
+    sums = torch.zeros(8, dtype=torch.float32, device=logits.device)
+    check(lib.ddrl_ppo_loss_categorical_dc(ptr(logits), A, ptr(actions), ptr(old_logp), ptr(adv), ptr(returns), ptr(v), B, A,
+                                           1.0 / float(b_global or B), C.byref(hp), int(shared), ptr(dlogits), A, ptr(dv),
+                                           ptr(sums), None, ptr(sums[3:]), None, ptr(prox_logp), float(is_clip or 0.0),
+                                           current_stream()), "ddrl_ppo_loss_categorical_dc")
+    return dlogits, dv, sums
+
+
+def ppo_loss_gaussian_dc(mu, log_std, actions, old_logp, adv, returns, v, hp: PPOHparams, shared: bool, prox_logp=None,
+                         is_clip: Optional[float] = None, b_global: Optional[int] = None):
+    """The decoupled loss (ddrl_ppo_loss_gaussian_dc) with the statistics on -> (dmu [B,A], dv [B], dlog_std [A], sums [8]),
+    sums as ppo_loss_categorical_dc."""
+    lib = _lib.load()
+    mu, log_std, actions, old_logp, adv, returns, v = map(_f32c, (mu, log_std, actions, old_logp, adv, returns, v))
+    prox_logp = None if prox_logp is None else _f32c(prox_logp)
+    B, A = mu.shape
+    dmu = torch.empty_like(mu)
+    dv = torch.empty(B, dtype=torch.float32, device=mu.device)
+    dls = torch.zeros(A, dtype=torch.float32, device=mu.device)
+    sums = torch.zeros(8, dtype=torch.float32, device=mu.device)
+    check(lib.ddrl_ppo_loss_gaussian_dc(ptr(mu), A, ptr(log_std), ptr(actions), ptr(old_logp), ptr(adv), ptr(returns), ptr(v),
+                                        B, A, 1.0 / float(b_global or B), C.byref(hp), int(shared), ptr(dmu), A, ptr(dv),
+                                        ptr(dls), ptr(sums), None, ptr(sums[3:]), None, ptr(prox_logp), float(is_clip or 0.0),
+                                        current_stream()), "ddrl_ppo_loss_gaussian_dc")
+    return dmu, dv, dls, sums
+
+
+def logp_actions_categorical(logits, actions) -> torch.Tensor:
+    """Log-probs [B] of the taken actions under Categorical(logits), bit-equal to the loss kernel's."""
+    logits, actions = _f32c(logits), _f32c(actions)
+    B, A = logits.shape
+    out = torch.empty(B, dtype=torch.float32, device=logits.device)
+    check(_lib.load().ddrl_logp_actions_categorical(ptr(logits), A, ptr(actions), B, A, ptr(out), current_stream()),
+          "ddrl_logp_actions_categorical")
+    return out
+
+
+def logp_actions_gaussian(mu, log_std, actions) -> torch.Tensor:
+    """Log-probs [B] of the action rows under Normal(mu, exp(log_std)) summed over A, bit-equal to the loss kernel's."""
+    mu, log_std, actions = _f32c(mu), _f32c(log_std), _f32c(actions)
+    B, A = mu.shape
+    out = torch.empty(B, dtype=torch.float32, device=mu.device)
+    check(_lib.load().ddrl_logp_actions_gaussian(ptr(mu), A, ptr(log_std), ptr(actions), B, A, ptr(out), current_stream()),
+          "ddrl_logp_actions_gaussian")
+    return out
+
+
+def net_log_prob(net, states, actions, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """ddrl_net_log_prob: log-probs [B] of `actions` under the current parameters of the PPO module `net`, for `states` as the
+    engine takes them (already normalised under NORM_OBS); written into `out` when given."""
+    net._ensure_engine()
+    keep, arr, n_obs, B = net._obs_ptrs(states)
+    actions = _f32c(actions.to(net._flat.device))
+    if out is None:
+        out = torch.empty(B, dtype=torch.float32, device=net._flat.device)
+    check(_lib.load().ddrl_net_log_prob(net._h, arr, n_obs, B, ptr(actions), ptr(out), current_stream()), "ddrl_net_log_prob")
+    return out
+
+
 def clip_adam(params, grads, m, v, seg_begin: Sequence[int], seg_lr: Sequence[float], step: int, hp: PPOHparams):
     """In-place fused clip_grad_norm_ + Adam over flat fp32 buffers; returns the pre-clip norm (device scalar)."""
     lib = _lib.load()

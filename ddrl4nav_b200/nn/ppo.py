@@ -113,6 +113,14 @@ class PPO(Basenn):
         # forward return its values denormalised
         self.value_rms = ValueRMS() if _flag_option(config_nn, "NORM_VALUE") else None
         self._norm_sums = None          # NORM_VALUE: the float64 moment sums a data-parallel learner all-reduces (+ NORM_OBS's)
+        # decoupled PPO (non-reference, off by default; Hilton, Cobbe & Schulman 2022): the clip is centred on the policy at the
+        # start of the learn call (the proximal log-probs) and the actor term is weighted by exp(prox - old), optionally
+        # truncated at DECOUPLED_IS_CLIP
+        self.decoupled = _flag_option(config_nn, "DECOUPLED_PPO")
+        self.decoupled_is_clip = _positive_option(config_nn, "DECOUPLED_IS_CLIP")
+        if self.decoupled_is_clip is not None and not self.decoupled:
+            raise DDRLError("DECOUPLED_IS_CLIP needs DECOUPLED_PPO=True")
+        self.last_prox_logps = None     # DECOUPLED_PPO: the proximal log-probs [B_local] of the last learn call (persistent)
         self.hp = kernels.make_hparams(
             ppo_clip=_cfg(config_nn, "PPO_CLIP", 0.2), dual_clip=_cfg(config_nn, "DUEL_PPO_CLIP", 3),
             v_coef=_cfg(config_nn, "V_LOSS_THETA", 1.0), ent_coef=_cfg(config_nn, "ENTROPY_LOSS_THETA", 0.05),
@@ -313,7 +321,7 @@ class PPO(Basenn):
             if old_m is not None and old_m.numel() == P:       # keep Adam state across a .to()/re-flatten
                 self._m.copy_(old_m)
                 self._v.copy_(old_v)
-            # {total, actor, v, entropy} (+ {approx KL, clip fraction, -, -} with PPO_STATS): one D2H copy per step
+            # {total, actor, v, entropy} (+ {approx KL, clip fraction, behaviour KL | -, -} with PPO_STATS): one D2H copy per step
             self._loss4 = torch.zeros(8 if self.ppo_stats else 4, dtype=torch.float32, device=dev)
         with torch.no_grad():
             for (pname, p), o in zip(plist, offsets):
@@ -561,10 +569,10 @@ class PPO(Basenn):
         self._peer = st
 
     def _allreduce_grads(self):
-        """Sum of grads[0 : P+4] (P+5 with PPO_STATS) over the ranks, in place: the peer-memory kernel when the buffer is
-        symmetric, else NCCL."""
+        """Sum of grads[0 : P+4] (P+5 with PPO_STATS, P+6 with PPO_STATS and DECOUPLED_PPO) over the ranks, in place: the
+        peer-memory kernel when the buffer is symmetric, else NCCL."""
         st = self._peer
-        tail = 5 if self.ppo_stats else 4
+        tail = (6 if self.decoupled else 5) if self.ppo_stats else 4
         if st is not None and st["grads"] is self._grads:
             st["seq"] += 1
             count = (self._P + tail + 3) // 4 * 4              # the buffer holds P + 8 floats
@@ -601,10 +609,11 @@ class PPO(Basenn):
 
     @_on_device
     def backward_only(self, states, advs, actions, old_logps, returns, b_global=None, obs_unchanged=False, minibatch=False,
-                      old_values=None):
+                      old_values=None, prox_logps=None):
         """forward + fused loss + backward for the local rows; grads (scaled 1/B_global) stay in flat_grads().
         minibatch: the inputs are the persistent minibatch buffers (ddrl_net_backward_minibatch; 0 rows allowed).
         old_values: critic 0's rollout values [B], needed exactly when VALUE_CLIP is set.
+        prox_logps: DECOUPLED_PPO's proximal log-probs [B] (device fp32, read in place), or None for the plain PPO loss.
         This is the engine-level pass: with NORM_OBS it takes `states` as given, so they must already be normalised."""
         self._ensure_engine()
         lib = _lib.load()
@@ -616,9 +625,18 @@ class PPO(Basenn):
         V = len(self._critics)
         if old_values is not None:
             old_values = old_values.to(device=dev, dtype=torch.float32).contiguous()
-        # the old-value pointer goes in before the hyper-parameters (ddrl_net_backward_v / _minibatch_v)
+        if prox_logps is not None and not self.decoupled:
+            raise DDRLError("prox_logps needs DECOUPLED_PPO=True")
+        # the old-value pointer goes in before the hyper-parameters (ddrl_net_backward_v / _minibatch_v); DECOUPLED_PPO adds
+        # the proximal log-probs and the truncation after it (ddrl_net_backward_dc / _minibatch_dc)
         args = args[:9] + (ptr(old_values),) + args[9:]
-        if minibatch:
+        if self.decoupled:
+            args = args[:10] + (ptr(prox_logps), float(self.decoupled_is_clip or 0.0)) + args[10:]
+            if minibatch:
+                check(lib.ddrl_net_backward_minibatch_dc(*args[:-1], current_stream()), "ddrl_net_backward_minibatch_dc")
+            else:
+                check(lib.ddrl_net_backward_dc(*args, current_stream()), "ddrl_net_backward_dc")
+        elif minibatch:
             check(lib.ddrl_net_backward_minibatch_v(*args[:-1], current_stream()), "ddrl_net_backward_minibatch_v")
         else:
             check(lib.ddrl_net_backward_v(*args, current_stream()), "ddrl_net_backward_v")
@@ -725,7 +743,10 @@ class PPO(Basenn):
         NORM_OBS: every step sees the observations normalised with the statistics held when the call started (those the
         Forward module acted with); the call's batch is folded into the statistics once, before the final step's yield.
         NORM_VALUE: the call's return targets are folded into critic 0's target statistics once, at the start, and the head
-        is rescaled to keep its outputs; every step then learns the targets normalised with the new statistics (PopArt)."""
+        is rescaled to keep its outputs; every step then learns the targets normalised with the new statistics (PopArt).
+        DECOUPLED_PPO: the log-probs of the batch under the parameters at the start of the call (after NORM_VALUE's rescale,
+        on the NORM_OBS-normalised batch) are the proximal policy every step clips around; the actor term is weighted by
+        exp(prox - old_logps), and PPO_STATS adds BehaviourKL, the mean of (rho - 1) - log rho with rho = exp(prox - old)."""
         if self.mini_batch_num > 1:
             yield from self._learn_minibatch(data)
             return
@@ -738,16 +759,17 @@ class PPO(Basenn):
             data = self._obs_norm_begin(data, b_global)
         if self.value_rms is not None:
             self._value_norm_begin(data, b_global)
-        options = self.norm_adv or self.value_clip is not None or self.ppo_stats or self.value_rms is not None
+        prox = self._decoupled_begin(data) if self.decoupled else None
+        options = self.norm_adv or self.value_clip is not None or self.ppo_stats or self.value_rms is not None or self.decoupled
         advs, old_values = self._full_batch_inputs(data) if options else (data.advs, None)
         for it in range(self.training_iter_time):
             start_time = time.time()
             if self._dp_world > 1 and not options:
                 self._backward_allreduce(data, b_global, obs_unchanged=it > 0)
             else:
-                # the options (and NORM_VALUE) take the whole (not the segmented) backward, as extra critics do
+                # the options (NORM_VALUE and DECOUPLED_PPO too) take the whole (not the segmented) backward, as extra critics do
                 self.backward_only(data.states, advs, data.actions, data.old_logps, data.values, b_global,
-                                   obs_unchanged=it > 0, old_values=old_values)
+                                   obs_unchanged=it > 0, old_values=old_values, prox_logps=prox)
                 if self._dp_world > 1:
                     self._allreduce_grads()
             loss_log = self._step_and_log(start_time)
@@ -803,6 +825,19 @@ class PPO(Basenn):
                 for k, p in (("weight", self.critic.critic_linear.weight), ("bias", self.critic.critic_linear.bias)))
         self.value_rms.merge(n_global, w, b)
 
+    @_on_device
+    def _decoupled_begin(self, data):
+        """DECOUPLED_PPO at the start of a learn call: the log-probs of the local rows' actions under the current parameters
+        (ddrl_net_log_prob, the backward's training forward and the loss kernels' log-prob) into the persistent buffer
+        last_prox_logps.  Per row: a data-parallel learner needs no collective."""
+        self._ensure_engine()
+        dev = self._flat.device
+        b = len(data.states[0])
+        if self.last_prox_logps is None or self.last_prox_logps.numel() != b or self.last_prox_logps.device != dev:
+            self.last_prox_logps = torch.empty(b, dtype=torch.float32, device=dev)
+        actions = data.actions if torch.is_tensor(data.actions) else torch.as_tensor(np.asarray(data.actions))
+        return kernels.net_log_prob(self, data.states, actions, out=self.last_prox_logps)
+
     def _step_and_log(self, start_time):
         """clip+Adam, then the loss dict of the step from ONE D2H copy (reference: four .item())."""
         loss = self.optimizer_step().tolist()
@@ -812,6 +847,8 @@ class PPO(Basenn):
         if self.ppo_stats:
             loss_log["ApproxKL"] = loss[4]
             loss_log["ClipFrac"] = loss[5]
+            if self.decoupled:
+                loss_log["BehaviourKL"] = loss[6]
         return loss_log
 
     def _kl_stop(self, loss_log):
@@ -863,7 +900,7 @@ class PPO(Basenn):
 
     def _minibatch_sources(self, data):
         """fp32 contiguous device tensors the minibatch rows are gathered from: state slots, actions, old log-probs,
-        advantages, and the return rows [V, B]."""
+        advantages, the return rows [V, B], and VALUE_CLIP's old values and DECOUPLED_PPO's proximal log-probs."""
         dev = self._flat.device
         f = lambda t: (t if torch.is_tensor(t) else torch.as_tensor(np.asarray(t))).to(device=dev, dtype=torch.float32).contiguous()
         n_obs = _lib.load().ddrl_net_num_obs(self._h)
@@ -875,7 +912,9 @@ class PPO(Basenn):
                    advs=f(data.advs), values=values)
         if self.value_clip is not None:
             src["old_values"] = self._old_values(data, src["advs"], values)     # from the raw advantages, once per call
-        if len(src["states"]) + 3 + values.shape[0] + ("old_values" in src) > _lib.GATHER_MAX_JOBS:
+        if self.decoupled:
+            src["prox_logps"] = self.last_prox_logps
+        if len(src["states"]) + 3 + values.shape[0] + ("old_values" in src) + ("prox_logps" in src) > _lib.GATHER_MAX_JOBS:
             raise DDRLError("minibatch gather: %d return rows exceed the job limit" % values.shape[0])
         return src
 
@@ -884,22 +923,23 @@ class PPO(Basenn):
         b_local, M and the shapes stay the same, which is what lets ddrl_net_backward_minibatch replay its graph."""
         dev = self._flat.device
         key = (b_local, self.mini_batch_num, dev, tuple(tuple(t.shape[1:]) for t in src["states"]), tuple(src["actions"].shape[1:]),
-               src["values"].shape[0], "old_values" in src)
+               src["values"].shape[0], "old_values" in src, "prox_logps" in src)
         if self._mb is None or self._mb["key"] != key:
             rows = max(mb_rows, 1)
             e = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
             self._mb = dict(key=key, states=[e(rows, *t.shape[1:]) for t in src["states"]],
                             actions=e(rows, *src["actions"].shape[1:]), old_logps=e(rows), advs=e(rows),
                             values=e(src["values"].shape[0] * rows), zeros=torch.zeros(rows, dtype=torch.float32, device=dev))
-            if "old_values" in src:
-                self._mb["old_values"] = e(rows)
+            for name in ("old_values", "prox_logps"):
+                if name in src:
+                    self._mb[name] = e(rows)
         return self._mb
 
     @_on_device
     def _gather_minibatch(self, src, rows):
         """Gathers the rows `rows` (int32 device) of every source into the minibatch buffers in ONE launch, then normalises
         the gathered advantages in place (NORM_ADV); returns the (states, advs, actions, old_logps, returns [V, n],
-        old_values | None) views backward_only takes."""
+        old_values | None, prox_logps | None) views backward_only takes."""
         mb, n = self._mb, rows.numel()
         V = src["values"].shape[0]
         ret = mb["values"][:V * n]
@@ -907,13 +947,16 @@ class PPO(Basenn):
             pairs = [(s, d) for s, d in zip(src["states"], mb["states"])]
             pairs += [(src["actions"], mb["actions"]), (src["old_logps"], mb["old_logps"]), (src["advs"], mb["advs"])]
             pairs += [(src["values"][v], ret[v * n:(v + 1) * n]) for v in range(V)]
-            if "old_values" in src:
-                pairs.append((src["old_values"], mb["old_values"]))
+            for name in ("old_values", "prox_logps"):
+                if name in src:
+                    pairs.append((src[name], mb[name]))
             kernels.gather_rows(rows, pairs)
         if self.norm_adv:
             self._normalize_advs(mb["advs"][:n], mb["advs"][:n])   # in place: the buffers keep their graph-replay addresses
         old_values = mb["old_values"][:n] if "old_values" in src else None
-        return [t[:n] for t in mb["states"]], mb["advs"][:n], mb["actions"][:n], mb["old_logps"][:n], ret.view(V, n), old_values
+        prox_logps = mb["prox_logps"][:n] if "prox_logps" in src else None
+        return ([t[:n] for t in mb["states"]], mb["advs"][:n], mb["actions"][:n], mb["old_logps"][:n], ret.view(V, n), old_values,
+                prox_logps)
 
     def _learn_minibatch(self, data):
         """TRAINING_ITER_TIME epochs; each draws a permutation of the local rows (net-owned generator) and cuts it into
@@ -932,6 +975,8 @@ class PPO(Basenn):
             data = self._obs_norm_begin(data, sum(b_globals))       # the gathers then read the normalised batch
         if self.value_rms is not None:
             self._value_norm_begin(data, sum(b_globals))
+        if self.decoupled:
+            self._decoupled_begin(data)
         src = self._minibatch_sources(data)
         self._minibatch_buffers(src, b_local, max(sizes))
         if self._mb_gen is None or self._mb_gen.device != dev:
@@ -945,8 +990,9 @@ class PPO(Basenn):
             self.last_minibatch_perms.append(perm)
             for k, ((lo, hi), b_global) in enumerate(zip(plan, b_globals)):
                 start_time = time.time()
-                states, advs, actions, old_logps, returns, old_values = self._gather_minibatch(src, perm[lo:hi])
-                self.backward_only(states, advs, actions, old_logps, returns, b_global, minibatch=True, old_values=old_values)
+                states, advs, actions, old_logps, returns, old_values, prox = self._gather_minibatch(src, perm[lo:hi])
+                self.backward_only(states, advs, actions, old_logps, returns, b_global, minibatch=True, old_values=old_values,
+                                   prox_logps=prox)
                 if self._dp_world > 1:
                     self._allreduce_grads()
                 loss_log = self._step_and_log(start_time)

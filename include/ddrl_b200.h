@@ -203,6 +203,30 @@ int ddrl_ppo_loss_gaussian_vn(const float* mu, int ld, const float* log_std, con
                               int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
                               float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums, const float* old_values,
                               float* stats, const float* value_norm, void* stream);
+/* The same with the decoupled PPO objective (non-reference option DECOUPLED_PPO; Hilton, Cobbe & Schulman 2022): prox_logp
+ * (DEVICE [B], the log-probs of the taken actions under the proximal policy, e.g. ddrl_logp_actions_*) or NULL.  When given,
+ * the ratio is r = exp(logp - prox_logp[b]) (clipped as above, dual clip included) and the actor term and its gradient are
+ * weighted by the behaviour weight w = exp(prox_logp[b] - old_logp[b]), a constant, truncated to min(w, is_clip) when is_clip > 0
+ * (is_clip <= 0: untruncated); the entropy and value terms are unchanged.  stats[0..1] are then taken on r, and stats then holds
+ * 3 floats: stats[2] += inv_B_global * sum((rho - 1) - log rho), rho = exp(prox_logp - old_logp) untruncated (behaviour KL).
+ * NULL: the _vn calls above (is_clip is ignored). */
+int ddrl_ppo_loss_categorical_dc(const float* logits, int ld, const float* actions, const float* old_logp,
+                                 const float* adv, const float* returns, const float* v, int B, int A,
+                                 float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                                 float* dlogits, int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
+                                 const float* value_norm, const float* prox_logp, float is_clip, void* stream);
+int ddrl_ppo_loss_gaussian_dc(const float* mu, int ld, const float* log_std, const float* actions,
+                              const float* old_logp, const float* adv, const float* returns, const float* v,
+                              int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                              float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums, const float* old_values,
+                              float* stats, const float* value_norm, const float* prox_logp, float is_clip, void* stream);
+/* out_logp[b] (DEVICE [B]) = log-prob of the taken action under Categorical(logits) (actions [B], integer-valued) or under
+ * Normal(mu, exp(log_std)) summed over A (actions [B, A]), computed by the same device code as the loss kernels above: equal
+ * logits / means give equal bits.  The proximal log-probs of DECOUPLED_PPO (ddrl_net_log_prob). */
+int ddrl_logp_actions_categorical(const float* logits, int ld, const float* actions, int B, int A, float* out_logp,
+                                  void* stream);
+int ddrl_logp_actions_gaussian(const float* mu, int ld, const float* log_std, const float* actions, int B, int A,
+                               float* out_logp, void* stream);
 
 /* ---- advantage normalisation (non-reference option NORM_ADV) -------------------------------
  * ddrl_adv_moments: m3[0..2] = {n, sum a, sum a^2} of adv[0..n) in fp64 (m3: DEVICE, 3 doubles); a data-parallel learner sums
@@ -292,7 +316,8 @@ int ddrl_net_tensor_info(const ddrl_net* net, int i, char* name, int name_cap,
                          int64_t* shape4, int* ndim, int64_t* offset);
 /* flat device buffers (reference layout/order).  grads has num_params + 8 floats: the tail
  * [P .. P+3] carries {actor, v, entropy, unused} loss sums so one all-reduce covers both; with hp->ppo_stats the backward
- * passes write [P .. P+4] = {actor, v, entropy, approx-KL, clip-fraction} sums.
+ * passes write [P .. P+4] = {actor, v, entropy, approx-KL, clip-fraction} sums (+ the behaviour KL in P+5 with the proximal
+ * log-probs of ddrl_net_backward_dc).
  * grads/m/v may be NULL for an inference-only net. */
 int ddrl_net_bind(ddrl_net* net, float* params, float* grads, float* adam_m, float* adam_v);
 /* Extra value heads (nn/ppo.py:63-64 `add_critic`, :75 `[critic(states) for critic in self._critics]`, :95-105 the V > 1
@@ -323,6 +348,15 @@ int64_t ddrl_net_obs_elems(const ddrl_net* net, int slot);
 int ddrl_net_forward(ddrl_net* net, const float* const* obs, int n_obs, int B, const float* draw,
                      float* actions, float* logp, float* values, float* pi_out, void* stream);
 
+/* DECOUPLED_PPO pre-pass: out_logp [B] (DEVICE) = log-probs of the taken actions (as ddrl_net_backward reads them) under the
+ * net's current parameters, for the observations obs[] (already normalised under NORM_OBS).  Runs the training forward of
+ * ddrl_net_backward micro-batch by micro-batch in the same training workspace (no reallocation between learn calls), then
+ * ddrl_logp_actions_*: for B within one micro-batch the result is bit-equal to the log-probs the next backward pass on the
+ * same parameters computes.  The observations it stages are not reused by a later ddrl_net_backward(obs_unchanged).  The
+ * caller owns out_logp. */
+int ddrl_net_log_prob(ddrl_net* net, const float* const* obs, int n_obs, int B, const float* actions, float* out_logp,
+                      void* stream);
+
 /* Stand-alone encoder forward: features [B, feat] of tower `tower` (0 = prenet / actor.pre, 1 = critic.pre) for the
  * observations obs[] -- replaces AtariPreNet.forward (nn/atari_encoder.py:25-32), NavPreNet / NavPedPreNet.forward
  * (nn/nav_encoder.py:35-43,66-79), NavPreNet1D.forward (nav_encoder.py:115-128), MLPPreNet.forward
@@ -343,6 +377,15 @@ int ddrl_net_backward(ddrl_net* net, const float* const* obs, int n_obs, int B_l
 int ddrl_net_backward_v(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
                         const float* actions, const float* old_logp, const float* adv, const float* returns,
                         const float* old_values, const ddrl_ppo_hparams* hp, int obs_unchanged, void* stream);
+/* ddrl_net_backward_v with the decoupled PPO objective (DECOUPLED_PPO, ddrl_ppo_loss_*_dc): prox_logp [B_local] (DEVICE, e.g.
+ * ddrl_net_log_prob at the start of the learn call; read, not owned) and the truncation is_clip of the behaviour weight
+ * (<= 0: none), or prox_logp NULL (is_clip ignored; this is ddrl_net_backward_v).  With prox_logp and hp->ppo_stats the tail
+ * slot P+5 receives the behaviour-KL sum, a data-parallel learner all-reduces grads[0 .. P+6), and the following
+ * ddrl_net_clip_adam writes loss4_out[6]. */
+int ddrl_net_backward_dc(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
+                         const float* actions, const float* old_logp, const float* adv, const float* returns,
+                         const float* old_values, const float* prox_logp, float is_clip, const ddrl_ppo_hparams* hp,
+                         int obs_unchanged, void* stream);
 /* The same pass in SEGMENTS, for a data-parallel learner that overlaps the gradient all-reduce with the rest of the
  * backward (nn/ppo.py:113-123 runs the actor and the critic backward one after the other; server/backward.py:167 "TODO multi
  * GPU").  Call with segment = 0, 1, ..., *n_segments - 1 in order and the SAME arguments; after segment k returns (stream
@@ -391,9 +434,15 @@ int ddrl_net_backward_minibatch(ddrl_net* net, const float* const* obs, int n_ob
 int ddrl_net_backward_minibatch_v(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
                                   const float* actions, const float* old_logp, const float* adv, const float* returns,
                                   const float* old_values, const ddrl_ppo_hparams* hp, void* stream);
+/* ddrl_net_backward_minibatch_v with prox_logp and is_clip, as ddrl_net_backward_dc (prox_logp NULL: the _v call). */
+int ddrl_net_backward_minibatch_dc(ddrl_net* net, const float* const* obs, int n_obs, int B_local, int B_global,
+                                   const float* actions, const float* old_logp, const float* adv, const float* returns,
+                                   const float* old_values, const float* prox_logp, float is_clip,
+                                   const ddrl_ppo_hparams* hp, void* stream);
 /* second half (nn/ppo.py:115-129): global-norm clip + the two (or one) Adam steps; then refreshes
  * the packed weights.  loss4_out (device, 4 floats, optional) = {total, actor, v, entropy}; with hp->ppo_stats it must
- * hold 6 floats and receives {total, actor, v, entropy, approx KL, clip fraction}. */
+ * hold 6 floats and receives {total, actor, v, entropy, approx KL, clip fraction}; when the last backward pass was
+ * ddrl_net_backward[_minibatch]_dc with prox_logp, it must hold 7 and loss4_out[6] receives the behaviour KL. */
 int ddrl_net_clip_adam(ddrl_net* net, int step, const ddrl_ppo_hparams* hp, float* loss4_out, void* stream);
 /* bytes of device workspace currently held */
 int64_t ddrl_net_workspace_bytes(const ddrl_net* net);
