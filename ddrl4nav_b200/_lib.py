@@ -41,7 +41,7 @@ class ConvDesc(C.Structure):
 
 
 ARCH = {"atari": 0, "nav": 1, "navped": 2, "nav1d": 3, "mlp": 4}
-DIST = {"categorical": 0, "gaussian": 1}
+DIST = {"categorical": 0, "gaussian": 1, "beta": 2}
 GEMM_MODE = {"simt": 0, "tc": 1, "tc2": 2, "tc3": 3}
 
 _P = C.c_void_p
@@ -66,6 +66,7 @@ SIGNATURES = {
     "ddrl_sample_categorical_probs": (_I, [_P, _I, _P, _I, _I, _P, _P, _P]),
     "ddrl_categorical_head": (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P]),
     "ddrl_gaussian_head": (_I, [_P, _I, _P, _P, _I, _I, _P, _P, _P]),
+    "ddrl_beta_head": (_I, [_P, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P]),
     "ddrl_ppo_loss_categorical": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P]),
     "ddrl_ppo_loss_gaussian": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P, _P]),
 "ddrl_ppo_loss_categorical_v": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P, _P,
@@ -82,6 +83,9 @@ SIGNATURES = {
                                        _P, _P, _P, _P, _F, _P]),
     "ddrl_logp_actions_categorical": (_I, [_P, _I, _P, _I, _I, _P, _P]),
     "ddrl_logp_actions_gaussian": (_I, [_P, _I, _P, _P, _I, _I, _P, _P]),
+    "ddrl_ppo_loss_beta": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P, _P,
+                                _P, _P, _F, _P]),
+    "ddrl_logp_actions_beta": (_I, [_P, _I, _P, _P, _P, _I, _I, _P, _P]),
     "ddrl_adv_moments":(_I, [_P, _I, _P, _P]),
     "ddrl_adv_normalize": (_I, [_P, _I, _P, _F, _P, _P]),
     "ddrl_obs_moments_ws_bytes": (_L, [_I, _I]),
@@ -104,6 +108,7 @@ SIGNATURES = {
     "ddrl_net_num_obs": (_I, [_P]),
     "ddrl_net_obs_elems": (_L, [_P, _I]),
     "ddrl_net_set_value_norm": (_I, [_P, _P]),
+    "ddrl_net_set_action_bounds": (_I, [_P, C.POINTER(_F), C.POINTER(_F)]),
     "ddrl_net_forward": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P, _P, _P, _P]),
     "ddrl_net_log_prob": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P]),
     "ddrl_net_encode": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P]),

@@ -9,8 +9,10 @@
 // the (probs, u) -> action map is bit-exact with the reference's numpy expression:
 //     (p.cumsum(axis=1) > u[:,None]).argmax(axis=1)
 // i.e. sequential fp32 prefix sum (__fadd_rn, never reassociated), strict '>', first hit,
-// no hit => 0.  These kernels are tiny (<= 8A+16 B per row); one thread per row.
+// no hit => 0.  These kernels are tiny (<= 8A+16 B per row); one thread per row, except the Beta head's fp64 inverse-CDF
+// solve, which runs one thread per (row, dimension).
 #include "common.cuh"
+#include "beta.cuh"
 
 namespace ddrl {
 
@@ -99,6 +101,41 @@ __global__ void gaussian_head_kernel(const float* __restrict__ mu, int ld, const
   logp[b] = lp;
 }
 
+// Beta head (beta.cuh): thread (r, j) of a block handles dimension j of the block's row r.  Sampling (u given): x = I^-1(u) in
+// fp64, clamped into [eps, 1 - eps], a = low + (high - low) * fp32(x) (mul then add); the row's log-prob is then beta_logp of the
+// emitted action.  Play mode (u null): the mean low + (high - low) * alpha / (alpha + beta), log-prob 0.  conc_out [B, 2A]
+// (optional) receives alpha | beta.
+constexpr int kBetaHeadThreads = 128;
+
+__global__ void __launch_bounds__(kBetaHeadThreads) beta_head_kernel(const float* __restrict__ z, int ld,
+                                                                    const float* __restrict__ low, const float* __restrict__ high,
+                                                                    const float* __restrict__ u, int B, int A,
+                                                                    float* __restrict__ action, float* __restrict__ logp,
+                                                                    float* __restrict__ conc_out) {
+  __shared__ float act_s[kBetaHeadThreads];
+  const int rows = kBetaHeadThreads / A;
+  const int r = threadIdx.x / A, j = threadIdx.x - r * A;
+  const long long b = (long long)blockIdx.x * rows + r;
+  const bool live = r < rows && b < B;
+  if (live) {
+    const float* zr = z + b * ld;
+    const float al = beta_conc(zr[j]), be = beta_conc(zr[A + j]);
+    if (conc_out) { conc_out[b * 2 * A + j] = al; conc_out[b * 2 * A + A + j] = be; }
+    const float w = high[j] - low[j];
+    float a;
+    if (u) {
+      const float x = (float)beta_clamp_x(beta_inc_inv(al, be, u[b * A + j]));
+      a = __fadd_rn(low[j], __fmul_rn(w, x));
+    } else {
+      a = __fadd_rn(low[j], __fmul_rn(w, __fdiv_rn(al, __fadd_rn(al, be))));
+    }
+    action[b * A + j] = a;
+    act_s[threadIdx.x] = a;
+  }
+  __syncthreads();
+  if (live && j == 0) logp[b] = u ? beta_logp(z + b * ld, low, high, act_s + threadIdx.x, A) : 0.f;
+}
+
 }  // namespace ddrl
 
 using namespace ddrl;
@@ -130,5 +167,17 @@ extern "C" int ddrl_gaussian_head(const float* mu, int ld, const float* log_std,
   if (!mu || !log_std || !action || !logp) return DDRL_E_ARG;
   gaussian_head_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(mu, ld, log_std, eps, B, A, action, logp);
   DDRL_LAUNCHED("gaussian_head_kernel");
+  return DDRL_OK;
+}
+
+extern "C" int ddrl_beta_head(const float* head, int ld, const float* low, const float* high, const float* u, int B, int A,
+                              float* action, float* logp, float* conc_out, void* stream) {
+  if (B < 0 || A < 1 || A > kBetaMaxA || ld < 2 * A) return DDRL_E_ARG;
+  if (B == 0) return DDRL_OK;
+  if (!head || !low || !high || !action || !logp) return DDRL_E_ARG;
+  const int rows = kBetaHeadThreads / A;
+  beta_head_kernel<<<ceil_div(B, rows), kBetaHeadThreads, 0, (cudaStream_t)stream>>>(head, ld, low, high, u, B, A, action, logp,
+                                                                                      conc_out);
+  DDRL_LAUNCHED("beta_head_kernel");
   return DDRL_OK;
 }

@@ -114,6 +114,8 @@ struct ddrl_net {
   // NORM_VALUE (ddrl_net_set_value_norm): device {mean32, scale32, sigma32}; critic 0 learns normalised targets and the
   // forward pass returns its values denormalised.  Null: off.
   const float* value_norm = nullptr;
+  // DDRL_DIST_BETA (ddrl_net_set_action_bounds): device [2 x act_dim] = low | high, owned.  Null: not set yet.
+  float* bounds = nullptr;
   // DECOUPLED_PPO with hp->ppo_stats: the last backward pass took proximal log-probs, so its loss tail holds the behaviour KL
   // in slot P+5 and ddrl_net_clip_adam reports it as loss4_out[6]
   bool behaviour_kl = false;
@@ -349,6 +351,10 @@ static void add_encoder_tensors(ddrl_net* n, const std::string& pre, int arch, i
 }
 
 static int round4(int x) { return (x + 3) & ~3; }
+// width of the actor head GEMM: the Beta head emits alpha | beta pre-activations per action dimension
+static int head_n(const ddrl_net* n) { return n->d.dist == DDRL_DIST_BETA ? 2 * n->d.act_dim : n->d.act_dim; }
+// a Beta net cannot run before its action bounds are set
+static bool bounds_missing(const ddrl_net* n) { return n->d.dist == DDRL_DIST_BETA && !n->bounds; }
 
 static Lin make_lin(ddrl_net* n, const std::string& wname, int N, int K, int I, int J, int act) {
   Lin l;
@@ -1481,8 +1487,9 @@ static int forward_chunk(ddrl_net* n, const float* const* obs, long long row0, i
   for (auto& t : n->towers) TRY(tower_forward(n, t, obs, row0, mb, train, s, reuse_obs));
   Tower& ta = n->towers[0];
   Tower& tc = n->towers[n->d.shared ? 0 : 1];
-  const int A = n->d.act_dim, F = n->d.feat;
-  TRY(skinny_fwd(ta.h, F, n->params + n->T[n->t_aw].offset, n->params + n->T[n->t_ab].offset, mb, A, F, n->logits, n->ldA, s));
+  const int F = n->d.feat;
+  TRY(skinny_fwd(ta.h, F, n->params + n->T[n->t_aw].offset, n->params + n->T[n->t_ab].offset, mb, head_n(n), F, n->logits, n->ldA,
+                 s));
   TRY(skinny_fwd(tc.h, F, n->params + n->T[n->t_cw].offset, n->params + n->T[n->t_cb].offset, mb, 1, F, n->vout, 1, s));
   for (size_t k = 0; k < n->extra.size(); ++k)       // [critic(states) for critic in self._critics], nn/ppo.py:75
     TRY(skinny_fwd(tc.h, F, n->extra[k].w, n->extra[k].b, mb, 1, F, n->vout_x + k * (size_t)n->MB, 1, s));
@@ -1498,7 +1505,7 @@ extern "C" int ddrl_net_create(const ddrl_net_desc* desc, ddrl_net** out) {
   if (!desc || !out) return DDRL_E_ARG;
   if (desc->arch < 0 || desc->arch > DDRL_ARCH_MLP || desc->act_dim < 1 || desc->in_ch < 1) return DDRL_E_ARG;
   if (desc->dist == DDRL_DIST_CATEGORICAL && desc->act_dim > 64) return DDRL_E_UNSUPPORTED;
-  if (desc->dist == DDRL_DIST_GAUSSIAN && desc->act_dim > 8) return DDRL_E_UNSUPPORTED;
+  if ((desc->dist == DDRL_DIST_GAUSSIAN || desc->dist == DDRL_DIST_BETA) && desc->act_dim > 8) return DDRL_E_UNSUPPORTED;
   if (desc->arch == DDRL_ARCH_NAVPED && desc->in_ch < 4) return DDRL_E_ARG;
   ddrl_net* n = new ddrl_net();
   n->d = *desc;
@@ -1509,8 +1516,8 @@ extern "C" int ddrl_net_create(const ddrl_net_desc* desc, ddrl_net** out) {
   if (n->d.shared) add_encoder_tensors(n, "prenet.", n->d.arch, n->d.in_ch, F);
   if (n->d.dist == DDRL_DIST_GAUSSIAN) add_tensor(n, "actor.log_std", {n->d.act_dim});
   if (!n->d.shared) add_encoder_tensors(n, "actor.pre.", n->d.arch, n->d.in_ch, F);
-  add_tensor(n, "actor.actor_linear.weight", {n->d.act_dim, F});
-  add_tensor(n, "actor.actor_linear.bias", {n->d.act_dim});
+  add_tensor(n, "actor.actor_linear.weight", {head_n(n), F});
+  add_tensor(n, "actor.actor_linear.bias", {head_n(n)});
   const int64_t critic_begin = n->P;
   add_tensor(n, "critic.critic_linear.weight", {1, F});
   add_tensor(n, "critic.critic_linear.bias", {1});
@@ -1520,7 +1527,7 @@ extern "C" int ddrl_net_create(const ddrl_net_desc* desc, ddrl_net** out) {
   n->t_cw = find_tensor(n, "critic.critic_linear.weight");
   n->t_cb = find_tensor(n, "critic.critic_linear.bias");
   n->t_logstd = find_tensor(n, "actor.log_std");
-  n->ldA = round4(n->d.act_dim);
+  n->ldA = round4(head_n(n));
   // Adam segments: shared -> one optimiser over everything (ppo.py:40); unshared -> actor_optim over
   // actor.* and critic_optim over critic.* (ppo.py:41-42), contiguous in the flat order
   if (n->d.shared) { n->nseg = 1; n->seg_begin[0] = 0; n->seg_begin[1] = n->P; }
@@ -1589,6 +1596,7 @@ extern "C" int ddrl_net_destroy(ddrl_net* n) {
   if (n->h16_base) cudaFree(n->h16_base);
   if (n->amax_dev) cudaFree(n->amax_dev);
   if (n->bias0c) cudaFree(n->bias0c);
+  if (n->bounds) cudaFree(n->bounds);
   delete n;
   return DDRL_OK;
 }
@@ -1674,10 +1682,21 @@ extern "C" int ddrl_net_set_value_norm(ddrl_net* n, const float* applied) {
   return DDRL_OK;
 }
 
+extern "C" int ddrl_net_set_action_bounds(ddrl_net* n, const float* low_host, const float* high_host) {
+  if (!n || !low_host || !high_host || n->d.dist != DDRL_DIST_BETA) return DDRL_E_ARG;
+  const int A = n->d.act_dim;
+  for (int j = 0; j < A; ++j)
+    if (!std::isfinite(low_host[j]) || !std::isfinite(high_host[j]) || !(low_host[j] < high_host[j])) return DDRL_E_ARG;
+  if (!n->bounds) DDRL_CUDA(cudaMalloc(&n->bounds, sizeof(float) * 2 * A));
+  DDRL_CUDA(cudaMemcpy(n->bounds, low_host, sizeof(float) * A, cudaMemcpyHostToDevice));
+  DDRL_CUDA(cudaMemcpy(n->bounds + A, high_host, sizeof(float) * A, cudaMemcpyHostToDevice));
+  return DDRL_OK;
+}
+
 extern "C" int ddrl_net_forward(ddrl_net* n, const float* const* obs, int n_obs, int B, const float* draw, float* actions,
                                 float* logp, float* values, float* pi_out, void* stream) {
   if (!n || B < 0) return DDRL_E_ARG;
-  if (!n->params) return DDRL_E_STATE;
+  if (!n->params || bounds_missing(n)) return DDRL_E_STATE;
   if (B == 0) return DDRL_OK;
   TRY(check_obs(n, obs, n_obs));
   if (!logp || !values || !actions) return DDRL_E_ARG;
@@ -1693,6 +1712,9 @@ extern "C" int ddrl_net_forward(ddrl_net* n, const float* const* obs, int n_obs,
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
       TRY(ddrl_categorical_head(n->logits, n->ldA, draw ? draw + r0 : nullptr, mb, A, actions + r0, logp + r0,
                                 pi_out ? pi_out + r0 * A : nullptr, s));
+    } else if (n->d.dist == DDRL_DIST_BETA) {
+      TRY(ddrl_beta_head(n->logits, n->ldA, n->bounds, n->bounds + A, draw ? draw + r0 * A : nullptr, mb, A, actions + r0 * A,
+                         logp + r0, pi_out ? pi_out + r0 * 2 * A : nullptr, s));
     } else {
       const float* ls = n->params + n->T[n->t_logstd].offset;
       TRY(ddrl_gaussian_head(n->logits, n->ldA, ls, draw ? draw + r0 * A : nullptr, mb, A, actions + r0 * A, logp + r0, s));
@@ -1738,7 +1760,7 @@ extern "C" int ddrl_net_encode(ddrl_net* n, const float* const* obs, int n_obs, 
 extern "C" int ddrl_net_log_prob(ddrl_net* n, const float* const* obs, int n_obs, int B, const float* actions, float* out_logp,
                                  void* stream) {
   if (!n || B < 0) return DDRL_E_ARG;
-  if (!n->params) return DDRL_E_STATE;
+  if (!n->params || bounds_missing(n)) return DDRL_E_STATE;
   if (B == 0) return DDRL_OK;
   TRY(check_obs(n, obs, n_obs));
   if (!actions || !out_logp) return DDRL_E_ARG;
@@ -1754,6 +1776,8 @@ extern "C" int ddrl_net_log_prob(ddrl_net* n, const float* const* obs, int n_obs
     TRY(forward_chunk(n, obs, r0, mb, true, s));
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
       TRY(ddrl_logp_actions_categorical(n->logits, n->ldA, actions + r0, mb, A, out_logp + r0, s));
+    } else if (n->d.dist == DDRL_DIST_BETA) {
+      TRY(ddrl_logp_actions_beta(n->logits, n->ldA, n->bounds, n->bounds + A, actions + r0 * A, mb, A, out_logp + r0, s));
     } else {
       TRY(ddrl_logp_actions_gaussian(n->logits, n->ldA, n->params + n->T[n->t_logstd].offset, actions + r0 * A, mb, A,
                                      out_logp + r0, s));
@@ -1790,6 +1814,11 @@ static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int 
                                        invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
                                        old_values ? old_values + r0 : nullptr, stats, n->value_norm,
                                        prox_logp ? prox_logp + r0 : nullptr, is_clip, s));
+    } else if (n->d.dist == DDRL_DIST_BETA) {
+      TRY(ddrl_ppo_loss_beta(n->logits, n->ldA, n->bounds, n->bounds + A, actions + r0 * A, old_logp + r0, adv + r0, returns + r0,
+                             n->vout, mb, A, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
+                             old_values ? old_values + r0 : nullptr, stats, n->value_norm, prox_logp ? prox_logp + r0 : nullptr,
+                             is_clip, s));
     } else {
       TRY(ddrl_ppo_loss_gaussian_dc(n->logits, n->ldA, n->params + n->T[n->t_logstd].offset, actions + r0 * A, old_logp + r0,
                                     adv + r0, returns + r0, n->vout, mb, A, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv,
@@ -1797,9 +1826,10 @@ static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int 
                                     n->value_norm, prox_logp ? prox_logp + r0 : nullptr, is_clip, s));
     }
     // heads backward (nn/actor.py:91 actor_linear, nn/critic.py:21 critic_linear)
-    TRY(skinny_wgrad(n->dlogits, n->ldA, ta.h, F, mb, A, F, n->grads + n->T[n->t_aw].offset, n->grads + n->T[n->t_ab].offset, s));
+    TRY(skinny_wgrad(n->dlogits, n->ldA, ta.h, F, mb, head_n(n), F, n->grads + n->T[n->t_aw].offset, n->grads + n->T[n->t_ab].offset,
+                     s));
     TRY(skinny_wgrad(n->dv, 1, tc.h, F, mb, 1, F, n->grads + n->T[n->t_cw].offset, n->grads + n->T[n->t_cb].offset, s));
-    TRY(skinny_dgrad(n->dlogits, n->ldA, aw, mb, A, F, ta.dh, F, 0, s));
+    TRY(skinny_dgrad(n->dlogits, n->ldA, aw, mb, head_n(n), F, ta.dh, F, 0, s));
     TRY(skinny_dgrad(n->dv, 1, cw, mb, 1, F, tc.dh, F, n->d.shared ? 1 : 0, s));
     // extra value heads (nn/ppo.py:99-107): returns row k+1, loss added to the value-loss sum, gradient into the shared feature
     for (size_t k = 0; k < n->extra.size(); ++k) {
@@ -1837,7 +1867,7 @@ static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_
                          int* nseg_out, cudaStream_t s) {
   if (!n || !hp || B_local < 0 || B_global < B_local || B_global < 1) return DDRL_E_ARG;
   if (B_local > 0 && !value_clip_ok(hp, old_values)) return DDRL_E_ARG;
-  if (!n->params || !n->grads) return DDRL_E_STATE;
+  if (!n->params || !n->grads || bounds_missing(n)) return DDRL_E_STATE;
   if (!prox_logp) is_clip = 0.f;
   n->behaviour_kl = prox_logp && hp->ppo_stats;
   if (nseg_out) *nseg_out = 1;
@@ -1929,7 +1959,7 @@ extern "C" int ddrl_net_backward_minibatch_dc(ddrl_net* n, const float* const* o
                                               const ddrl_ppo_hparams* hp, void* stream) {
   if (!n || !hp || B_local < 0 || B_global < B_local || B_global < 1) return DDRL_E_ARG;
   if (B_local > 0 && !value_clip_ok(hp, old_values)) return DDRL_E_ARG;
-  if (!n->params || !n->grads) return DDRL_E_STATE;
+  if (!n->params || !n->grads || bounds_missing(n)) return DDRL_E_STATE;
   if (!prox_logp) is_clip = 0.f;
   n->behaviour_kl = prox_logp && hp->ppo_stats;
   cudaStream_t s = (cudaStream_t)stream;

@@ -25,7 +25,11 @@
 //          term and its gradient are weighted by the behaviour weight w = exp(prox - old_logp) (min(w, is_clip) when is_clip > 0):
 //          w * term(r, A) and w * dterm * r.  stats[2] += inv_B*((rho - 1) - log rho), rho = exp(prox - old_logp) untruncated.
 //          With prox null, w = 1 and every product by it is exact: the kernels compute exactly the loss without it.
+// Beta actor (beta.cuh): head z [B, 2A] -> alpha | beta = 1 + softplus(z); the log-prob is beta_logp, the entropy per element is
+// beta_entropy, both in fp64 and rounded once; the gradient follows the softplus chain (digamma for the log-prob, trigamma for
+// the entropy).
 #include "common.cuh"
+#include "beta.cuh"
 
 namespace ddrl {
 
@@ -284,6 +288,77 @@ __global__ void __launch_bounds__(128) ppo_loss_gaussian_kernel(
   }
 }
 
+// Beta actor: the loss of ppo_loss_gaussian_kernel with the Beta log-prob and entropy; dz [B, 2A] replaces dmu / dlog_std
+__global__ void __launch_bounds__(128) ppo_loss_beta_kernel(
+    const float* __restrict__ z, int ld, const float* __restrict__ low, const float* __restrict__ high,
+    const float* __restrict__ actions, const float* __restrict__ old_logp, const float* __restrict__ adv,
+    const float* __restrict__ returns, const float* __restrict__ v, int B, int A, LossParams hp, float* __restrict__ dz, int ld_d,
+    float* __restrict__ dv, float* __restrict__ loss_sums, const float* __restrict__ old_v, float* __restrict__ stats, DetSeq det) {
+  __shared__ float scratch[32];
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  float l_actor = 0.f, l_v = 0.f, l_ent = 0.f, l_kl = 0.f, l_cf = 0.f, l_bkl = 0.f;
+  if (b < B) {
+    const float* zr = z + (size_t)b * ld;
+    const float* ar = actions + (size_t)b * A;
+    const float lp = beta_logp(zr, low, high, ar, A);
+    const float Ai = adv[b];
+    float w;
+    const float log_ratio = decoupled_log_ratio(lp, old_logp, b, hp, stats != nullptr, &w, &l_bkl);
+    const float ratio = expf(log_ratio);
+    float dterm;
+    const float term = surrogate(ratio, Ai, hp, &dterm);
+    l_actor = -(w * term) * hp.inv_B;
+    if (stats) {
+      l_kl = ((ratio - 1.f) - log_ratio) * hp.inv_B;
+      l_cf = fabsf(ratio - 1.f) > hp.ppo_clip ? hp.inv_B : 0.f;
+    }
+    const double w_lp = -hp.inv_B * (w * dterm) * ratio;                          // dLoss/dlogp
+    const double w_ent = hp.shared ? -hp.ent_coef * hp.inv_B / (float)A : 0.f;    // dLoss/dH per element (shared only)
+    double H = 0.0;
+    float* dzr = dz + (size_t)b * ld_d;
+    for (int j = 0; j < A; ++j) {
+      const double al = beta_conc(zr[j]), be = beta_conc(zr[A + j]);
+      const double lo = low[j], wd = (double)high[j] - lo;
+      const double x = beta_clamp_x(((double)ar[j] - lo) / wd);
+      H += beta_entropy(al, be, wd);
+      const double pab = beta_digamma(al + be);
+      double ga = w_lp * (log(x) - beta_digamma(al) + pab);                      // dlogp/dalpha = log x - psi(a) + psi(a+b)
+      double gb = w_lp * (log1p(-x) - beta_digamma(be) + pab);
+      if (hp.shared) {                                                             // dH/dalpha = -(a-1) psi'(a) + (a+b-2) psi'(a+b)
+        const double tab = (al + be - 2.0) * beta_trigamma(al + be);
+        ga += w_ent * (tab - (al - 1.0) * beta_trigamma(al));
+        gb += w_ent * (tab - (be - 1.0) * beta_trigamma(be));
+      }
+      dzr[j] = (float)ga * beta_softplus_grad(zr[j]);
+      dzr[A + j] = (float)gb * beta_softplus_grad(zr[A + j]);
+    }
+    l_ent = (float)H * hp.inv_B / (float)A;     // mean over all [B,A] elements
+    float dl;
+    l_v = value_loss_clipped(returns[b], v[b], old_v, b, hp.value_clip, hp.smooth_l1, hp.value_norm, &dl) * hp.inv_B;
+    dv[b] = dl * hp.inv_B * (hp.shared ? hp.v_coef : 1.f);
+  }
+  l_actor = block_sum(l_actor, scratch);
+  l_v = block_sum(l_v, scratch);
+  l_ent = block_sum(l_ent, scratch);
+  if (stats) {
+    l_kl = block_sum(l_kl, scratch);
+    l_cf = block_sum(l_cf, scratch);
+    if (hp.prox) l_bkl = block_sum(l_bkl, scratch);
+  }
+  if (threadIdx.x == 0) {
+    if (det.ctr) det_enter(det.ctr, blockIdx.x);         // deterministic mode: the blocks add in block order
+    det_add(det.ctr != nullptr, loss_sums + 0, l_actor);
+    det_add(det.ctr != nullptr, loss_sums + 1, l_v);
+    det_add(det.ctr != nullptr, loss_sums + 2, l_ent);
+    if (stats) {
+      det_add(det.ctr != nullptr, stats + 0, l_kl);
+      det_add(det.ctr != nullptr, stats + 1, l_cf);
+      if (hp.prox) det_add(det.ctr != nullptr, stats + 2, l_bkl);
+    }
+    if (det.ctr) det_leave(det.ctr, blockIdx.x, gridDim.x);
+  }
+}
+
 // value loss of one extra critic head (nn/ppo.py:97-104)
 __global__ void __launch_bounds__(128) value_loss_kernel(const float* __restrict__ returns, const float* __restrict__ v, int B,
                                                          LossParams hp, float* __restrict__ dv, float* __restrict__ loss_sums, DetSeq det) {
@@ -321,6 +396,14 @@ __global__ void __launch_bounds__(128) logp_actions_gaussian_kernel(const float*
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   out_logp[b] = gaussian_logp(mu + (size_t)b * ld, log_std, actions + (size_t)b * A, A);
+}
+
+__global__ void __launch_bounds__(128) logp_actions_beta_kernel(const float* __restrict__ z, int ld, const float* __restrict__ low,
+                                                                const float* __restrict__ high, const float* __restrict__ actions,
+                                                                int B, int A, float* __restrict__ out_logp) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  out_logp[b] = beta_logp(z + (size_t)b * ld, low, high, actions + (size_t)b * A, A);
 }
 
 static LossParams make_params(const ddrl_ppo_hparams* hp, float inv_B, int shared, const float* value_norm = nullptr,
@@ -461,4 +544,33 @@ extern "C" int ddrl_ppo_loss_gaussian(const float* mu, int ld, const float* log_
                                       float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums, void* stream) {
   return ddrl_ppo_loss_gaussian_v(mu, ld, log_std, actions, old_logp, adv, returns, v, B, A, inv_B_global, hp, shared, dmu,
                                   ld_d, dv, dlog_std, loss_sums, nullptr, nullptr, stream);
+}
+
+extern "C" int ddrl_ppo_loss_beta(const float* head, int ld, const float* low, const float* high, const float* actions,
+                                  const float* old_logp, const float* adv, const float* returns, const float* v, int B, int A,
+                                  float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dhead, int ld_d, float* dv,
+                                  float* loss_sums, const float* old_values, float* stats, const float* value_norm,
+                                  const float* prox_logp, float is_clip, void* stream) {
+  if (B < 0 || A < 1 || A > kBetaMaxA || ld < 2 * A || ld_d < 2 * A || !hp) return DDRL_E_ARG;
+  if (!value_clip_args_ok(hp, old_values)) return DDRL_E_ARG;
+  if (B == 0) return DDRL_OK;
+  if (!head || !low || !high || !actions || !old_logp || !adv || !returns || !v || !dhead || !dv || !loss_sums) return DDRL_E_ARG;
+  ppo_loss_beta_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(
+      head, ld, low, high, actions, old_logp, adv, returns, v, B, A,
+      make_params(hp, inv_B_global, shared, value_norm, prox_logp, is_clip), dhead, ld_d, dv, loss_sums, old_values, stats,
+      det_seq(1));
+  prof_work((20.0 * A + 20.0 + (old_values ? 4.0 : 0.0) + (prox_logp ? 4.0 : 0.0)) * B);
+  DDRL_LAUNCHED("ppo_loss_beta_kernel");
+  return DDRL_OK;
+}
+
+extern "C" int ddrl_logp_actions_beta(const float* head, int ld, const float* low, const float* high, const float* actions, int B,
+                                      int A, float* out_logp, void* stream) {
+  if (B < 0 || A < 1 || A > kBetaMaxA || ld < 2 * A) return DDRL_E_ARG;
+  if (B == 0) return DDRL_OK;
+  if (!head || !low || !high || !actions || !out_logp) return DDRL_E_ARG;
+  logp_actions_beta_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(head, ld, low, high, actions, B, A, out_logp);
+  prof_work((12.0 * A + 4.0) * B);
+  DDRL_LAUNCHED("logp_actions_beta_kernel");
+  return DDRL_OK;
 }

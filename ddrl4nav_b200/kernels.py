@@ -215,6 +215,49 @@ def logp_actions_gaussian(mu, log_std, actions) -> torch.Tensor:
     return out
 
 
+def beta_head(head, low, high, u: Optional[torch.Tensor], want_conc: bool = True):
+    """(head [B, 2A], low [A], high [A] device, u [B, A] uniforms | None = play mode) -> (action [B, A], logp [B], alpha | beta
+    [B, 2A] or None); ddrl_beta_head."""
+    head, low, high = _f32c(head), _f32c(low), _f32c(high)
+    B, A2 = head.shape
+    A = A2 // 2
+    action = torch.empty((B, A), dtype=torch.float32, device=head.device)
+    logp = torch.empty(B, dtype=torch.float32, device=head.device)
+    conc = torch.empty((B, A2), dtype=torch.float32, device=head.device) if want_conc else None
+    u = None if u is None else _f32c(u)
+    check(_lib.load().ddrl_beta_head(ptr(head), A2, ptr(low), ptr(high), ptr(u), B, A, ptr(action), ptr(logp), ptr(conc),
+                                     current_stream()), "ddrl_beta_head")
+    return action, logp, conc
+
+
+def ppo_loss_beta(head, low, high, actions, old_logp, adv, returns, v, hp: PPOHparams, shared: bool, old_values=None,
+                  value_norm=None, prox_logp=None, is_clip: Optional[float] = None, b_global: Optional[int] = None):
+    """ddrl_ppo_loss_beta with the statistics on -> (dhead [B, 2A], dv [B], sums [8]), sums as ppo_loss_categorical_dc.
+    old_values (VALUE_CLIP; needs hp.value_clip > 0), value_norm (device {mean32, scale32, sigma32}) and prox_logp
+    (DECOUPLED_PPO) are optional."""
+    head, low, high, actions, old_logp, adv, returns, v = map(_f32c, (head, low, high, actions, old_logp, adv, returns, v))
+    old_values, value_norm, prox_logp = (None if t is None else _f32c(t) for t in (old_values, value_norm, prox_logp))
+    B, A2 = head.shape
+    dhead = torch.empty_like(head)
+    dv = torch.empty(B, dtype=torch.float32, device=head.device)
+    sums = torch.zeros(8, dtype=torch.float32, device=head.device)
+    check(_lib.load().ddrl_ppo_loss_beta(ptr(head), A2, ptr(low), ptr(high), ptr(actions), ptr(old_logp), ptr(adv), ptr(returns),
+                                         ptr(v), B, A2 // 2, 1.0 / float(b_global or B), C.byref(hp), int(shared), ptr(dhead), A2,
+                                         ptr(dv), ptr(sums), ptr(old_values), ptr(sums[3:]), ptr(value_norm), ptr(prox_logp),
+                                         float(is_clip or 0.0), current_stream()), "ddrl_ppo_loss_beta")
+    return dhead, dv, sums
+
+
+def logp_actions_beta(head, low, high, actions) -> torch.Tensor:
+    """Log-probs [B] of the action rows [B, A] under the Beta head [B, 2A], bit-equal to the loss and head kernels'."""
+    head, low, high, actions = map(_f32c, (head, low, high, actions))
+    B, A2 = head.shape
+    out = torch.empty(B, dtype=torch.float32, device=head.device)
+    check(_lib.load().ddrl_logp_actions_beta(ptr(head), A2, ptr(low), ptr(high), ptr(actions), B, A2 // 2, ptr(out),
+                                             current_stream()), "ddrl_logp_actions_beta")
+    return out
+
+
 def net_log_prob(net, states, actions, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """ddrl_net_log_prob: log-probs [B] of `actions` under the current parameters of the PPO module `net`, for `states` as the
     engine takes them (already normalised under NORM_OBS); written into `out` when given."""

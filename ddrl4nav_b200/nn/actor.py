@@ -1,11 +1,18 @@
 """Actor heads -- USTC_lab/nn/actor.py:10-101.
 
 `pre` is registered before `actor_linear`, and GaussionActor's `log_std` is a direct Parameter
-(so it precedes everything in named_parameters()), exactly as in the reference."""
+(so it precedes everything in named_parameters()), exactly as in the reference.  BetaActor is this library's own
+(non-reference) head for bounded continuous actions."""
+import numpy as np
 import torch
 from torch import nn
+from torch.distributions.beta import Beta
 from torch.distributions.categorical import Categorical
 from torch.distributions.normal import Normal
+from torch.distributions.transformed_distribution import TransformedDistribution
+from torch.distributions.transforms import AffineTransform
+
+from .._lib import DDRLError
 
 
 class Actor(nn.Module):
@@ -84,3 +91,60 @@ class CategoricalActor(*_reference_bases("CategoricalActor")):
 
     def _log_prob_from_distribution(self, pi, act):
         return pi.log_prob(act)
+
+
+def _bound_list(v, n, what):
+    vals = list(v) if isinstance(v, (list, tuple, np.ndarray, torch.Tensor)) else [v] * n
+    if len(vals) != n:
+        raise DDRLError("%s must be a number or a sequence of %d numbers (got %r)" % (what, n, v))
+    out = []
+    for x in vals:
+        x = x.item() if isinstance(x, (np.generic, torch.Tensor)) else x
+        if isinstance(x, bool) or not isinstance(x, (int, float)) or not abs(x) <= float(np.finfo(np.float32).max):
+            raise DDRLError("%s must hold finite fp32 numbers (got %r)" % (what, v))
+        out.append(float(np.float32(x)))
+    return tuple(out)
+
+
+class BetaActor(Actor):
+    """Beta policy on [low_j, high_j] per action dimension (Chou, Maturana & Scherer, ICML 2017): actor_linear is
+    Linear(F, 2A), columns [0, A) give alpha = 1 + softplus(.) and columns [A, 2A) beta = 1 + softplus(.).  Every sample lies
+    inside the bounds, so no action is ever clipped.  low / high (numbers or length-A sequences, finite, low < high) are
+    configuration: they are not parameters, not in the state_dict and not in the weight blob, so a predictor must be built
+    with the learner's bounds.
+
+    Not derived from a reference class: the reference's ForwardThread only knows Gaussian and Categorical actors; a Beta net
+    is served by PPO.act, ForwardModule and server.threads.ForwardThread, which do not dispatch on the actor type."""
+    DIST = "beta"
+
+    def __init__(self, action_output_dim=1, device="cpu", soft_max_grid=True, last_input_dim=512, pre=None,
+                 nn_dtype=torch.float32, low=-1.0, high=1.0):
+        Actor.__init__(self, pre=pre, device=device)
+        if isinstance(action_output_dim, bool) or not isinstance(action_output_dim, (int, np.integer)) or action_output_dim < 1:
+            raise DDRLError("BetaActor needs action_output_dim >= 1 (got %r)" % (action_output_dim,))
+        self.action_output_dim = int(action_output_dim)
+        self.action_low = _bound_list(low, self.action_output_dim, "low")
+        self.action_high = _bound_list(high, self.action_output_dim, "high")
+        if not all(lo < hi for lo, hi in zip(self.action_low, self.action_high)):
+            raise DDRLError("BetaActor needs low < high in every dimension (got low=%r, high=%r)" % (low, high))
+        self.actor_linear = nn.Linear(last_input_dim, 2 * self.action_output_dim)
+
+    def bounds(self, device):
+        """(low [A], high [A]) fp32 tensors on `device`."""
+        f = lambda v: torch.tensor(v, dtype=torch.float32, device=device)
+        return f(self.action_low), f(self.action_high)
+
+    def distribution(self, conc):
+        """Beta(alpha, beta) mapped onto [low, high], from the concentrations alpha | beta [B, 2A] of the head kernel."""
+        low, high = self.bounds(conc.device)
+        A = self.action_output_dim
+        return TransformedDistribution(Beta(conc[:, :A], conc[:, A:]), AffineTransform(low, high - low))
+
+    def _distribution(self, head, play_mode=False):
+        from .. import kernels
+        low, high = self.bounds(head.device)
+        mean, _, conc = kernels.beta_head(head, low, high, None)
+        return mean if play_mode else self.distribution(conc)
+
+    def _log_prob_from_distribution(self, pi, act):
+        return pi.log_prob(act).sum(axis=-1)

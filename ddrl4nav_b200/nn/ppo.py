@@ -169,13 +169,18 @@ class PPO(Basenn):
     def _encoder(self):
         return self.prenet if self.prenet is not None else self.actor.pre
 
+    def _act_dim(self):
+        """Action dimensions A: the Beta head emits alpha | beta pre-activations, 2A columns."""
+        n = self.actor.actor_linear.out_features
+        return n // 2 if self.actor.DIST == "beta" else n
+
     def _spec(self):
         enc = self._encoder()
         if enc is None or getattr(enc, "ARCH", None) is None:
             raise DDRLError("PPO needs a ddrl4nav_b200 encoder (AtariPreNet / NavPreNet / NavPedPreNet / NavPreNet1D / MLPPreNet)")
         if self.prenet is None and type(self.critic.pre) is not type(enc):
             raise DDRLError("unshared mode needs the same encoder family in actor.pre and critic.pre")
-        return dict(arch=enc.ARCH, in_ch=enc.engine_in_ch(), act_dim=self.actor.actor_linear.out_features,
+        return dict(arch=enc.ARCH, in_ch=enc.engine_in_ch(), act_dim=self._act_dim(),
                     dist=self.actor.DIST, shared=self.prenet is not None, feat=self.actor.actor_linear.in_features,
                     laser_ch=int(getattr(enc, "laser_channel", 0)))
 
@@ -283,6 +288,10 @@ class PPO(Basenn):
         h = C.c_void_p()
         check(lib.ddrl_net_create(C.byref(desc), C.byref(h)), "ddrl_net_create")
         self._h = h
+        if s["dist"] == "beta":
+            A = s["act_dim"]
+            check(lib.ddrl_net_set_action_bounds(h, (C.c_float * A)(*self.actor.action_low), (C.c_float * A)(*self.actor.action_high)),
+                  "ddrl_net_set_action_bounds")
         if self.obs_rms is not None:
             try:
                 self.obs_rms.bind(lib.ddrl_net_num_obs(h), lambda i: lib.ddrl_net_obs_elems(h, i), dev)
@@ -456,9 +465,9 @@ class PPO(Basenn):
     def act(self, states, draw=None, play_mode=False, want_pi=False):
         """Fused compute body of ForwardThread.run (server/forward.py:128-146).
 
-        draw: uniforms [B] (categorical) or standard normals [B,A] (gaussian); generated on the device
-        when None and not play_mode.  Returns (actions [B] | [B,A], logps [B], values [V,B,1][, pi]); V = number of
-        critics (1 unless add_critic was called)."""
+        draw: uniforms [B] (categorical), standard normals [B,A] (gaussian) or uniforms [B,A] (beta); generated on the
+        device when None and not play_mode.  Returns (actions [B] | [B,A], logps [B], values [V,B,1][, pi]); V = number of
+        critics (1 unless add_critic was called); pi = probs [B,A], mu [B,A] or alpha | beta [B,2A]."""
         self._ensure_engine()
         lib = _lib.load()
         if self.obs_rms is not None:
@@ -467,19 +476,21 @@ class PPO(Basenn):
             self.value_rms.refresh()
         keep, arr, n_obs, B = self._obs_ptrs(states)
         dev = self._flat.device
-        A = self.actor.actor_linear.out_features
-        gauss = self.actor.DIST == "gaussian"
+        A = self._act_dim()
+        dist_name = self.actor.DIST
         if play_mode:
             draw = None
+        elif draw is None and dist_name == "categorical":
+            draw = torch.rand(B, device=dev)
         elif draw is None:
-            draw = torch.randn(B, A, device=dev) if gauss else torch.rand(B, device=dev)
+            draw = (torch.randn if dist_name == "gaussian" else torch.rand)(B, A, device=dev)
         else:
             draw = draw.to(device=dev, dtype=torch.float32).contiguous()
-        actions = torch.empty((B, A) if gauss else (B,), dtype=torch.float32, device=dev)
+        actions = torch.empty((B,) if dist_name == "categorical" else (B, A), dtype=torch.float32, device=dev)
         logps = torch.empty(B, dtype=torch.float32, device=dev)
         V = len(self._critics)
         values = torch.empty(V, B, dtype=torch.float32, device=dev)       # shared mode: the engine fills all V rows
-        pi = torch.empty((B, A), dtype=torch.float32, device=dev) if want_pi else None
+        pi = torch.empty((B, 2 * A if dist_name == "beta" else A), dtype=torch.float32, device=dev) if want_pi else None
         check(lib.ddrl_net_forward(self._h, arr, n_obs, B, ptr(draw), ptr(actions), ptr(logps), ptr(values), ptr(pi),
                                    current_stream()), "ddrl_net_forward")
         if V > 1 and self.prenet is None:                                  # unshared: each extra critic on its own engine
@@ -502,10 +513,13 @@ class PPO(Basenn):
 
     def forward(self, states, act=None, play_mode=False):
         """Reference-shaped output: ((pi, log_p), [values [B,1]]) with pi = Categorical / Normal, or the raw
-        softmax / mu tensor in play mode (nn/actor.py:58-67,90-98)."""
-        _, _, values, pi_raw = self.act(states, draw=None, play_mode=True, want_pi=True)
+        softmax / mu tensor in play mode (nn/actor.py:58-67,90-98).  BetaActor: the Beta mapped onto the bounds
+        (BetaActor.distribution), or the mean action [B,A] in play mode."""
+        mean, _, values, pi_raw = self.act(states, draw=None, play_mode=True, want_pi=True)
         if self.actor.DIST == "categorical":
             pi = pi_raw if play_mode else Categorical(pi_raw)
+        elif self.actor.DIST == "beta":
+            pi = mean if play_mode else self.actor.distribution(pi_raw)
         else:
             pi = pi_raw if play_mode else Normal(pi_raw, torch.exp(self.actor.log_std.detach()))
         log_p = None

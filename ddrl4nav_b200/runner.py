@@ -6,8 +6,21 @@ from types import SimpleNamespace
 
 import torch
 
-from .nn import (PPO, AtariPreNet, CategoricalActor, Critic, GaussionActor, MLPPreNet, NavPedPreNet, NavPreNet,
+from .nn import (PPO, AtariPreNet, BetaActor, CategoricalActor, Critic, GaussionActor, MLPPreNet, NavPedPreNet, NavPreNet,
                  NavPreNet1D)
+
+
+def _bounds_kwargs(actor_cls, config_nn):
+    """BetaActor's action interval from the optional config_nn.ACTION_LOW / ACTION_HIGH (numbers or length-A sequences;
+    BetaActor validates them).  Other actors take no bounds."""
+    if actor_cls is not BetaActor:
+        return {}
+    kw = {}
+    for key, arg in (("ACTION_LOW", "low"), ("ACTION_HIGH", "high")):
+        v = getattr(config_nn, key, None)
+        if v is not None:
+            kw[arg] = v
+    return kw
 
 
 def create_net(configs):
@@ -20,7 +33,8 @@ def create_net(configs):
 
     def heads(pre_a, pre_c):
         actor = actor_cls(action_output_dim=config_nn.ACTION_OUTPUT_DIM, device=dev, soft_max_grid=config_nn.SOFT_MAX_GRID,
-                          last_input_dim=feat, nn_dtype=config_nn.MODULE_TENSOR_DTYPE, pre=pre_a)
+                          last_input_dim=feat, nn_dtype=config_nn.MODULE_TENSOR_DTYPE, pre=pre_a,
+                          **_bounds_kwargs(actor_cls, config_nn))
         return actor, Critic(device=dev, last_input_dim=feat, pre=pre_c)
 
     share = config_nn.SHARE_CNN_NET
@@ -58,12 +72,16 @@ _KINDS = {
     "navimg": (lambda: NavPreNet(image_channel=1), "categorical", 28, True),        # C5
     "navped": (lambda: NavPedPreNet(image_channel=4), "categorical", 28, True),
     "mlp": (lambda: MLPPreNet(4, 128), "categorical", 2, False),
+    # NON-reference Beta actor on [ACTION_LOW, ACTION_HIGH] (default [-1, 1]) per dimension: C2's encoder, and C5's
+    "navlaser_beta": (lambda: NavPreNet1D(image_channel=3), "beta", 2, False),
+    "navimg_beta": (lambda: NavPreNet(image_channel=1), "beta", 2, True),
 }
 
 
 def make_net(kind: str, device="cuda", gemm_mode=None, **hyper):
     """PPO net of one of the named configurations with the reference's default hyper-parameters
-    (config/config_nn.py:27-57); `hyper` overrides ConfigNN attribute names (e.g. TRAINING_ITER_TIME=1)."""
+    (config/config_nn.py:27-57); `hyper` overrides ConfigNN attribute names (e.g. TRAINING_ITER_TIME=1, or ACTION_LOW /
+    ACTION_HIGH for the Beta kinds)."""
     mk, dist, act_dim, shared = _KINDS[kind]
     cfg_nn = dict(SHARE_CNN_NET=shared, PPO_CLIP=0.2, DUEL_PPO_CLIP=3, V_LOSS_THETA=1.0, ENTROPY_LOSS_THETA=0.05,
                   CLIP_GRID=True, CLIP_GRID_NUM=0.5, SMOOTH_L1_LOSS=False, LEARNING_RATE=2e-4, ACTOR_LEARNING_RATE=5e-5,
@@ -74,13 +92,14 @@ def make_net(kind: str, device="cuda", gemm_mode=None, **hyper):
     config_nn = SimpleNamespace(**cfg_nn)
     config = SimpleNamespace(DEVICE=device, TASK_NAME="t-127.0.0.1", MODULE_KEY="MODEL")
     feat = 128 if kind == "mlp" else 512
-    actor_cls = GaussionActor if dist == "gaussian" else CategoricalActor
+    actor_cls = {"gaussian": GaussionActor, "beta": BetaActor}.get(dist, CategoricalActor)
+    bounds = _bounds_kwargs(actor_cls, config_nn)
     if shared:
-        actor = actor_cls(action_output_dim=act_dim, device=device, last_input_dim=feat)
+        actor = actor_cls(action_output_dim=act_dim, device=device, last_input_dim=feat, **bounds)
         critic = Critic(device=device, last_input_dim=feat)
         prenet = mk()
     else:
-        actor = actor_cls(action_output_dim=act_dim, device=device, last_input_dim=feat, pre=mk())
+        actor = actor_cls(action_output_dim=act_dim, device=device, last_input_dim=feat, pre=mk(), **bounds)
         critic = Critic(device=device, last_input_dim=feat, pre=mk())
         prenet = None
     net = PPO(actor, critic, prenet, None, config, config_nn)

@@ -36,7 +36,12 @@ enum ddrl_arch {               /* encoder family (USTC_lab/nn/__init__.py:12-18)
   DDRL_ARCH_NAV1D = 3,         /* NavPreNet1D   nn/nav_encoder.py:82-128 */
   DDRL_ARCH_MLP = 4            /* MLPPreNet     nn/mlp_encoder.py:12-29 */
 };
-enum ddrl_dist { DDRL_DIST_CATEGORICAL = 0, DDRL_DIST_GAUSSIAN = 1 };   /* nn/actor.py:75,43 */
+enum ddrl_dist {
+  DDRL_DIST_CATEGORICAL = 0,   /* nn/actor.py:75 */
+  DDRL_DIST_GAUSSIAN = 1,      /* nn/actor.py:43 */
+  DDRL_DIST_BETA = 2           /* non-reference: Beta on [low_j, high_j] per action dimension (ddrl4nav_b200/nn/actor.py BetaActor);
+                                  act_dim = A <= 8 dimensions, head width 2A; needs ddrl_net_set_action_bounds */
+};
 enum ddrl_gemm_mode {
   DDRL_GEMM_SIMT_F32 = 0,      /* CUDA-core fp32 FMA (reference / fallback-free baseline) */
   DDRL_GEMM_TC_3XTF32 = 1,     /* tcgen05 kind::tf32, hi/lo split in shared memory, one tile per CTA (gemm_tc.cu) */
@@ -158,6 +163,14 @@ int ddrl_categorical_head(const float* logits, int ld, const float* u, int B, in
  * logp = sum_j Normal(mu,std).log_prob(a); eps NULL => play mode (a = mu, logp = 0). */
 int ddrl_gaussian_head(const float* mu, int ld, const float* log_std, const float* eps, int B, int A,
                        float* action, float* logp, void* stream);
+/* Beta head (non-reference): head [B, 2A] (row stride ld >= 2A), alpha_j = 1 + softplus(head[:, j]), beta_j = 1 +
+ * softplus(head[:, A + j]) (torch's F.softplus), A <= 8; low / high DEVICE [A].  u [B, A] uniforms: x = I^-1_{alpha,beta}(u)
+ * (the inverse regularised incomplete beta, fp64, capped iterations), clamped into [1e-6, 1 - 1e-6], action = low + (high -
+ * low) * fp32(x) (mul, then add), logp = the Beta log-prob of that action (ddrl_logp_actions_beta's bits).  A non-finite
+ * concentration or u gives a NaN action and log-prob.  u NULL => play mode: action = low + (high - low) * alpha / (alpha + beta),
+ * logp = 0.  conc_out (optional, [B, 2A]) receives alpha | beta. */
+int ddrl_beta_head(const float* head, int ld, const float* low, const float* high, const float* u, int B, int A,
+                   float* action, float* logp, float* conc_out, void* stream);
 
 /* ---- K6: fused PPO loss forward + backward --------------------------------------------
  * replaces nn/ppo.py:85-108 (+ the head part of autograd).  Per sample: dual-clip surrogate,
@@ -220,6 +233,16 @@ int ddrl_ppo_loss_gaussian_dc(const float* mu, int ld, const float* log_std, con
                               int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
                               float* dmu, int ld_d, float* dv, float* dlog_std, float* loss_sums, const float* old_values,
                               float* stats, const float* value_norm, const float* prox_logp, float is_clip, void* stream);
+/* Beta actor (non-reference): the loss of ddrl_ppo_loss_gaussian_dc, every option included, with the Beta head of
+ * ddrl_beta_head (head [B, 2A], low / high DEVICE [A], actions [B, A] in env units).  logp = sum_j (alpha-1) log x + (beta-1)
+ * log1p(-x) - lbeta(alpha, beta) - log(high - low), x = clamp((a - low) / (high - low), 1e-6, 1 - 1e-6), in fp64 rounded once;
+ * entropy per element H(Beta(alpha, beta)) + log(high - low), loss_sums[2] its mean over [B, A].  dhead [B, 2A] (row stride
+ * ld_d >= 2A) receives d(loss)/d(head) through the softplus; the entropy term reaches it only when shared. */
+int ddrl_ppo_loss_beta(const float* head, int ld, const float* low, const float* high, const float* actions,
+                       const float* old_logp, const float* adv, const float* returns, const float* v, int B, int A,
+                       float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dhead, int ld_d, float* dv,
+                       float* loss_sums, const float* old_values, float* stats, const float* value_norm, const float* prox_logp,
+                       float is_clip, void* stream);
 /* out_logp[b] (DEVICE [B]) = log-prob of the taken action under Categorical(logits) (actions [B], integer-valued) or under
  * Normal(mu, exp(log_std)) summed over A (actions [B, A]), computed by the same device code as the loss kernels above: equal
  * logits / means give equal bits.  The proximal log-probs of DECOUPLED_PPO (ddrl_net_log_prob). */
@@ -227,6 +250,9 @@ int ddrl_logp_actions_categorical(const float* logits, int ld, const float* acti
                                   void* stream);
 int ddrl_logp_actions_gaussian(const float* mu, int ld, const float* log_std, const float* actions, int B, int A,
                                float* out_logp, void* stream);
+/* the same for the Beta actor (actions [B, A], head / low / high as ddrl_ppo_loss_beta) */
+int ddrl_logp_actions_beta(const float* head, int ld, const float* low, const float* high, const float* actions, int B, int A,
+                           float* out_logp, void* stream);
 
 /* ---- advantage normalisation (non-reference option NORM_ADV) -------------------------------
  * ddrl_adv_moments: m3[0..2] = {n, sum a, sum a^2} of adv[0..n) in fp64 (m3: DEVICE, 3 doubles); a data-parallel learner sums
@@ -335,6 +361,11 @@ int ddrl_net_set_extra_critics(ddrl_net* net, int count, const float* const* w, 
  * While set, the backward passes normalise critic 0's targets (ddrl_ppo_loss_*_vn), ddrl_net_forward returns critic 0's
  * values as v * sigma32 + mean32 (two roundings), and ddrl_net_backward_segment returns DDRL_E_ARG. */
 int ddrl_net_set_value_norm(ddrl_net* net, const float* applied);
+/* DDRL_DIST_BETA: the action interval [low_host[j], high_host[j]] of each of the act_dim dimensions (HOST arrays, copied into
+ * a net-owned device buffer by a synchronous cudaMemcpy before the call returns).  Every bound must be finite and low < high,
+ * else DDRL_E_ARG; another distribution: DDRL_E_ARG.  Until it is called, ddrl_net_forward, ddrl_net_log_prob and the backward
+ * passes of a Beta net return DDRL_E_STATE.  Captured graphs read the buffer when they replay, so new bounds need no recapture. */
+int ddrl_net_set_action_bounds(ddrl_net* net, const float* low_host, const float* high_host);
 /* tell the net the flat params were changed behind its back (load_state_dict, updatenn_by_redis) */
 int ddrl_net_params_changed(ddrl_net* net);
 /* number of observation slots and per-sample element count of each (for argument checking) */
@@ -342,9 +373,9 @@ int ddrl_net_num_obs(const ddrl_net* net);
 int64_t ddrl_net_obs_elems(const ddrl_net* net, int slot);
 
 /* Forward module compute body (server/forward.py:128-146): obs[i] fp32 device [B, ...] in the
- * reference's NCHW/state-list order; draw = uniforms [B] (categorical) or N(0,1) [B,A]
- * (gaussian), NULL => play mode.  Outputs: actions [B] or [B,A]; logp [B]; values [B] (the
- * caller views it as [V=1,B,1]); pi_out (optional) probs [B,A] or mu [B,A]. */
+ * reference's NCHW/state-list order; draw = uniforms [B] (categorical), N(0,1) [B,A]
+ * (gaussian) or uniforms [B,A] (beta), NULL => play mode.  Outputs: actions [B] or [B,A]; logp [B]; values [B] (the
+ * caller views it as [V=1,B,1]); pi_out (optional) probs [B,A], mu [B,A] or alpha | beta [B,2A]. */
 int ddrl_net_forward(ddrl_net* net, const float* const* obs, int n_obs, int B, const float* draw,
                      float* actions, float* logp, float* values, float* pi_out, void* stream);
 
