@@ -65,6 +65,7 @@ SIGNATURES = {
     "ddrl_easybytes_encode_replies": (_I, [_P, _I, _P, _P, _I, _I, _I, _I, _P, _P]),
     "ddrl_sample_categorical_probs": (_I, [_P, _I, _P, _I, _I, _P, _P, _P]),
     "ddrl_categorical_head": (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P]),
+    "ddrl_categorical_head_m": (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P, _P]),
     "ddrl_gaussian_head": (_I, [_P, _I, _P, _P, _I, _I, _P, _P, _P]),
     "ddrl_beta_head": (_I, [_P, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P]),
     "ddrl_ppo_loss_categorical": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P]),
@@ -81,7 +82,10 @@ SIGNATURES = {
                                           _P, _P, _P, _F, _P]),
     "ddrl_ppo_loss_gaussian_dc": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P,
                                        _P, _P, _P, _P, _F, _P]),
+    "ddrl_ppo_loss_categorical_m": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P,
+                                         _P, _P, _P, _F, _P, _P]),
     "ddrl_logp_actions_categorical": (_I, [_P, _I, _P, _I, _I, _P, _P]),
+    "ddrl_logp_actions_categorical_m": (_I, [_P, _I, _P, _I, _I, _P, _P, _P]),
     "ddrl_logp_actions_gaussian": (_I, [_P, _I, _P, _P, _I, _I, _P, _P]),
     "ddrl_ppo_loss_beta": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P, _P,
                                 _P, _P, _F, _P]),
@@ -109,6 +113,7 @@ SIGNATURES = {
     "ddrl_net_obs_elems": (_L, [_P, _I]),
     "ddrl_net_set_value_norm": (_I, [_P, _P]),
     "ddrl_net_set_action_bounds": (_I, [_P, C.POINTER(_F), C.POINTER(_F)]),
+    "ddrl_net_set_action_mask": (_I, [_P, _I]),
     "ddrl_net_forward": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P, _P, _P, _P]),
     "ddrl_net_log_prob": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P]),
     "ddrl_net_encode": (_I, [_P, C.POINTER(_P), _I, _I, _I, _P, _P]),

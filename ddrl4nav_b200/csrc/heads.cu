@@ -11,28 +11,34 @@
 // i.e. sequential fp32 prefix sum (__fadd_rn, never reassociated), strict '>', first hit,
 // no hit => 0.  These kernels are tiny (<= 8A+16 B per row); one thread per row, except the Beta head's fp64 inverse-CDF
 // solve, which runs one thread per (row, dimension).
+// ACTION_MASK (categorical.cuh): the categorical head takes an optional mask [B, A]; the draw then inverts the CDF of the masked
+// q, and no hit gives the first allowed action (0 without a mask, as above), so a masked action is never emitted.
 #include "common.cuh"
 #include "beta.cuh"
+#include "categorical.cuh"
 
 namespace ddrl {
 
 constexpr float kEps = 1.1920928955078125e-07f;   // torch.finfo(float32).eps
 constexpr float kLogSqrt2Pi = 0.918938533204672741780329736406f;
 
-__device__ __forceinline__ int inverse_cdf(const float* __restrict__ p, int A, float u) {
+// mask (categorical_row_mask) / j0 (categorical_first_allowed): only allowed actions are hits, and no hit gives j0
+__device__ __forceinline__ int inverse_cdf(const float* __restrict__ p, int A, float u, const float* __restrict__ mask = nullptr,
+                                           int j0 = 0) {
   float c = 0.f;
   for (int j = 0; j < A; ++j) {
     c = __fadd_rn(c, p[j]);
-    if (c > u) return j;
+    if (c > u && categorical_allowed(mask, j)) return j;
   }
-  return 0;   // numpy argmax of an all-False row
+  return j0;  // numpy argmax of an all-False row (0 without a mask)
 }
 
-__device__ __forceinline__ int argmax_first(const float* __restrict__ p, int A) {
-  int best = 0;
-  float bv = p[0];
-  for (int j = 1; j < A; ++j)
-    if (p[j] > bv) { bv = p[j]; best = j; }
+__device__ __forceinline__ int argmax_first(const float* __restrict__ p, int A, const float* __restrict__ mask = nullptr,
+                                            int j0 = 0) {
+  int best = j0;
+  float bv = p[j0];
+  for (int j = j0 + 1; j < A; ++j)
+    if (categorical_allowed(mask, j) && p[j] > bv) { bv = p[j]; best = j; }
   return best;
 }
 
@@ -53,28 +59,26 @@ __global__ void sample_probs_kernel(const float* __restrict__ probs, int ld, con
 
 constexpr int kMaxA = 64;
 
-// logits -> softmax -> Categorical(probs): q = p / sum(p); logits' = log(clamp(q, eps, 1-eps))
+// logits -> softmax -> Categorical(probs): q = p / sum(p); logits' = log(clamp(q, eps, 1-eps)).  mask: [B, A] (row stride A) or
+// null (categorical.cuh)
 __global__ void categorical_head_kernel(const float* __restrict__ logits, int ld, const float* __restrict__ u, int B, int A,
                                         float* __restrict__ action, float* __restrict__ logp,
-                                        float* __restrict__ probs_out) {
+                                        float* __restrict__ probs_out, const float* __restrict__ mask) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const float* x = logits + (size_t)b * ld;
+  const float* mk = categorical_row_mask(mask ? mask + (size_t)b * A : nullptr, A);
+  const int j0 = categorical_first_allowed(mk, A);
   float q[kMaxA];
-  float m = x[0];
-  for (int j = 1; j < A; ++j) m = fmaxf(m, x[j]);
-  float s = 0.f;
-  for (int j = 0; j < A; ++j) { q[j] = expf(x[j] - m); s += q[j]; }
-  float s2 = 0.f;
-  for (int j = 0; j < A; ++j) { q[j] = q[j] / s; s2 += q[j]; }     // F.softmax (nn/actor.py:94)
+  const float s2 = categorical_softmax(x, mk, A, j0, q);              // F.softmax (nn/actor.py:94)
   if (u) {
     for (int j = 0; j < A; ++j) q[j] = q[j] / s2;                   // categorical.py:70
-    const int a = inverse_cdf(q, A, u[b]);
+    const int a = inverse_cdf(q, A, u[b], mk, j0);
     action[b] = (float)a;
     logp[b] = logf(fminf(fmaxf(q[a], kEps), 1.f - kEps));
     if (probs_out) for (int j = 0; j < A; ++j) probs_out[(size_t)b * A + j] = q[j];
   } else {
-    action[b] = (float)argmax_first(q, A);    // play mode works on the raw softmax output
+    action[b] = (float)argmax_first(q, A, mk, j0);    // play mode works on the raw softmax output
     logp[b] = 0.f;
     if (probs_out) for (int j = 0; j < A; ++j) probs_out[(size_t)b * A + j] = q[j];
   }
@@ -150,14 +154,20 @@ extern "C" int ddrl_sample_categorical_probs(const float* probs, int ld, const f
   return DDRL_OK;
 }
 
-extern "C" int ddrl_categorical_head(const float* logits, int ld, const float* u, int B, int A, float* action,
-                                     float* logp, float* probs_out, void* stream) {
+extern "C" int ddrl_categorical_head_m(const float* logits, int ld, const float* u, int B, int A, float* action,
+                                       float* logp, float* probs_out, const float* mask, void* stream) {
   if (B < 0 || A < 1 || A > kMaxA || ld < A) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!logits || !action || !logp) return DDRL_E_ARG;
-  categorical_head_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, u, B, A, action, logp, probs_out);
+  categorical_head_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, u, B, A, action, logp, probs_out,
+                                                                              mask);
   DDRL_LAUNCHED("categorical_head_kernel");
   return DDRL_OK;
+}
+
+extern "C" int ddrl_categorical_head(const float* logits, int ld, const float* u, int B, int A, float* action,
+                                     float* logp, float* probs_out, void* stream) {
+  return ddrl_categorical_head_m(logits, ld, u, B, A, action, logp, probs_out, nullptr, stream);
 }
 
 extern "C" int ddrl_gaussian_head(const float* mu, int ld, const float* log_std, const float* eps, int B, int A,

@@ -116,6 +116,9 @@ struct ddrl_net {
   const float* value_norm = nullptr;
   // DDRL_DIST_BETA (ddrl_net_set_action_bounds): device [2 x act_dim] = low | high, owned.  Null: not set yet.
   float* bounds = nullptr;
+  // ACTION_MASK (ddrl_net_set_action_mask, categorical nets): one more observation slot after the encoder's, [B, act_dim] fp32,
+  // read by the head, the log-prob pre-pass and the loss kernels
+  bool action_mask = false;
   // DECOUPLED_PPO with hp->ppo_stats: the last backward pass took proximal log-probs, so its loss tail holds the behaviour KL
   // in slot P+5 and ddrl_net_clip_adam reports it as loss4_out[6]
   bool behaviour_kl = false;
@@ -355,6 +358,20 @@ static int round4(int x) { return (x + 3) & ~3; }
 static int head_n(const ddrl_net* n) { return n->d.dist == DDRL_DIST_BETA ? 2 * n->d.act_dim : n->d.act_dim; }
 // a Beta net cannot run before its action bounds are set
 static bool bounds_missing(const ddrl_net* n) { return n->d.dist == DDRL_DIST_BETA && !n->bounds; }
+
+// observation slots the encoder reads (the action mask, when on, is the slot after them)
+static int encoder_slots(const ddrl_net* n) {
+  switch (n->d.arch) {
+    case DDRL_ARCH_ATARI: case DDRL_ARCH_MLP: return 1;
+    case DDRL_ARCH_NAV: return 2;
+    default: return 3;
+  }
+}
+
+// ACTION_MASK: rows [r0, ...) of the mask slot, or null when the mask is off
+static const float* mask_rows(const ddrl_net* n, const float* const* obs, long long r0) {
+  return n->action_mask ? obs[encoder_slots(n)] + r0 * n->d.act_dim : nullptr;
+}
 
 static Lin make_lin(ddrl_net* n, const std::string& wname, int N, int K, int I, int J, int act) {
   Lin l;
@@ -1648,14 +1665,11 @@ extern "C" int ddrl_net_params_changed(ddrl_net* n) {
 
 extern "C" int ddrl_net_num_obs(const ddrl_net* n) {
   if (!n) return DDRL_E_ARG;
-  switch (n->d.arch) {
-    case DDRL_ARCH_ATARI: case DDRL_ARCH_MLP: return 1;
-    case DDRL_ARCH_NAV: return 2;
-    default: return 3;
-  }
+  return encoder_slots(n) + (n->action_mask ? 1 : 0);
 }
 extern "C" int64_t ddrl_net_obs_elems(const ddrl_net* n, int slot) {
   if (!n) return DDRL_E_ARG;
+  if (n->action_mask && slot == encoder_slots(n)) return n->d.act_dim;
   switch (n->d.arch) {
     case DDRL_ARCH_ATARI: return slot == 0 ? (int64_t)n->d.in_ch * 84 * 84 : 0;
     case DDRL_ARCH_MLP: return slot == 0 ? n->d.in_ch : 0;
@@ -1693,6 +1707,13 @@ extern "C" int ddrl_net_set_action_bounds(ddrl_net* n, const float* low_host, co
   return DDRL_OK;
 }
 
+extern "C" int ddrl_net_set_action_mask(ddrl_net* n, int on) {
+  if (!n || n->d.dist != DDRL_DIST_CATEGORICAL) return DDRL_E_ARG;
+  if (n->ws.base) return DDRL_E_STATE;      // a pass has sized the workspace and keyed its graphs on the slot layout
+  n->action_mask = on != 0;
+  return DDRL_OK;
+}
+
 extern "C" int ddrl_net_forward(ddrl_net* n, const float* const* obs, int n_obs, int B, const float* draw, float* actions,
                                 float* logp, float* values, float* pi_out, void* stream) {
   if (!n || B < 0) return DDRL_E_ARG;
@@ -1710,8 +1731,8 @@ extern "C" int ddrl_net_forward(ddrl_net* n, const float* const* obs, int n_obs,
     amax_new_pass(n, s, false);      // every micro-batch rewrites the workspace: amax entries live for one chunk
     TRY(forward_chunk(n, obs, r0, mb, false, s));
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
-      TRY(ddrl_categorical_head(n->logits, n->ldA, draw ? draw + r0 : nullptr, mb, A, actions + r0, logp + r0,
-                                pi_out ? pi_out + r0 * A : nullptr, s));
+      TRY(ddrl_categorical_head_m(n->logits, n->ldA, draw ? draw + r0 : nullptr, mb, A, actions + r0, logp + r0,
+                                  pi_out ? pi_out + r0 * A : nullptr, mask_rows(n, obs, r0), s));
     } else if (n->d.dist == DDRL_DIST_BETA) {
       TRY(ddrl_beta_head(n->logits, n->ldA, n->bounds, n->bounds + A, draw ? draw + r0 * A : nullptr, mb, A, actions + r0 * A,
                          logp + r0, pi_out ? pi_out + r0 * 2 * A : nullptr, s));
@@ -1775,7 +1796,7 @@ extern "C" int ddrl_net_log_prob(ddrl_net* n, const float* const* obs, int n_obs
     amax_new_pass(n, s, false);
     TRY(forward_chunk(n, obs, r0, mb, true, s));
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
-      TRY(ddrl_logp_actions_categorical(n->logits, n->ldA, actions + r0, mb, A, out_logp + r0, s));
+      TRY(ddrl_logp_actions_categorical_m(n->logits, n->ldA, actions + r0, mb, A, out_logp + r0, mask_rows(n, obs, r0), s));
     } else if (n->d.dist == DDRL_DIST_BETA) {
       TRY(ddrl_logp_actions_beta(n->logits, n->ldA, n->bounds, n->bounds + A, actions + r0 * A, mb, A, out_logp + r0, s));
     } else {
@@ -1810,10 +1831,10 @@ static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int 
     amax_new_pass(n, s, reuse_obs);
     TRY(forward_chunk(n, obs, r0, mb, true, s, reuse_obs));
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
-      TRY(ddrl_ppo_loss_categorical_dc(n->logits, n->ldA, actions + r0, old_logp + r0, adv + r0, returns + r0, n->vout, mb, A,
-                                       invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
-                                       old_values ? old_values + r0 : nullptr, stats, n->value_norm,
-                                       prox_logp ? prox_logp + r0 : nullptr, is_clip, s));
+      TRY(ddrl_ppo_loss_categorical_m(n->logits, n->ldA, actions + r0, old_logp + r0, adv + r0, returns + r0, n->vout, mb, A,
+                                      invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
+                                      old_values ? old_values + r0 : nullptr, stats, n->value_norm,
+                                      prox_logp ? prox_logp + r0 : nullptr, is_clip, mask_rows(n, obs, r0), s));
     } else if (n->d.dist == DDRL_DIST_BETA) {
       TRY(ddrl_ppo_loss_beta(n->logits, n->ldA, n->bounds, n->bounds + A, actions + r0 * A, old_logp + r0, adv + r0, returns + r0,
                              n->vout, mb, A, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
@@ -1879,8 +1900,9 @@ static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_
   }
   TRY(check_obs(n, obs, n_obs));
   if (!actions || !old_logp || !adv || !returns) return DDRL_E_ARG;
-  const std::string key = graph_key("bwd", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, actions, old_logp,
-                                            adv, returns, old_values, n->value_norm, prox_logp, n->params, n->grads, n->ws.base},
+  const std::string key = graph_key("bwd", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, mask_rows(n, obs, 0),
+                                            actions, old_logp, adv, returns, old_values, n->value_norm, prox_logp, n->params, n->grads,
+                                            n->ws.base},
                                     {B_local, B_global, is_clip_key(is_clip)}, hp, sizeof(*hp));
   auto launch_seg = [&](ddrl_net::GraphEntry* e, int k) {
     const int pre = (int)e->pre_execs.size();
@@ -1978,9 +2000,9 @@ extern "C" int ddrl_net_backward_minibatch_dc(ddrl_net* n, const float* const* o
     return backward_body(n, obs, B_local, B_global, actions, old_logp, adv, returns, old_values, prox_logp, is_clip, hp, false, cs);
   };
   if (B_local > n->MB || !n->extra.empty() || !graphs_enabled(n) || n->mb_graphs_off) return body(s);
-  const std::string key = graph_key("bwd_mb", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, actions,
-                                               old_logp, adv, returns, old_values, n->value_norm, prox_logp, n->params, n->grads,
-                                               n->ws.base},
+  const std::string key = graph_key("bwd_mb", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr,
+                                               mask_rows(n, obs, 0), actions, old_logp, adv, returns, old_values, n->value_norm,
+                                               prox_logp, n->params, n->grads, n->ws.base},
                                     {B_local, B_global, is_clip_key(is_clip)}, hp, sizeof(*hp));
   if (std::find(n->mb_seen.begin(), n->mb_seen.end(), key) == n->mb_seen.end()) {
     if (n->mb_seen.size() >= 16) n->mb_seen.erase(n->mb_seen.begin());

@@ -28,8 +28,12 @@
 // Beta actor (beta.cuh): head z [B, 2A] -> alpha | beta = 1 + softplus(z); the log-prob is beta_logp, the entropy per element is
 // beta_entropy, both in fp64 and rounded once; the gradient follows the softplus chain (digamma for the log-prob, trigamma for
 // the entropy).
+// ACTION_MASK (categorical.cuh): the categorical kernels take an optional mask [B, A].  Masked entries have p = q = 0, so they add
+// 0 * log(eps) = 0 to the entropy and their logits get exactly zero gradient; a masked taken action (corrupt data) has log-prob
+// log(eps), and the clamp's zero gradient outside [eps, 1 - eps] makes its actor term constant.
 #include "common.cuh"
 #include "beta.cuh"
+#include "categorical.cuh"
 
 namespace ddrl {
 
@@ -46,16 +50,14 @@ struct LossParams {
   float is_clip;                  // DECOUPLED_PPO: truncation of the behaviour weight, <= 0: none
 };
 
-// log-prob of the taken action a (clamped into [0, A)) under Categorical(logits = x[0..A)): the softmax -> q = p / sum(p) ->
-// clamp(eps, 1 - eps) -> log chain of torch.  Leaves the softmax p[0..A) and s2 = sum(p) for the loss kernel's gradient.  The
-// loss kernel and logp_actions_categorical_kernel share it, so equal logits give equal log-prob bits.
-__device__ __forceinline__ float categorical_logp(const float* __restrict__ x, int A, float action, float* p, float* s2_out) {
-  float m = x[0];
-  for (int j = 1; j < A; ++j) m = fmaxf(m, x[j]);
-  float s = 0.f;
-  for (int j = 0; j < A; ++j) { p[j] = expf(x[j] - m); s += p[j]; }
-  float s2 = 0.f;
-  for (int j = 0; j < A; ++j) { p[j] = p[j] / s; s2 += p[j]; }
+// log-prob of the taken action a (clamped into [0, A)) under Categorical(logits = x[0..A)) with the row's mask (or null): the
+// masked softmax (categorical.cuh) -> q = p / sum(p) -> clamp(eps, 1 - eps) -> log chain of torch.  Leaves the softmax p[0..A)
+// and s2 = sum(p) for the loss kernel's gradient.  The loss kernel and logp_actions_categorical_kernel share it, and the head
+// kernel the same softmax, so equal logits and masks give equal log-prob bits.
+__device__ __forceinline__ float categorical_logp(const float* __restrict__ x, const float* __restrict__ mask, int A, float action,
+                                                  float* p, float* s2_out) {
+  mask = categorical_row_mask(mask, A);
+  const float s2 = categorical_softmax(x, mask, A, categorical_first_allowed(mask, A), p);
   int a = (int)action;                      // Categorical.log_prob: value.long()
   a = a < 0 ? 0 : (a >= A ? A - 1 : a);     // the reference raises on an action outside [0, A); never read out of bounds
   const float qa = p[a] / s2;
@@ -151,7 +153,7 @@ __global__ void __launch_bounds__(128) ppo_loss_categorical_kernel(
     const float* __restrict__ logits, int ld, const float* __restrict__ actions, const float* __restrict__ old_logp,
     const float* __restrict__ adv, const float* __restrict__ returns, const float* __restrict__ v, int B, int A,
     LossParams hp, float* __restrict__ dlogits, int ld_d, float* __restrict__ dv, float* __restrict__ loss_sums,
-    const float* __restrict__ old_v, float* __restrict__ stats, DetSeq det) {
+    const float* __restrict__ old_v, float* __restrict__ stats, const float* __restrict__ mask, DetSeq det) {
   __shared__ float scratch[32];
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   float l_actor = 0.f, l_v = 0.f, l_ent = 0.f, l_kl = 0.f, l_cf = 0.f, l_bkl = 0.f;
@@ -159,7 +161,7 @@ __global__ void __launch_bounds__(128) ppo_loss_categorical_kernel(
     const float* x = logits + (size_t)b * ld;
     float p[kMaxAL];
     float s2;
-    const float logp = categorical_logp(x, A, actions[b], p, &s2);      // log-prob of the taken action
+    const float logp = categorical_logp(x, mask ? mask + (size_t)b * A : nullptr, A, actions[b], p, &s2);   // of the taken action
     int a = (int)actions[b];
     a = a < 0 ? 0 : (a >= A ? A - 1 : a);
     const float Ai = adv[b];
@@ -381,12 +383,12 @@ __global__ void __launch_bounds__(128) value_loss_kernel(const float* __restrict
 // DECOUPLED_PPO pre-pass: out_logp[b] = log-prob of the taken action, bit-equal to the loss kernels' on the same logits / means
 __global__ void __launch_bounds__(128) logp_actions_categorical_kernel(const float* __restrict__ logits, int ld,
                                                                        const float* __restrict__ actions, int B, int A,
-                                                                       float* __restrict__ out_logp) {
+                                                                       float* __restrict__ out_logp, const float* __restrict__ mask) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   float p[kMaxAL];
   float s2;
-  out_logp[b] = categorical_logp(logits + (size_t)b * ld, A, actions[b], p, &s2);
+  out_logp[b] = categorical_logp(logits + (size_t)b * ld, mask ? mask + (size_t)b * A : nullptr, A, actions[b], p, &s2);
 }
 
 __global__ void __launch_bounds__(128) logp_actions_gaussian_kernel(const float* __restrict__ mu, int ld,
@@ -424,21 +426,31 @@ static bool value_clip_args_ok(const ddrl_ppo_hparams* hp, const float* old_valu
   return old_values ? hp->value_clip > 0.f : !(hp->value_clip > 0.f);
 }
 
-extern "C" int ddrl_ppo_loss_categorical_dc(const float* logits, int ld, const float* actions, const float* old_logp,
-                                            const float* adv, const float* returns, const float* v, int B, int A,
-                                            float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dlogits,
-                                            int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
-                                            const float* value_norm, const float* prox_logp, float is_clip, void* stream) {
+extern "C" int ddrl_ppo_loss_categorical_m(const float* logits, int ld, const float* actions, const float* old_logp,
+                                           const float* adv, const float* returns, const float* v, int B, int A,
+                                           float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dlogits,
+                                           int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
+                                           const float* value_norm, const float* prox_logp, float is_clip, const float* mask,
+                                           void* stream) {
   if (B < 0 || A < 1 || A > kMaxAL || ld < A || ld_d < A || !hp) return DDRL_E_ARG;
   if (!value_clip_args_ok(hp, old_values)) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!logits || !actions || !old_logp || !adv || !returns || !v || !dlogits || !dv || !loss_sums) return DDRL_E_ARG;
   ppo_loss_categorical_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(
       logits, ld, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared, value_norm, prox_logp, is_clip),
-      dlogits, ld_d, dv, loss_sums, old_values, stats, det_seq(1));
-  prof_work((8.0 * A + 24.0 + (old_values ? 4.0 : 0.0) + (prox_logp ? 4.0 : 0.0)) * B);
+      dlogits, ld_d, dv, loss_sums, old_values, stats, mask, det_seq(1));
+  prof_work((8.0 * A + 24.0 + (old_values ? 4.0 : 0.0) + (prox_logp ? 4.0 : 0.0) + (mask ? 4.0 * A : 0.0)) * B);
   DDRL_LAUNCHED("ppo_loss_categorical_kernel");
   return DDRL_OK;
+}
+
+extern "C" int ddrl_ppo_loss_categorical_dc(const float* logits, int ld, const float* actions, const float* old_logp,
+                                            const float* adv, const float* returns, const float* v, int B, int A,
+                                            float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dlogits,
+                                            int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
+                                            const float* value_norm, const float* prox_logp, float is_clip, void* stream) {
+  return ddrl_ppo_loss_categorical_m(logits, ld, actions, old_logp, adv, returns, v, B, A, inv_B_global, hp, shared, dlogits,
+                                     ld_d, dv, loss_sums, old_values, stats, value_norm, prox_logp, is_clip, nullptr, stream);
 }
 
 extern "C" int ddrl_ppo_loss_categorical_vn(const float* logits, int ld, const float* actions, const float* old_logp,
@@ -507,15 +519,20 @@ extern "C" int ddrl_ppo_loss_gaussian_vn(const float* mu, int ld, const float* l
                                    ld_d, dv, dlog_std, loss_sums, old_values, stats, value_norm, nullptr, 0.f, stream);
 }
 
-extern "C" int ddrl_logp_actions_categorical(const float* logits, int ld, const float* actions, int B, int A, float* out_logp,
-                                             void* stream) {
+extern "C" int ddrl_logp_actions_categorical_m(const float* logits, int ld, const float* actions, int B, int A, float* out_logp,
+                                               const float* mask, void* stream) {
   if (B < 0 || A < 1 || A > kMaxAL || ld < A) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!logits || !actions || !out_logp) return DDRL_E_ARG;
-  logp_actions_categorical_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, actions, B, A, out_logp);
-  prof_work((4.0 * A + 8.0) * B);
+  logp_actions_categorical_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, actions, B, A, out_logp, mask);
+  prof_work((4.0 * A + 8.0 + (mask ? 4.0 * A : 0.0)) * B);
   DDRL_LAUNCHED("logp_actions_categorical_kernel");
   return DDRL_OK;
+}
+
+extern "C" int ddrl_logp_actions_categorical(const float* logits, int ld, const float* actions, int B, int A, float* out_logp,
+                                             void* stream) {
+  return ddrl_logp_actions_categorical_m(logits, ld, actions, B, A, out_logp, nullptr, stream);
 }
 
 extern "C" int ddrl_logp_actions_gaussian(const float* mu, int ld, const float* log_std, const float* actions, int B, int A,

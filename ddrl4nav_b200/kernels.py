@@ -113,6 +113,32 @@ def categorical_head(logits: torch.Tensor, u: Optional[torch.Tensor], want_probs
     return action, logp, probs
 
 
+def categorical_head_m(logits: torch.Tensor, u: Optional[torch.Tensor], mask: Optional[torch.Tensor], want_probs: bool = True):
+    """ddrl_categorical_head_m: categorical_head with the action mask [B, A] (any dtype, allowed iff != 0; None: no mask) ->
+    (action [B], logp [B], the masked probs [B, A] or None)."""
+    lib = _lib.load()
+    logits = _f32c(logits)
+    B, A = logits.shape
+    mask = _mask_f32(mask, B, A)
+    action = torch.empty(B, dtype=torch.float32, device=logits.device)
+    logp = torch.empty(B, dtype=torch.float32, device=logits.device)
+    probs = torch.empty((B, A), dtype=torch.float32, device=logits.device) if want_probs else None
+    u = None if u is None else _f32c(u)
+    check(lib.ddrl_categorical_head_m(ptr(logits), A, ptr(u), B, A, ptr(action), ptr(logp), ptr(probs), ptr(mask),
+                                      current_stream()), "ddrl_categorical_head_m")
+    return action, logp, probs
+
+
+def _mask_f32(mask, B: int, A: int):
+    """ACTION_MASK: the mask as the kernels read it, contiguous fp32 [B, A] (None stays None)."""
+    if mask is None:
+        return None
+    mask = _f32c(mask)
+    if mask.numel() != B * A:
+        raise DDRLError("action mask has shape %s; expected [B=%d, A=%d]" % (tuple(mask.shape), B, A))
+    return mask
+
+
 def gaussian_head(mu: torch.Tensor, log_std: torch.Tensor, eps: Optional[torch.Tensor]):
     lib = _lib.load()
     mu = _f32c(mu)
@@ -176,6 +202,26 @@ def ppo_loss_categorical_dc(logits, actions, old_logp, adv, returns, v, hp: PPOH
     return dlogits, dv, sums
 
 
+def ppo_loss_categorical_m(logits, actions, old_logp, adv, returns, v, hp: PPOHparams, shared: bool, mask=None, old_values=None,
+                           value_norm=None, prox_logp=None, is_clip: Optional[float] = None, b_global: Optional[int] = None):
+    """ddrl_ppo_loss_categorical_m with the statistics on -> (dlogits [B,A], dv [B], sums [8]), sums as ppo_loss_categorical_dc.
+    mask [B, A] (ACTION_MASK; None: no mask), old_values (VALUE_CLIP; needs hp.value_clip > 0), value_norm (device {mean32,
+    scale32, sigma32}) and prox_logp (DECOUPLED_PPO) are optional."""
+    lib = _lib.load()
+    logits, actions, old_logp, adv, returns, v = map(_f32c, (logits, actions, old_logp, adv, returns, v))
+    old_values, value_norm, prox_logp = (None if t is None else _f32c(t) for t in (old_values, value_norm, prox_logp))
+    B, A = logits.shape
+    mask = _mask_f32(mask, B, A)
+    dlogits = torch.empty_like(logits)
+    dv = torch.empty(B, dtype=torch.float32, device=logits.device)
+    sums = torch.zeros(8, dtype=torch.float32, device=logits.device)
+    check(lib.ddrl_ppo_loss_categorical_m(ptr(logits), A, ptr(actions), ptr(old_logp), ptr(adv), ptr(returns), ptr(v), B, A,
+                                          1.0 / float(b_global or B), C.byref(hp), int(shared), ptr(dlogits), A, ptr(dv),
+                                          ptr(sums), ptr(old_values), ptr(sums[3:]), ptr(value_norm), ptr(prox_logp),
+                                          float(is_clip or 0.0), ptr(mask), current_stream()), "ddrl_ppo_loss_categorical_m")
+    return dlogits, dv, sums
+
+
 def ppo_loss_gaussian_dc(mu, log_std, actions, old_logp, adv, returns, v, hp: PPOHparams, shared: bool, prox_logp=None,
                          is_clip: Optional[float] = None, b_global: Optional[int] = None):
     """The decoupled loss (ddrl_ppo_loss_gaussian_dc) with the statistics on -> (dmu [B,A], dv [B], dlog_std [A], sums [8]),
@@ -202,6 +248,18 @@ def logp_actions_categorical(logits, actions) -> torch.Tensor:
     out = torch.empty(B, dtype=torch.float32, device=logits.device)
     check(_lib.load().ddrl_logp_actions_categorical(ptr(logits), A, ptr(actions), B, A, ptr(out), current_stream()),
           "ddrl_logp_actions_categorical")
+    return out
+
+
+def logp_actions_categorical_m(logits, actions, mask=None) -> torch.Tensor:
+    """Log-probs [B] of the taken actions under the masked Categorical(logits) (mask [B, A] or None), bit-equal to the loss and
+    head kernels'."""
+    logits, actions = _f32c(logits), _f32c(actions)
+    B, A = logits.shape
+    mask = _mask_f32(mask, B, A)
+    out = torch.empty(B, dtype=torch.float32, device=logits.device)
+    check(_lib.load().ddrl_logp_actions_categorical_m(ptr(logits), A, ptr(actions), B, A, ptr(out), ptr(mask), current_stream()),
+          "ddrl_logp_actions_categorical_m")
     return out
 
 

@@ -41,13 +41,16 @@ class ObsRMS(torch.nn.Module):
     def applied(self, s):
         return getattr(self, "mean32_%d" % s), getattr(self, "scale32_%d" % s)
 
-    def bind(self, n_obs, elems, dev):
+    def bind(self, n_obs, elems, dev, mask_slot=None):
         """Resolves the slots against an engine with `n_obs` observation slots of elems(s) elements each, and creates (or checks
-        and moves) the buffers on `dev`."""
-        slots = tuple(range(n_obs)) if self.wanted is None else self.wanted
+        and moves) the buffers on `dev`.  mask_slot: the ACTION_MASK slot, which is never normalised (every slot means every
+        other slot; a list that names it is an error)."""
+        slots = tuple(s for s in range(n_obs) if s != mask_slot) if self.wanted is None else self.wanted
         bad = [s for s in slots if s >= n_obs]
         if bad:
             raise DDRLError("NORM_OBS slot(s) %s out of range: the net has %d observation slot(s)" % (bad, n_obs))
+        if mask_slot is not None and mask_slot in slots:
+            raise DDRLError("NORM_OBS slot %d is the ACTION_MASK slot, which is never normalised" % mask_slot)
         dims = {}
         for s in slots:
             D = int(elems(s))

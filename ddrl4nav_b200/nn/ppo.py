@@ -121,6 +121,11 @@ class PPO(Basenn):
         if self.decoupled_is_clip is not None and not self.decoupled:
             raise DDRLError("DECOUPLED_IS_CLIP needs DECOUPLED_PPO=True")
         self.last_prox_logps = None     # DECOUPLED_PPO: the proximal log-probs [B_local] of the last learn call (persistent)
+        # invalid-action masking (non-reference, off by default; Huang & Ontanon 2022): one more state slot after the encoder's,
+        # [B, A], action j allowed iff != 0; act / forward sample, and learn trains, the masked categorical distribution
+        self.action_mask = _flag_option(config_nn, "ACTION_MASK")
+        if self.action_mask and getattr(actor, "DIST", None) != "categorical":
+            raise DDRLError("ACTION_MASK needs a CategoricalActor (got %s)" % type(actor).__name__)
         self.hp = kernels.make_hparams(
             ppo_clip=_cfg(config_nn, "PPO_CLIP", 0.2), dual_clip=_cfg(config_nn, "DUEL_PPO_CLIP", 3),
             v_coef=_cfg(config_nn, "V_LOSS_THETA", 1.0), ent_coef=_cfg(config_nn, "ENTROPY_LOSS_THETA", 0.05),
@@ -292,9 +297,12 @@ class PPO(Basenn):
             A = s["act_dim"]
             check(lib.ddrl_net_set_action_bounds(h, (C.c_float * A)(*self.actor.action_low), (C.c_float * A)(*self.actor.action_high)),
                   "ddrl_net_set_action_bounds")
+        if self.action_mask:
+            check(lib.ddrl_net_set_action_mask(h, 1), "ddrl_net_set_action_mask")
         if self.obs_rms is not None:
+            n_obs = lib.ddrl_net_num_obs(h)
             try:
-                self.obs_rms.bind(lib.ddrl_net_num_obs(h), lambda i: lib.ddrl_net_obs_elems(h, i), dev)
+                self.obs_rms.bind(n_obs, lambda i: lib.ddrl_net_obs_elems(h, i), dev, n_obs - 1 if self.action_mask else None)
             except DDRLError:
                 self._destroy()
                 raise
@@ -514,7 +522,8 @@ class PPO(Basenn):
     def forward(self, states, act=None, play_mode=False):
         """Reference-shaped output: ((pi, log_p), [values [B,1]]) with pi = Categorical / Normal, or the raw
         softmax / mu tensor in play mode (nn/actor.py:58-67,90-98).  BetaActor: the Beta mapped onto the bounds
-        (BetaActor.distribution), or the mean action [B,A] in play mode."""
+        (BetaActor.distribution), or the mean action [B,A] in play mode.  ACTION_MASK: the engine's softmax is the masked one,
+        so the Categorical gives masked actions probability 0."""
         mean, _, values, pi_raw = self.act(states, draw=None, play_mode=True, want_pi=True)
         if self.actor.DIST == "categorical":
             pi = pi_raw if play_mode else Categorical(pi_raw)

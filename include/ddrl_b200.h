@@ -159,6 +159,14 @@ int ddrl_sample_categorical_probs(const float* probs, int ld, const float* u, in
  * probs_out may be NULL. */
 int ddrl_categorical_head(const float* logits, int ld, const float* u, int B, int A,
                           float* action, float* logp, float* probs_out, void* stream);
+/* The same with an action mask (non-reference option ACTION_MASK): mask DEVICE [B, A] fp32 (row stride A) or NULL (the call
+ * above).  Action j of row b is allowed iff mask[b, j] != 0; a row that allows nothing is treated as allowing everything.  The
+ * softmax is torch's softmax(logits.masked_fill(~m, -inf)): max over the allowed entries, masked p = 0 exactly, the rest of
+ * the chain unchanged, so an all-ones mask gives the bits of no mask.  Sampling inverts the CDF of the masked q with strict >,
+ * and no hit gives the first allowed action; play mode is the first-max argmax of the masked softmax; probs_out holds the
+ * masked probabilities.  Masked logits are never read. */
+int ddrl_categorical_head_m(const float* logits, int ld, const float* u, int B, int A,
+                            float* action, float* logp, float* probs_out, const float* mask, void* stream);
 /* Gaussian head (nn/actor.py:58-70): a = mu + exp(log_std)*eps (mul, then add);
  * logp = sum_j Normal(mu,std).log_prob(a); eps NULL => play mode (a = mu, logp = 0). */
 int ddrl_gaussian_head(const float* mu, int ld, const float* log_std, const float* eps, int B, int A,
@@ -228,6 +236,15 @@ int ddrl_ppo_loss_categorical_dc(const float* logits, int ld, const float* actio
                                  float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
                                  float* dlogits, int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
                                  const float* value_norm, const float* prox_logp, float is_clip, void* stream);
+/* The same with an action mask (ACTION_MASK; mask as ddrl_categorical_head_m, NULL: the _dc call above).  The log-prob and the
+ * entropy are those of the masked distribution: masked entries add 0 to the entropy and their dlogits are exactly 0.  A taken
+ * action that is masked (corrupt data) has log-prob log(eps) and, through the clamp, a zero log-prob gradient. */
+int ddrl_ppo_loss_categorical_m(const float* logits, int ld, const float* actions, const float* old_logp,
+                                const float* adv, const float* returns, const float* v, int B, int A,
+                                float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                                float* dlogits, int ld_d, float* dv, float* loss_sums, const float* old_values, float* stats,
+                                const float* value_norm, const float* prox_logp, float is_clip, const float* mask,
+                                void* stream);
 int ddrl_ppo_loss_gaussian_dc(const float* mu, int ld, const float* log_std, const float* actions,
                               const float* old_logp, const float* adv, const float* returns, const float* v,
                               int B, int A, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
@@ -248,6 +265,10 @@ int ddrl_ppo_loss_beta(const float* head, int ld, const float* low, const float*
  * logits / means give equal bits.  The proximal log-probs of DECOUPLED_PPO (ddrl_net_log_prob). */
 int ddrl_logp_actions_categorical(const float* logits, int ld, const float* actions, int B, int A, float* out_logp,
                                   void* stream);
+/* the categorical one with an action mask (mask as ddrl_categorical_head_m, NULL: the call above): the bits of
+ * ddrl_ppo_loss_categorical_m's log-prob, and of ddrl_categorical_head_m's for the action it emitted */
+int ddrl_logp_actions_categorical_m(const float* logits, int ld, const float* actions, int B, int A, float* out_logp,
+                                    const float* mask, void* stream);
 int ddrl_logp_actions_gaussian(const float* mu, int ld, const float* log_std, const float* actions, int B, int A,
                                float* out_logp, void* stream);
 /* the same for the Beta actor (actions [B, A], head / low / high as ddrl_ppo_loss_beta) */
@@ -366,6 +387,12 @@ int ddrl_net_set_value_norm(ddrl_net* net, const float* applied);
  * else DDRL_E_ARG; another distribution: DDRL_E_ARG.  Until it is called, ddrl_net_forward, ddrl_net_log_prob and the backward
  * passes of a Beta net return DDRL_E_STATE.  Captured graphs read the buffer when they replay, so new bounds need no recapture. */
 int ddrl_net_set_action_bounds(ddrl_net* net, const float* low_host, const float* high_host);
+/* ACTION_MASK (DDRL_DIST_CATEGORICAL only, else DDRL_E_ARG): on != 0 adds one observation slot after the encoder's, the action
+ * mask [B, act_dim] (fp32, action j allowed iff != 0), which ddrl_net_forward, ddrl_net_log_prob and the backward passes hand
+ * to the _m head, log-prob and loss kernels micro-batch by micro-batch; ddrl_net_num_obs then counts it and
+ * ddrl_net_obs_elems(mask slot) returns act_dim.  The encoders never read it.  Call it before the first pass: once a pass has
+ * run it returns DDRL_E_STATE.  It adds no parameter. */
+int ddrl_net_set_action_mask(ddrl_net* net, int on);
 /* tell the net the flat params were changed behind its back (load_state_dict, updatenn_by_redis) */
 int ddrl_net_params_changed(ddrl_net* net);
 /* number of observation slots and per-sample element count of each (for argument checking) */
