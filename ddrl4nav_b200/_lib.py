@@ -41,7 +41,7 @@ class ConvDesc(C.Structure):
 
 
 ARCH = {"atari": 0, "nav": 1, "navped": 2, "nav1d": 3, "mlp": 4}
-DIST = {"categorical": 0, "gaussian": 1, "beta": 2}
+DIST = {"categorical": 0, "gaussian": 1, "beta": 2, "multi_categorical": 3}
 GEMM_MODE = {"simt": 0, "tc": 1, "tc2": 2, "tc3": 3}
 
 _P = C.c_void_p
@@ -66,6 +66,7 @@ SIGNATURES = {
     "ddrl_sample_categorical_probs": (_I, [_P, _I, _P, _I, _I, _P, _P, _P]),
     "ddrl_categorical_head": (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P]),
     "ddrl_categorical_head_m": (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P, _P]),
+    "ddrl_multi_categorical_head": (_I, [_P, _I, _P, _I, _I, C.POINTER(C.c_int32), _P, _P, _P, _P, _P]),
     "ddrl_gaussian_head": (_I, [_P, _I, _P, _P, _I, _I, _P, _P, _P]),
     "ddrl_beta_head": (_I, [_P, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P]),
     "ddrl_ppo_loss_categorical": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P]),
@@ -84,8 +85,11 @@ SIGNATURES = {
                                        _P, _P, _P, _P, _F, _P]),
     "ddrl_ppo_loss_categorical_m": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P,
                                          _P, _P, _P, _F, _P, _P]),
+    "ddrl_ppo_loss_multi_categorical": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, C.POINTER(C.c_int32), _F, C.POINTER(PPOHparams), _I,
+                                             _P, _I, _P, _P, _P, _P, _P, _P, _F, _P, _P]),
     "ddrl_logp_actions_categorical": (_I, [_P, _I, _P, _I, _I, _P, _P]),
     "ddrl_logp_actions_categorical_m": (_I, [_P, _I, _P, _I, _I, _P, _P, _P]),
+    "ddrl_logp_actions_multi_categorical": (_I, [_P, _I, _P, _I, _I, C.POINTER(C.c_int32), _P, _P, _P]),
     "ddrl_logp_actions_gaussian": (_I, [_P, _I, _P, _P, _I, _I, _P, _P]),
     "ddrl_ppo_loss_beta": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _P, _I, _I, _F, C.POINTER(PPOHparams), _I, _P, _I, _P, _P, _P, _P,
                                 _P, _P, _F, _P]),
@@ -113,6 +117,7 @@ SIGNATURES = {
     "ddrl_net_obs_elems": (_L, [_P, _I]),
     "ddrl_net_set_value_norm": (_I, [_P, _P]),
     "ddrl_net_set_action_bounds": (_I, [_P, C.POINTER(_F), C.POINTER(_F)]),
+    "ddrl_net_set_action_branches": (_I, [_P, _I, C.POINTER(C.c_int32)]),
     "ddrl_net_set_action_mask": (_I, [_P, _I]),
     "ddrl_net_forward": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P, _P, _P, _P]),
     "ddrl_net_log_prob": (_I, [_P, C.POINTER(_P), _I, _I, _P, _P, _P]),

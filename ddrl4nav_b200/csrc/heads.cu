@@ -13,6 +13,7 @@
 // solve, which runs one thread per (row, dimension).
 // ACTION_MASK (categorical.cuh): the categorical head takes an optional mask [B, A]; the draw then inverts the CDF of the masked
 // q, and no hit gives the first allowed action (0 without a mask, as above), so a masked action is never emitted.
+// MultiDiscrete (categorical.cuh): the same head per branch, on the branch's slice, with draws u [B, K] and actions [B, K].
 #include "common.cuh"
 #include "beta.cuh"
 #include "categorical.cuh"
@@ -57,30 +58,42 @@ __global__ void sample_probs_kernel(const float* __restrict__ probs, int ld, con
   }
 }
 
-constexpr int kMaxA = 64;
+constexpr int kMaxA = kCatMaxA;
 
 // logits -> softmax -> Categorical(probs): q = p / sum(p); logits' = log(clamp(q, eps, 1-eps)).  mask: [B, A] (row stride A) or
-// null (categorical.cuh)
+// null (categorical.cuh).  kBranched (MultiDiscrete): branch i samples its own slice with u[b, i] into action[b, i]; the row's
+// log-prob is categorical_logp_row of the emitted actions.  Without it (the categorical actor) K = 1 and n_0 = A at compile time.
+template <bool kBranched>
 __global__ void categorical_head_kernel(const float* __restrict__ logits, int ld, const float* __restrict__ u, int B, int A,
-                                        float* __restrict__ action, float* __restrict__ logp,
+                                        CatBranches br, float* __restrict__ action, float* __restrict__ logp,
                                         float* __restrict__ probs_out, const float* __restrict__ mask) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
+  const int K = kBranched ? br.K : 1;
   const float* x = logits + (size_t)b * ld;
-  const float* mk = categorical_row_mask(mask ? mask + (size_t)b * A : nullptr, A);
-  const int j0 = categorical_first_allowed(mk, A);
+  const float* mrow = mask ? mask + (size_t)b * A : nullptr;
   float q[kMaxA];
-  const float s2 = categorical_softmax(x, mk, A, j0, q);              // F.softmax (nn/actor.py:94)
-  if (u) {
-    for (int j = 0; j < A; ++j) q[j] = q[j] / s2;                   // categorical.py:70
-    const int a = inverse_cdf(q, A, u[b], mk, j0);
-    action[b] = (float)a;
-    logp[b] = logf(fminf(fmaxf(q[a], kEps), 1.f - kEps));
-    if (probs_out) for (int j = 0; j < A; ++j) probs_out[(size_t)b * A + j] = q[j];
-  } else {
-    action[b] = (float)argmax_first(q, A, mk, j0);    // play mode works on the raw softmax output
+  for (int i = 0, o = 0; i < K; ++i) {
+    const int n = kBranched ? br.n[i] : A;
+    const float* mk = categorical_row_mask(mrow ? mrow + o : nullptr, n);
+    const int j0 = categorical_first_allowed(mk, n);
+    const float s2 = categorical_softmax(x + o, mk, n, j0, q + o);   // F.softmax (nn/actor.py:94)
+    if (u) {
+      for (int j = 0; j < n; ++j) q[o + j] = q[o + j] / s2;        // categorical.py:70
+      const int a = inverse_cdf(q + o, n, u[(size_t)b * K + i], mk, j0);
+      action[(size_t)b * K + i] = (float)a;
+      if (!kBranched) logp[b] = logf(fminf(fmaxf(q[a], kEps), 1.f - kEps));
+    } else {
+      action[(size_t)b * K + i] = (float)argmax_first(q + o, n, mk, j0);   // play mode works on the raw softmax output
+    }
+    o += n;
+  }
+  if (probs_out) for (int j = 0; j < A; ++j) probs_out[(size_t)b * A + j] = q[j];
+  if (!u) {
     logp[b] = 0.f;
-    if (probs_out) for (int j = 0; j < A; ++j) probs_out[(size_t)b * A + j] = q[j];
+  } else if (kBranched) {
+    float s2[kCatMaxBranches];
+    logp[b] = categorical_logp_row<true>(x, mrow, A, br, action + (size_t)b * K, q, s2);   // q is scratch now
   }
 }
 
@@ -159,9 +172,24 @@ extern "C" int ddrl_categorical_head_m(const float* logits, int ld, const float*
   if (B < 0 || A < 1 || A > kMaxA || ld < A) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!logits || !action || !logp) return DDRL_E_ARG;
-  categorical_head_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, u, B, A, action, logp, probs_out,
-                                                                              mask);
+  categorical_head_kernel<false><<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, u, B, A, CatBranches{}, action,
+                                                                                     logp, probs_out, mask);
   DDRL_LAUNCHED("categorical_head_kernel");
+  return DDRL_OK;
+}
+
+extern "C" int ddrl_multi_categorical_head(const float* logits, int ld, const float* u, int B, int K, const int32_t* nvec,
+                                           float* action, float* logp, float* probs_out, const float* mask, void* stream) {
+  CatBranches br;
+  int A = 0;
+  const int e = cat_branches(K, nvec, &br, &A);
+  if (e != DDRL_OK) return e;
+  if (B < 0 || ld < A) return DDRL_E_ARG;
+  if (B == 0) return DDRL_OK;
+  if (!logits || !action || !logp) return DDRL_E_ARG;
+  categorical_head_kernel<true><<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, u, B, A, br, action, logp,
+                                                                                    probs_out, mask);
+  DDRL_LAUNCHED("multi_categorical_head_kernel");
   return DDRL_OK;
 }
 

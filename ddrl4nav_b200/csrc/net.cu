@@ -21,6 +21,7 @@
 #include <unordered_map>
 #include <vector>
 
+#include "categorical.cuh"
 #include "common.cuh"
 #include "layer_ops.h"
 #include "prep_kernels.cuh"
@@ -116,6 +117,10 @@ struct ddrl_net {
   const float* value_norm = nullptr;
   // DDRL_DIST_BETA (ddrl_net_set_action_bounds): device [2 x act_dim] = low | high, owned.  Null: not set yet.
   float* bounds = nullptr;
+  // DDRL_DIST_MULTI_CATEGORICAL (ddrl_net_set_action_branches): the branch sizes, handed to the kernels by value.  K = 0: not set
+  // yet.  Fixed before the first pass, so no graph key needs them.
+  int32_t nvec[kCatMaxBranches] = {};
+  int nbranch = 0;
   // ACTION_MASK (ddrl_net_set_action_mask, categorical nets): one more observation slot after the encoder's, [B, act_dim] fp32,
   // read by the head, the log-prob pre-pass and the loss kernels
   bool action_mask = false;
@@ -356,8 +361,10 @@ static void add_encoder_tensors(ddrl_net* n, const std::string& pre, int arch, i
 static int round4(int x) { return (x + 3) & ~3; }
 // width of the actor head GEMM: the Beta head emits alpha | beta pre-activations per action dimension
 static int head_n(const ddrl_net* n) { return n->d.dist == DDRL_DIST_BETA ? 2 * n->d.act_dim : n->d.act_dim; }
-// a Beta net cannot run before its action bounds are set
-static bool bounds_missing(const ddrl_net* n) { return n->d.dist == DDRL_DIST_BETA && !n->bounds; }
+// a Beta net cannot run before its action bounds are set, nor a MultiDiscrete net before its branches are
+static bool bounds_missing(const ddrl_net* n) {
+  return (n->d.dist == DDRL_DIST_BETA && !n->bounds) || (n->d.dist == DDRL_DIST_MULTI_CATEGORICAL && n->nbranch == 0);
+}
 
 // observation slots the encoder reads (the action mask, when on, is the slot after them)
 static int encoder_slots(const ddrl_net* n) {
@@ -1521,7 +1528,8 @@ static int forward_chunk(ddrl_net* n, const float* const* obs, long long row0, i
 extern "C" int ddrl_net_create(const ddrl_net_desc* desc, ddrl_net** out) {
   if (!desc || !out) return DDRL_E_ARG;
   if (desc->arch < 0 || desc->arch > DDRL_ARCH_MLP || desc->act_dim < 1 || desc->in_ch < 1) return DDRL_E_ARG;
-  if (desc->dist == DDRL_DIST_CATEGORICAL && desc->act_dim > 64) return DDRL_E_UNSUPPORTED;
+  if ((desc->dist == DDRL_DIST_CATEGORICAL || desc->dist == DDRL_DIST_MULTI_CATEGORICAL) && desc->act_dim > kCatMaxA)
+    return DDRL_E_UNSUPPORTED;
   if ((desc->dist == DDRL_DIST_GAUSSIAN || desc->dist == DDRL_DIST_BETA) && desc->act_dim > 8) return DDRL_E_UNSUPPORTED;
   if (desc->arch == DDRL_ARCH_NAVPED && desc->in_ch < 4) return DDRL_E_ARG;
   ddrl_net* n = new ddrl_net();
@@ -1707,8 +1715,19 @@ extern "C" int ddrl_net_set_action_bounds(ddrl_net* n, const float* low_host, co
   return DDRL_OK;
 }
 
+extern "C" int ddrl_net_set_action_branches(ddrl_net* n, int K, const int32_t* nvec_host) {
+  if (!n || n->d.dist != DDRL_DIST_MULTI_CATEGORICAL) return DDRL_E_ARG;
+  if (n->ws.base) return DDRL_E_STATE;      // the branch table is fixed before the first pass (graph keys do not hold it)
+  CatBranches br;
+  int A = 0;
+  if (cat_branches(K, nvec_host, &br, &A) != DDRL_OK || A != n->d.act_dim) return DDRL_E_ARG;
+  for (int i = 0; i < K; ++i) n->nvec[i] = br.n[i];
+  n->nbranch = K;
+  return DDRL_OK;
+}
+
 extern "C" int ddrl_net_set_action_mask(ddrl_net* n, int on) {
-  if (!n || n->d.dist != DDRL_DIST_CATEGORICAL) return DDRL_E_ARG;
+  if (!n || (n->d.dist != DDRL_DIST_CATEGORICAL && n->d.dist != DDRL_DIST_MULTI_CATEGORICAL)) return DDRL_E_ARG;
   if (n->ws.base) return DDRL_E_STATE;      // a pass has sized the workspace and keyed its graphs on the slot layout
   n->action_mask = on != 0;
   return DDRL_OK;
@@ -1733,6 +1752,10 @@ extern "C" int ddrl_net_forward(ddrl_net* n, const float* const* obs, int n_obs,
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
       TRY(ddrl_categorical_head_m(n->logits, n->ldA, draw ? draw + r0 : nullptr, mb, A, actions + r0, logp + r0,
                                   pi_out ? pi_out + r0 * A : nullptr, mask_rows(n, obs, r0), s));
+    } else if (n->d.dist == DDRL_DIST_MULTI_CATEGORICAL) {
+      const int K = n->nbranch;
+      TRY(ddrl_multi_categorical_head(n->logits, n->ldA, draw ? draw + r0 * K : nullptr, mb, K, n->nvec, actions + r0 * K, logp + r0,
+                                      pi_out ? pi_out + r0 * A : nullptr, mask_rows(n, obs, r0), s));
     } else if (n->d.dist == DDRL_DIST_BETA) {
       TRY(ddrl_beta_head(n->logits, n->ldA, n->bounds, n->bounds + A, draw ? draw + r0 * A : nullptr, mb, A, actions + r0 * A,
                          logp + r0, pi_out ? pi_out + r0 * 2 * A : nullptr, s));
@@ -1797,6 +1820,9 @@ extern "C" int ddrl_net_log_prob(ddrl_net* n, const float* const* obs, int n_obs
     TRY(forward_chunk(n, obs, r0, mb, true, s));
     if (n->d.dist == DDRL_DIST_CATEGORICAL) {
       TRY(ddrl_logp_actions_categorical_m(n->logits, n->ldA, actions + r0, mb, A, out_logp + r0, mask_rows(n, obs, r0), s));
+    } else if (n->d.dist == DDRL_DIST_MULTI_CATEGORICAL) {
+      TRY(ddrl_logp_actions_multi_categorical(n->logits, n->ldA, actions + r0 * n->nbranch, mb, n->nbranch, n->nvec, out_logp + r0,
+                                              mask_rows(n, obs, r0), s));
     } else if (n->d.dist == DDRL_DIST_BETA) {
       TRY(ddrl_logp_actions_beta(n->logits, n->ldA, n->bounds, n->bounds + A, actions + r0 * A, mb, A, out_logp + r0, s));
     } else {
@@ -1835,6 +1861,11 @@ static int backward_body(ddrl_net* n, const float* const* obs, int B_local, int 
                                       invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
                                       old_values ? old_values + r0 : nullptr, stats, n->value_norm,
                                       prox_logp ? prox_logp + r0 : nullptr, is_clip, mask_rows(n, obs, r0), s));
+    } else if (n->d.dist == DDRL_DIST_MULTI_CATEGORICAL) {
+      TRY(ddrl_ppo_loss_multi_categorical(n->logits, n->ldA, actions + r0 * n->nbranch, old_logp + r0, adv + r0, returns + r0, n->vout,
+                                          mb, n->nbranch, n->nvec, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
+                                          old_values ? old_values + r0 : nullptr, stats, n->value_norm,
+                                          prox_logp ? prox_logp + r0 : nullptr, is_clip, mask_rows(n, obs, r0), s));
     } else if (n->d.dist == DDRL_DIST_BETA) {
       TRY(ddrl_ppo_loss_beta(n->logits, n->ldA, n->bounds, n->bounds + A, actions + r0 * A, old_logp + r0, adv + r0, returns + r0,
                              n->vout, mb, A, invB, hp, n->d.shared, n->dlogits, n->ldA, n->dv, loss_sums,
@@ -1900,6 +1931,8 @@ static int backward_impl(ddrl_net* n, const float* const* obs, int n_obs, int B_
   }
   TRY(check_obs(n, obs, n_obs));
   if (!actions || !old_logp || !adv || !returns) return DDRL_E_ARG;
+  // the action bounds (Beta) and the branch table (MultiDiscrete) are not in the key: the bounds live in a net-owned buffer the
+  // graphs read at replay, and the branch table is fixed before the first pass (ddrl_net_set_action_branches)
   const std::string key = graph_key("bwd", {obs[0], n_obs > 1 ? obs[1] : nullptr, n_obs > 2 ? obs[2] : nullptr, mask_rows(n, obs, 0),
                                             actions, old_logp, adv, returns, old_values, n->value_norm, prox_logp, n->params, n->grads,
                                             n->ws.base},

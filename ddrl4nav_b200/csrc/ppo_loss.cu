@@ -28,6 +28,8 @@
 // Beta actor (beta.cuh): head z [B, 2A] -> alpha | beta = 1 + softplus(z); the log-prob is beta_logp, the entropy per element is
 // beta_entropy, both in fp64 and rounded once; the gradient follows the softplus chain (digamma for the log-prob, trigamma for
 // the entropy).
+// MultiDiscrete (categorical.cuh): the categorical loss per branch on its slice; the joint ratio r = exp(sum_i logp_i - old) goes
+// through the same surrogate, and the entropy of a row is the sum of its branch entropies (loss_sums[2] = its mean over rows).
 // ACTION_MASK (categorical.cuh): the categorical kernels take an optional mask [B, A].  Masked entries have p = q = 0, so they add
 // 0 * log(eps) = 0 to the entropy and their logits get exactly zero gradient; a masked taken action (corrupt data) has log-prob
 // log(eps), and the clamp's zero gradient outside [eps, 1 - eps] makes its actor term constant.
@@ -40,7 +42,7 @@ namespace ddrl {
 constexpr float kEpsL = 1.1920928955078125e-07f;
 constexpr float kF32Min = -3.4028234663852886e+38f;
 constexpr float kLogSqrt2PiL = 0.918938533204672741780329736406f;
-constexpr int kMaxAL = 64;
+constexpr int kMaxAL = kCatMaxA;
 
 struct LossParams {
   float ppo_clip, dual_clip, v_coef, ent_coef, inv_B, value_clip;
@@ -49,22 +51,6 @@ struct LossParams {
   const float* prox;              // DECOUPLED_PPO: proximal log-probs [B], or null
   float is_clip;                  // DECOUPLED_PPO: truncation of the behaviour weight, <= 0: none
 };
-
-// log-prob of the taken action a (clamped into [0, A)) under Categorical(logits = x[0..A)) with the row's mask (or null): the
-// masked softmax (categorical.cuh) -> q = p / sum(p) -> clamp(eps, 1 - eps) -> log chain of torch.  Leaves the softmax p[0..A)
-// and s2 = sum(p) for the loss kernel's gradient.  The loss kernel and logp_actions_categorical_kernel share it, and the head
-// kernel the same softmax, so equal logits and masks give equal log-prob bits.
-__device__ __forceinline__ float categorical_logp(const float* __restrict__ x, const float* __restrict__ mask, int A, float action,
-                                                  float* p, float* s2_out) {
-  mask = categorical_row_mask(mask, A);
-  const float s2 = categorical_softmax(x, mask, A, categorical_first_allowed(mask, A), p);
-  int a = (int)action;                      // Categorical.log_prob: value.long()
-  a = a < 0 ? 0 : (a >= A ? A - 1 : a);     // the reference raises on an action outside [0, A); never read out of bounds
-  const float qa = p[a] / s2;
-  const float ca = fminf(fmaxf(qa, kEpsL), 1.f - kEpsL);
-  *s2_out = s2;
-  return logf(ca);
-}
 
 // log-prob of the action row act[0..A) under Normal(mu[0..A), exp(log_std)) summed over A (normal.py log_prob); shared by the
 // Gaussian loss kernel and logp_actions_gaussian_kernel
@@ -149,21 +135,25 @@ __device__ __forceinline__ float value_loss_clipped(float R, float v, const floa
   return fmaxf(lu, lc);
 }
 
+// kBranched (MultiDiscrete, categorical.cuh): actions [B, K]; logp = categorical_logp_row (the sum over the branches), the row's
+// entropy is the sum of the branch entropies, and each branch's dlogits is the categorical gradient on its slice with the common
+// dLoss/dlogp.  Without it (the categorical actor) K = 1 and n_0 = A at compile time.
+template <bool kBranched>
 __global__ void __launch_bounds__(128) ppo_loss_categorical_kernel(
     const float* __restrict__ logits, int ld, const float* __restrict__ actions, const float* __restrict__ old_logp,
-    const float* __restrict__ adv, const float* __restrict__ returns, const float* __restrict__ v, int B, int A,
+    const float* __restrict__ adv, const float* __restrict__ returns, const float* __restrict__ v, int B, int A, CatBranches br,
     LossParams hp, float* __restrict__ dlogits, int ld_d, float* __restrict__ dv, float* __restrict__ loss_sums,
     const float* __restrict__ old_v, float* __restrict__ stats, const float* __restrict__ mask, DetSeq det) {
   __shared__ float scratch[32];
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   float l_actor = 0.f, l_v = 0.f, l_ent = 0.f, l_kl = 0.f, l_cf = 0.f, l_bkl = 0.f;
   if (b < B) {
+    const int K = kBranched ? br.K : 1;
     const float* x = logits + (size_t)b * ld;
+    const float* act = actions + (size_t)b * K;
     float p[kMaxAL];
-    float s2;
-    const float logp = categorical_logp(x, mask ? mask + (size_t)b * A : nullptr, A, actions[b], p, &s2);   // of the taken action
-    int a = (int)actions[b];
-    a = a < 0 ? 0 : (a >= A ? A - 1 : a);
+    float s2[kBranched ? kCatMaxBranches : 1];
+    const float logp = categorical_logp_row<kBranched>(x, mask ? mask + (size_t)b * A : nullptr, A, br, act, p, s2);
     const float Ai = adv[b];
     float w;
     const float log_ratio = decoupled_log_ratio(logp, old_logp, b, hp, stats != nullptr, &w, &l_bkl);
@@ -177,26 +167,33 @@ __global__ void __launch_bounds__(128) ppo_loss_categorical_kernel(
     }
     const float w_lp = -hp.inv_B * (w * dterm) * ratio;                 // dLoss/dlogp
     const float w_ent = hp.shared ? -hp.ent_coef * hp.inv_B : 0.f;      // dLoss/dH_b
-    // gradient wrt q (normalised probs): gq_j
-    float H = 0.f, dot_q = 0.f;
+    float H = 0.f;
     float gq[kMaxAL];
-    for (int j = 0; j < A; ++j) {
-      const float q = p[j] / s2;
-      const float c = fminf(fmaxf(q, kEpsL), 1.f - kEpsL);
-      const float L = fmaxf(logf(c), kF32Min);
-      const float inr = (q >= kEpsL && q <= 1.f - kEpsL) ? 1.f : 0.f;
-      H -= q * L;
-      float g = w_ent * (-(L + inr * q / c));
-      if (j == a) g += w_lp * inr / c;
-      gq[j] = g;
-      dot_q += g * q;
+    float* dx = dlogits + (size_t)b * ld_d;
+    for (int i = 0, o = 0; i < K; ++i) {
+      const int n = kBranched ? br.n[i] : A;
+      int a = (int)act[i];
+      a = a < 0 ? 0 : (a >= n ? n - 1 : a);
+      // gradient wrt q (normalised probs): gq_j
+      float dot_q = 0.f;
+      for (int j = 0; j < n; ++j) {
+        const float q = p[o + j] / s2[i];
+        const float c = fminf(fmaxf(q, kEpsL), 1.f - kEpsL);
+        const float L = fmaxf(logf(c), kF32Min);
+        const float inr = (q >= kEpsL && q <= 1.f - kEpsL) ? 1.f : 0.f;
+        H -= q * L;
+        float g = w_ent * (-(L + inr * q / c));
+        if (j == a) g += w_lp * inr / c;
+        gq[o + j] = g;
+        dot_q += g * q;
+      }
+      // q = p / s2  ->  gp_k = (gq_k - sum_j gq_j q_j) / s2 ;  softmax: dx_k = p_k (gp_k - sum_j gp_j p_j)
+      float dot_p = 0.f;
+      for (int j = 0; j < n; ++j) { gq[o + j] = (gq[o + j] - dot_q) / s2[i]; dot_p += gq[o + j] * p[o + j]; }
+      for (int j = 0; j < n; ++j) dx[o + j] = p[o + j] * (gq[o + j] - dot_p);
+      o += n;
     }
     l_ent = H * hp.inv_B;
-    // q = p / s2  ->  gp_k = (gq_k - sum_j gq_j q_j) / s2 ;  softmax: dx_k = p_k (gp_k - sum_j gp_j p_j)
-    float dot_p = 0.f;
-    for (int j = 0; j < A; ++j) { gq[j] = (gq[j] - dot_q) / s2; dot_p += gq[j] * p[j]; }
-    float* dx = dlogits + (size_t)b * ld_d;
-    for (int j = 0; j < A; ++j) dx[j] = p[j] * (gq[j] - dot_p);
     float dl;
     l_v = value_loss_clipped(returns[b], v[b], old_v, b, hp.value_clip, hp.smooth_l1, hp.value_norm, &dl) * hp.inv_B;
     dv[b] = dl * hp.inv_B * (hp.shared ? hp.v_coef : 1.f);
@@ -381,14 +378,17 @@ __global__ void __launch_bounds__(128) value_loss_kernel(const float* __restrict
 }
 
 // DECOUPLED_PPO pre-pass: out_logp[b] = log-prob of the taken action, bit-equal to the loss kernels' on the same logits / means
+template <bool kBranched>
 __global__ void __launch_bounds__(128) logp_actions_categorical_kernel(const float* __restrict__ logits, int ld,
                                                                        const float* __restrict__ actions, int B, int A,
-                                                                       float* __restrict__ out_logp, const float* __restrict__ mask) {
+                                                                       CatBranches br, float* __restrict__ out_logp,
+                                                                       const float* __restrict__ mask) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   float p[kMaxAL];
-  float s2;
-  out_logp[b] = categorical_logp(logits + (size_t)b * ld, mask ? mask + (size_t)b * A : nullptr, A, actions[b], p, &s2);
+  float s2[kBranched ? kCatMaxBranches : 1];
+  out_logp[b] = categorical_logp_row<kBranched>(logits + (size_t)b * ld, mask ? mask + (size_t)b * A : nullptr, A, br,
+                                                actions + (size_t)b * (kBranched ? br.K : 1), p, s2);
 }
 
 __global__ void __launch_bounds__(128) logp_actions_gaussian_kernel(const float* __restrict__ mu, int ld,
@@ -436,9 +436,10 @@ extern "C" int ddrl_ppo_loss_categorical_m(const float* logits, int ld, const fl
   if (!value_clip_args_ok(hp, old_values)) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!logits || !actions || !old_logp || !adv || !returns || !v || !dlogits || !dv || !loss_sums) return DDRL_E_ARG;
-  ppo_loss_categorical_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(
-      logits, ld, actions, old_logp, adv, returns, v, B, A, make_params(hp, inv_B_global, shared, value_norm, prox_logp, is_clip),
-      dlogits, ld_d, dv, loss_sums, old_values, stats, mask, det_seq(1));
+  ppo_loss_categorical_kernel<false><<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(
+      logits, ld, actions, old_logp, adv, returns, v, B, A, CatBranches{},
+      make_params(hp, inv_B_global, shared, value_norm, prox_logp, is_clip), dlogits, ld_d, dv, loss_sums, old_values, stats, mask,
+      det_seq(1));
   prof_work((8.0 * A + 24.0 + (old_values ? 4.0 : 0.0) + (prox_logp ? 4.0 : 0.0) + (mask ? 4.0 * A : 0.0)) * B);
   DDRL_LAUNCHED("ppo_loss_categorical_kernel");
   return DDRL_OK;
@@ -477,6 +478,28 @@ extern "C" int ddrl_ppo_loss_categorical(const float* logits, int ld, const floa
                                          int ld_d, float* dv, float* loss_sums, void* stream) {
   return ddrl_ppo_loss_categorical_v(logits, ld, actions, old_logp, adv, returns, v, B, A, inv_B_global, hp, shared, dlogits,
                                      ld_d, dv, loss_sums, nullptr, nullptr, stream);
+}
+
+extern "C" int ddrl_ppo_loss_multi_categorical(const float* logits, int ld, const float* actions, const float* old_logp,
+                                               const float* adv, const float* returns, const float* v, int B, int K,
+                                               const int32_t* nvec, float inv_B_global, const ddrl_ppo_hparams* hp, int shared,
+                                               float* dlogits, int ld_d, float* dv, float* loss_sums, const float* old_values,
+                                               float* stats, const float* value_norm, const float* prox_logp, float is_clip,
+                                               const float* mask, void* stream) {
+  CatBranches br;
+  int A = 0;
+  const int e = cat_branches(K, nvec, &br, &A);
+  if (e != DDRL_OK) return e;
+  if (B < 0 || ld < A || ld_d < A || !hp) return DDRL_E_ARG;
+  if (!value_clip_args_ok(hp, old_values)) return DDRL_E_ARG;
+  if (B == 0) return DDRL_OK;
+  if (!logits || !actions || !old_logp || !adv || !returns || !v || !dlogits || !dv || !loss_sums) return DDRL_E_ARG;
+  ppo_loss_categorical_kernel<true><<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(
+      logits, ld, actions, old_logp, adv, returns, v, B, A, br, make_params(hp, inv_B_global, shared, value_norm, prox_logp, is_clip),
+      dlogits, ld_d, dv, loss_sums, old_values, stats, mask, det_seq(1));
+  prof_work((8.0 * A + 4.0 * K + 20.0 + (old_values ? 4.0 : 0.0) + (prox_logp ? 4.0 : 0.0) + (mask ? 4.0 * A : 0.0)) * B);
+  DDRL_LAUNCHED("ppo_loss_multi_categorical_kernel");
+  return DDRL_OK;
 }
 
 extern "C" int ddrl_value_loss(const float* returns, const float* v, int B, float inv_B_global, const ddrl_ppo_hparams* hp,
@@ -524,7 +547,8 @@ extern "C" int ddrl_logp_actions_categorical_m(const float* logits, int ld, cons
   if (B < 0 || A < 1 || A > kMaxAL || ld < A) return DDRL_E_ARG;
   if (B == 0) return DDRL_OK;
   if (!logits || !actions || !out_logp) return DDRL_E_ARG;
-  logp_actions_categorical_kernel<<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, actions, B, A, out_logp, mask);
+  logp_actions_categorical_kernel<false><<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, actions, B, A, CatBranches{},
+                                                                                             out_logp, mask);
   prof_work((4.0 * A + 8.0 + (mask ? 4.0 * A : 0.0)) * B);
   DDRL_LAUNCHED("logp_actions_categorical_kernel");
   return DDRL_OK;
@@ -533,6 +557,22 @@ extern "C" int ddrl_logp_actions_categorical_m(const float* logits, int ld, cons
 extern "C" int ddrl_logp_actions_categorical(const float* logits, int ld, const float* actions, int B, int A, float* out_logp,
                                              void* stream) {
   return ddrl_logp_actions_categorical_m(logits, ld, actions, B, A, out_logp, nullptr, stream);
+}
+
+extern "C" int ddrl_logp_actions_multi_categorical(const float* logits, int ld, const float* actions, int B, int K,
+                                                   const int32_t* nvec, float* out_logp, const float* mask, void* stream) {
+  CatBranches br;
+  int A = 0;
+  const int e = cat_branches(K, nvec, &br, &A);
+  if (e != DDRL_OK) return e;
+  if (B < 0 || ld < A) return DDRL_E_ARG;
+  if (B == 0) return DDRL_OK;
+  if (!logits || !actions || !out_logp) return DDRL_E_ARG;
+  logp_actions_categorical_kernel<true><<<ceil_div(B, 128), 128, 0, (cudaStream_t)stream>>>(logits, ld, actions, B, A, br, out_logp,
+                                                                                            mask);
+  prof_work((4.0 * A + 4.0 * K + 4.0 + (mask ? 4.0 * A : 0.0)) * B);
+  DDRL_LAUNCHED("logp_actions_multi_categorical_kernel");
+  return DDRL_OK;
 }
 
 extern "C" int ddrl_logp_actions_gaussian(const float* mu, int ld, const float* log_std, const float* actions, int B, int A,

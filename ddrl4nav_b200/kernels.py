@@ -316,6 +316,62 @@ def logp_actions_beta(head, low, high, actions) -> torch.Tensor:
     return out
 
 
+def _nvec_arg(nvec):
+    """MultiDiscrete branch sizes -> (K, int32 host array); the C entry points validate them."""
+    n = [int(x) for x in nvec]
+    return len(n), (C.c_int32 * max(len(n), 1))(*n)
+
+
+def multi_categorical_head(logits, nvec, u: Optional[torch.Tensor], mask=None, want_probs: bool = True):
+    """ddrl_multi_categorical_head: (logits [B, sum n], branch sizes nvec, uniforms u [B, K] | None = play mode, mask [B, sum n] |
+    None) -> (actions [B, K], logp [B], the per-branch probabilities [B, sum n] or None)."""
+    logits = _f32c(logits)
+    B, A = logits.shape
+    K, arr = _nvec_arg(nvec)
+    mask = _mask_f32(mask, B, A)
+    action = torch.empty((B, K), dtype=torch.float32, device=logits.device)
+    logp = torch.empty(B, dtype=torch.float32, device=logits.device)
+    probs = torch.empty((B, A), dtype=torch.float32, device=logits.device) if want_probs else None
+    u = None if u is None else _f32c(u)
+    check(_lib.load().ddrl_multi_categorical_head(ptr(logits), A, ptr(u), B, K, arr, ptr(action), ptr(logp), ptr(probs), ptr(mask),
+                                                  current_stream()), "ddrl_multi_categorical_head")
+    return action, logp, probs
+
+
+def ppo_loss_multi_categorical(logits, nvec, actions, old_logp, adv, returns, v, hp: PPOHparams, shared: bool, mask=None,
+                               old_values=None, value_norm=None, prox_logp=None, is_clip: Optional[float] = None,
+                               b_global: Optional[int] = None):
+    """ddrl_ppo_loss_multi_categorical with the statistics on -> (dlogits [B, sum n], dv [B], sums [8]), sums as
+    ppo_loss_categorical_dc; actions [B, K]; the options as ppo_loss_categorical_m."""
+    logits, actions, old_logp, adv, returns, v = map(_f32c, (logits, actions, old_logp, adv, returns, v))
+    old_values, value_norm, prox_logp = (None if t is None else _f32c(t) for t in (old_values, value_norm, prox_logp))
+    B, A = logits.shape
+    K, arr = _nvec_arg(nvec)
+    mask = _mask_f32(mask, B, A)
+    dlogits = torch.empty_like(logits)
+    dv = torch.empty(B, dtype=torch.float32, device=logits.device)
+    sums = torch.zeros(8, dtype=torch.float32, device=logits.device)
+    check(_lib.load().ddrl_ppo_loss_multi_categorical(ptr(logits), A, ptr(actions), ptr(old_logp), ptr(adv), ptr(returns), ptr(v), B,
+                                                      K, arr, 1.0 / float(b_global or B), C.byref(hp), int(shared), ptr(dlogits),
+                                                      A, ptr(dv), ptr(sums), ptr(old_values), ptr(sums[3:]), ptr(value_norm),
+                                                      ptr(prox_logp), float(is_clip or 0.0), ptr(mask), current_stream()),
+          "ddrl_ppo_loss_multi_categorical")
+    return dlogits, dv, sums
+
+
+def logp_actions_multi_categorical(logits, nvec, actions, mask=None) -> torch.Tensor:
+    """Log-probs [B] of the action rows [B, K] under the MultiDiscrete head (mask [B, sum n] or None), bit-equal to the loss and
+    head kernels'."""
+    logits, actions = _f32c(logits), _f32c(actions)
+    B, A = logits.shape
+    K, arr = _nvec_arg(nvec)
+    mask = _mask_f32(mask, B, A)
+    out = torch.empty(B, dtype=torch.float32, device=logits.device)
+    check(_lib.load().ddrl_logp_actions_multi_categorical(ptr(logits), A, ptr(actions), B, K, arr, ptr(out), ptr(mask),
+                                                          current_stream()), "ddrl_logp_actions_multi_categorical")
+    return out
+
+
 def net_log_prob(net, states, actions, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """ddrl_net_log_prob: log-probs [B] of `actions` under the current parameters of the PPO module `net`, for `states` as the
     engine takes them (already normalised under NORM_OBS); written into `out` when given."""

@@ -3,7 +3,7 @@
 from .utils import mlp, merge
 from .base import Basenn, PreNet
 from .critic import Critic
-from .actor import BetaActor, CategoricalActor, Actor, GaussionActor
+from .actor import BetaActor, CategoricalActor, Actor, GaussionActor, MultiCategorical, MultiCategoricalActor
 from .ppo import PPO
 from .nav_encoder import NavPreNet, NavPedPreNet, NavPreNet1D
 from .atari_encoder import AtariPreNet
@@ -12,4 +12,5 @@ from .mlp_encoder import MLPPreNet
 NETWORK_MAP = {"ppo": PPO}
 
 __all__ = ["PPO", "NavPreNet", "Basenn", "PreNet", "NETWORK_MAP", "CategoricalActor", "GaussionActor", "BetaActor", "Critic",
+           "MultiCategoricalActor", "MultiCategorical",
            "AtariPreNet", "MLPPreNet", "Actor", "mlp", "merge", "NavPedPreNet", "NavPreNet1D"]

@@ -2,7 +2,7 @@
 
 `pre` is registered before `actor_linear`, and GaussionActor's `log_std` is a direct Parameter
 (so it precedes everything in named_parameters()), exactly as in the reference.  BetaActor is this library's own
-(non-reference) head for bounded continuous actions."""
+(non-reference) head for bounded continuous actions, and MultiCategoricalActor its own head for MultiDiscrete actions."""
 import numpy as np
 import torch
 from torch import nn
@@ -148,3 +148,82 @@ class BetaActor(Actor):
 
     def _log_prob_from_distribution(self, pi, act):
         return pi.log_prob(act).sum(axis=-1)
+
+
+MAX_BRANCHES = 8           # kCatMaxBranches (csrc/categorical.cuh)
+MAX_HEAD_WIDTH = 64        # kCatMaxA
+
+
+def branch_sizes(nvec):
+    """Validated MultiDiscrete branch sizes: a sequence of 1..8 integers >= 1 whose sum is <= 64 -> tuple of ints."""
+    ok = isinstance(nvec, (list, tuple, np.ndarray, torch.Tensor)) and 1 <= len(nvec) <= MAX_BRANCHES
+    vals = []
+    if ok:
+        for n in nvec:
+            n = n.item() if isinstance(n, (np.generic, torch.Tensor)) else n
+            if isinstance(n, (bool, np.bool_)) or not isinstance(n, (int, np.integer)) or n < 1:
+                ok = False
+                break
+            vals.append(int(n))
+    if not ok or sum(vals) > MAX_HEAD_WIDTH:
+        raise DDRLError("nvec must be a sequence of 1..%d integers >= 1 with a sum <= %d (got %r)" % (MAX_BRANCHES, MAX_HEAD_WIDTH,
+                                                                                                  nvec))
+    return tuple(vals)
+
+
+class MultiCategorical:
+    """The product of independent Categoricals, one per branch, over per-branch probabilities [B, sum n] (gym's MultiDiscrete):
+    sample() -> [..., B, K], log_prob(actions [B, K]) and entropy() summed over the branches in branch order."""
+
+    def __init__(self, probs, nvec):
+        self.nvec = tuple(nvec)
+        self.probs = probs
+        self.dists = [Categorical(p) for p in torch.split(probs, list(self.nvec), dim=-1)]
+
+    def sample(self, sample_shape=torch.Size()):
+        return torch.stack([d.sample(sample_shape) for d in self.dists], dim=-1)
+
+    def log_prob(self, actions):
+        out = self.dists[0].log_prob(actions[..., 0])
+        for i, d in enumerate(self.dists[1:], 1):
+            out = out + d.log_prob(actions[..., i])
+        return out
+
+    def entropy(self):
+        out = self.dists[0].entropy()
+        for d in self.dists[1:]:
+            out = out + d.entropy()
+        return out
+
+
+class MultiCategoricalActor(Actor):
+    """MultiDiscrete policy: K independent categorical branches of nvec = (n_1, ..., n_K) actions (1 <= K <= 8, sum n_i <= 64)
+    over one head.  actor_linear is Linear(F, sum n_i); columns [o_i, o_i + n_i), o_i = n_1 + ... + n_{i-1}, hold branch i's
+    logits.  Actions are [B, K] (fp32 holding integers); the log-prob and the entropy are the sums over the branches.
+    nvec = (A,) is the CategoricalActor, with actions [B, 1].
+
+    nvec is configuration, like BetaActor's bounds: no parameter, no state_dict key, no weight-blob byte, so a predictor must be
+    built with the learner's nvec.  A different sum n_i is caught by the parameter shapes; a different split with the same sum
+    cannot be detected.  action_output_dim, when given, must equal sum n_i.
+
+    Not derived from a reference class: the reference's ForwardThread only knows Gaussian and Categorical actors; a MultiDiscrete
+    net is served by PPO.act, ForwardModule and server.threads.ForwardThread, which do not dispatch on the actor type."""
+    DIST = "multi_categorical"
+
+    def __init__(self, nvec, device="cpu", last_input_dim=512, pre=None, action_output_dim=None, soft_max_grid=True,
+                 nn_dtype=torch.float32):
+        Actor.__init__(self, pre=pre, device=device)
+        self.nvec = branch_sizes(nvec)
+        if action_output_dim is not None and action_output_dim != sum(self.nvec):
+            raise DDRLError("MultiCategoricalActor: action_output_dim %r differs from sum(nvec) = %d" % (action_output_dim,
+                                                                                                       sum(self.nvec)))
+        self.action_output_dim = sum(self.nvec)
+        self.actor_linear = nn.Linear(last_input_dim, self.action_output_dim)
+
+    def _distribution(self, logits, play_mode=False):
+        from .. import kernels
+        _, _, probs = kernels.multi_categorical_head(logits, self.nvec, None)    # per-branch softmax (play-mode path)
+        return probs if play_mode else MultiCategorical(probs, self.nvec)
+
+    def _log_prob_from_distribution(self, pi, act):
+        return pi.log_prob(act)

@@ -122,10 +122,11 @@ class PPO(Basenn):
             raise DDRLError("DECOUPLED_IS_CLIP needs DECOUPLED_PPO=True")
         self.last_prox_logps = None     # DECOUPLED_PPO: the proximal log-probs [B_local] of the last learn call (persistent)
         # invalid-action masking (non-reference, off by default; Huang & Ontanon 2022): one more state slot after the encoder's,
-        # [B, A], action j allowed iff != 0; act / forward sample, and learn trains, the masked categorical distribution
+        # [B, A], action j allowed iff != 0; act / forward sample, and learn trains, the masked categorical distribution (per branch
+        # for a MultiCategoricalActor, whose mask is [B, sum n])
         self.action_mask = _flag_option(config_nn, "ACTION_MASK")
-        if self.action_mask and getattr(actor, "DIST", None) != "categorical":
-            raise DDRLError("ACTION_MASK needs a CategoricalActor (got %s)" % type(actor).__name__)
+        if self.action_mask and getattr(actor, "DIST", None) not in ("categorical", "multi_categorical"):
+            raise DDRLError("ACTION_MASK needs a CategoricalActor or a MultiCategoricalActor (got %s)" % type(actor).__name__)
         self.hp = kernels.make_hparams(
             ppo_clip=_cfg(config_nn, "PPO_CLIP", 0.2), dual_clip=_cfg(config_nn, "DUEL_PPO_CLIP", 3),
             v_coef=_cfg(config_nn, "V_LOSS_THETA", 1.0), ent_coef=_cfg(config_nn, "ENTROPY_LOSS_THETA", 0.05),
@@ -175,7 +176,8 @@ class PPO(Basenn):
         return self.prenet if self.prenet is not None else self.actor.pre
 
     def _act_dim(self):
-        """Action dimensions A: the Beta head emits alpha | beta pre-activations, 2A columns."""
+        """Action dimensions A: the Beta head emits alpha | beta pre-activations, 2A columns.  MultiCategoricalActor: the head
+        width sum n_i."""
         n = self.actor.actor_linear.out_features
         return n // 2 if self.actor.DIST == "beta" else n
 
@@ -297,6 +299,9 @@ class PPO(Basenn):
             A = s["act_dim"]
             check(lib.ddrl_net_set_action_bounds(h, (C.c_float * A)(*self.actor.action_low), (C.c_float * A)(*self.actor.action_high)),
                   "ddrl_net_set_action_bounds")
+        if s["dist"] == "multi_categorical":
+            nvec = self.actor.nvec
+            check(lib.ddrl_net_set_action_branches(h, len(nvec), (C.c_int32 * len(nvec))(*nvec)), "ddrl_net_set_action_branches")
         if self.action_mask:
             check(lib.ddrl_net_set_action_mask(h, 1), "ddrl_net_set_action_mask")
         if self.obs_rms is not None:
@@ -473,9 +478,10 @@ class PPO(Basenn):
     def act(self, states, draw=None, play_mode=False, want_pi=False):
         """Fused compute body of ForwardThread.run (server/forward.py:128-146).
 
-        draw: uniforms [B] (categorical), standard normals [B,A] (gaussian) or uniforms [B,A] (beta); generated on the
-        device when None and not play_mode.  Returns (actions [B] | [B,A], logps [B], values [V,B,1][, pi]); V = number of
-        critics (1 unless add_critic was called); pi = probs [B,A], mu [B,A] or alpha | beta [B,2A]."""
+        draw: uniforms [B] (categorical), standard normals [B,A] (gaussian), uniforms [B,A] (beta) or uniforms [B,K]
+        (multi-categorical, K branches); generated on the device when None and not play_mode.  Returns (actions [B] | [B,A] |
+        [B,K], logps [B], values [V,B,1][, pi]); V = number of critics (1 unless add_critic was called); pi = probs [B,A], mu
+        [B,A], alpha | beta [B,2A] or the per-branch probabilities [B,A] (A = sum n_i)."""
         self._ensure_engine()
         lib = _lib.load()
         if self.obs_rms is not None:
@@ -490,11 +496,14 @@ class PPO(Basenn):
             draw = None
         elif draw is None and dist_name == "categorical":
             draw = torch.rand(B, device=dev)
+        elif draw is None and dist_name == "multi_categorical":
+            draw = torch.rand(B, len(self.actor.nvec), device=dev)
         elif draw is None:
             draw = (torch.randn if dist_name == "gaussian" else torch.rand)(B, A, device=dev)
         else:
             draw = draw.to(device=dev, dtype=torch.float32).contiguous()
-        actions = torch.empty((B,) if dist_name == "categorical" else (B, A), dtype=torch.float32, device=dev)
+        shape = (B,) if dist_name == "categorical" else ((B, len(self.actor.nvec)) if dist_name == "multi_categorical" else (B, A))
+        actions = torch.empty(shape, dtype=torch.float32, device=dev)
         logps = torch.empty(B, dtype=torch.float32, device=dev)
         V = len(self._critics)
         values = torch.empty(V, B, dtype=torch.float32, device=dev)       # shared mode: the engine fills all V rows
@@ -522,11 +531,15 @@ class PPO(Basenn):
     def forward(self, states, act=None, play_mode=False):
         """Reference-shaped output: ((pi, log_p), [values [B,1]]) with pi = Categorical / Normal, or the raw
         softmax / mu tensor in play mode (nn/actor.py:58-67,90-98).  BetaActor: the Beta mapped onto the bounds
-        (BetaActor.distribution), or the mean action [B,A] in play mode.  ACTION_MASK: the engine's softmax is the masked one,
-        so the Categorical gives masked actions probability 0."""
+        (BetaActor.distribution), or the mean action [B,A] in play mode.  MultiCategoricalActor: a MultiCategorical (one
+        Categorical per branch), or the per-branch softmax [B, sum n] in play mode.  ACTION_MASK: the engine's softmax is the
+        masked one, so the Categorical gives masked actions probability 0."""
         mean, _, values, pi_raw = self.act(states, draw=None, play_mode=True, want_pi=True)
         if self.actor.DIST == "categorical":
             pi = pi_raw if play_mode else Categorical(pi_raw)
+        elif self.actor.DIST == "multi_categorical":
+            from .actor import MultiCategorical
+            pi = pi_raw if play_mode else MultiCategorical(pi_raw, self.actor.nvec)
         elif self.actor.DIST == "beta":
             pi = mean if play_mode else self.actor.distribution(pi_raw)
         else:

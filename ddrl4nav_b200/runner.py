@@ -6,13 +6,20 @@ from types import SimpleNamespace
 
 import torch
 
-from .nn import (PPO, AtariPreNet, BetaActor, CategoricalActor, Critic, GaussionActor, MLPPreNet, NavPedPreNet, NavPreNet,
-                 NavPreNet1D)
+from ._lib import DDRLError
+from .nn import (PPO, AtariPreNet, BetaActor, CategoricalActor, Critic, GaussionActor, MLPPreNet, MultiCategoricalActor, NavPedPreNet,
+                 NavPreNet, NavPreNet1D)
 
 
 def _bounds_kwargs(actor_cls, config_nn):
     """BetaActor's action interval from the optional config_nn.ACTION_LOW / ACTION_HIGH (numbers or length-A sequences;
-    BetaActor validates them).  Other actors take no bounds."""
+    BetaActor validates them), and MultiCategoricalActor's branch sizes from config_nn.ACTION_NVEC (required; the actor
+    validates them).  Other actors take neither."""
+    if actor_cls is MultiCategoricalActor:
+        nvec = getattr(config_nn, "ACTION_NVEC", None)
+        if nvec is None:
+            raise DDRLError("MultiCategoricalActor needs config_nn.ACTION_NVEC (the branch sizes)")
+        return {"nvec": nvec}
     if actor_cls is not BetaActor:
         return {}
     kw = {}
@@ -75,14 +82,21 @@ _KINDS = {
     # NON-reference Beta actor on [ACTION_LOW, ACTION_HIGH] (default [-1, 1]) per dimension: C2's encoder, and C5's
     "navlaser_beta": (lambda: NavPreNet1D(image_channel=3), "beta", 2, False),
     "navimg_beta": (lambda: NavPreNet(image_channel=1), "beta", 2, True),
+    # NON-reference MultiDiscrete actor (act_dim: the default branch sizes, ACTION_NVEC overrides them): C5's 28 (v, w) commands
+    # as 4 speeds x 7 turn rates on the shared encoder, and a 5 x 9 grid on C2's unshared one
+    "navimg_md": (lambda: NavPreNet(image_channel=1), "multi_categorical", (4, 7), True),
+    "navlaser_md": (lambda: NavPreNet1D(image_channel=3), "multi_categorical", (5, 9), False),
 }
 
 
 def make_net(kind: str, device="cuda", gemm_mode=None, **hyper):
     """PPO net of one of the named configurations with the reference's default hyper-parameters
-    (config/config_nn.py:27-57); `hyper` overrides ConfigNN attribute names (e.g. TRAINING_ITER_TIME=1, or ACTION_LOW /
-    ACTION_HIGH for the Beta kinds)."""
+    (config/config_nn.py:27-57); `hyper` overrides ConfigNN attribute names (e.g. TRAINING_ITER_TIME=1, ACTION_LOW /
+    ACTION_HIGH for the Beta kinds, or ACTION_NVEC for the MultiDiscrete kinds)."""
     mk, dist, act_dim, shared = _KINDS[kind]
+    if dist == "multi_categorical":
+        hyper.setdefault("ACTION_NVEC", act_dim)
+        act_dim = None
     cfg_nn = dict(SHARE_CNN_NET=shared, PPO_CLIP=0.2, DUEL_PPO_CLIP=3, V_LOSS_THETA=1.0, ENTROPY_LOSS_THETA=0.05,
                   CLIP_GRID=True, CLIP_GRID_NUM=0.5, SMOOTH_L1_LOSS=False, LEARNING_RATE=2e-4, ACTOR_LEARNING_RATE=5e-5,
                   CRITIC_LEARNING_RATE=1e-3, TRAINING_ITER_TIME=10)
@@ -92,7 +106,7 @@ def make_net(kind: str, device="cuda", gemm_mode=None, **hyper):
     config_nn = SimpleNamespace(**cfg_nn)
     config = SimpleNamespace(DEVICE=device, TASK_NAME="t-127.0.0.1", MODULE_KEY="MODEL")
     feat = 128 if kind == "mlp" else 512
-    actor_cls = {"gaussian": GaussionActor, "beta": BetaActor}.get(dist, CategoricalActor)
+    actor_cls = {"gaussian": GaussionActor, "beta": BetaActor, "multi_categorical": MultiCategoricalActor}.get(dist, CategoricalActor)
     bounds = _bounds_kwargs(actor_cls, config_nn)
     if shared:
         actor = actor_cls(action_output_dim=act_dim, device=device, last_input_dim=feat, **bounds)

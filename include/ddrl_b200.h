@@ -39,8 +39,11 @@ enum ddrl_arch {               /* encoder family (USTC_lab/nn/__init__.py:12-18)
 enum ddrl_dist {
   DDRL_DIST_CATEGORICAL = 0,   /* nn/actor.py:75 */
   DDRL_DIST_GAUSSIAN = 1,      /* nn/actor.py:43 */
-  DDRL_DIST_BETA = 2           /* non-reference: Beta on [low_j, high_j] per action dimension (ddrl4nav_b200/nn/actor.py BetaActor);
+  DDRL_DIST_BETA = 2,          /* non-reference: Beta on [low_j, high_j] per action dimension (ddrl4nav_b200/nn/actor.py BetaActor);
                                   act_dim = A <= 8 dimensions, head width 2A; needs ddrl_net_set_action_bounds */
+  DDRL_DIST_MULTI_CATEGORICAL = 3  /* non-reference: MultiDiscrete, K <= 8 independent categorical branches of n_1..n_K actions
+                                      over one head (ddrl4nav_b200/nn/actor.py MultiCategoricalActor); act_dim = n_1 + ... + n_K
+                                      <= 64 (the head width); needs ddrl_net_set_action_branches */
 };
 enum ddrl_gemm_mode {
   DDRL_GEMM_SIMT_F32 = 0,      /* CUDA-core fp32 FMA (reference / fallback-free baseline) */
@@ -167,6 +170,15 @@ int ddrl_categorical_head(const float* logits, int ld, const float* u, int B, in
  * masked probabilities.  Masked logits are never read. */
 int ddrl_categorical_head_m(const float* logits, int ld, const float* u, int B, int A,
                             float* action, float* logp, float* probs_out, const float* mask, void* stream);
+/* MultiDiscrete head (non-reference): nvec HOST [K] branch sizes n_i >= 1, 1 <= K <= 8 (else DDRL_E_ARG), A = sum n_i <= 64 (else
+ * DDRL_E_UNSUPPORTED); logits [B, A] (row stride ld >= A), branch i on the columns [o_i, o_i + n_i), o_i = n_1 + ... + n_{i-1}.
+ * Each branch is ddrl_categorical_head_m on its own slice (its own mask slice, with its own "allows nothing" rule): u [B, K]
+ * uniforms, branch i inverts its CDF with u[b, i] into action[b, i] (actions [B, K] fp32, integer-valued); logp[b] = the sum over
+ * the branches of log(clamp(q_i[a_i], eps, 1 - eps)), added in branch order in fp32 (ddrl_logp_actions_multi_categorical's bits).
+ * u NULL => play mode: the first-max argmax per branch, logp = 0.  probs_out (optional) [B, A]: the per-branch probabilities
+ * (play mode: the per-branch softmax).  mask [B, A] or NULL.  K = 1 gives ddrl_categorical_head_m's bits. */
+int ddrl_multi_categorical_head(const float* logits, int ld, const float* u, int B, int K, const int32_t* nvec,
+                                float* action, float* logp, float* probs_out, const float* mask, void* stream);
 /* Gaussian head (nn/actor.py:58-70): a = mu + exp(log_std)*eps (mul, then add);
  * logp = sum_j Normal(mu,std).log_prob(a); eps NULL => play mode (a = mu, logp = 0). */
 int ddrl_gaussian_head(const float* mu, int ld, const float* log_std, const float* eps, int B, int A,
@@ -260,6 +272,16 @@ int ddrl_ppo_loss_beta(const float* head, int ld, const float* low, const float*
                        float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dhead, int ld_d, float* dv,
                        float* loss_sums, const float* old_values, float* stats, const float* value_norm, const float* prox_logp,
                        float is_clip, void* stream);
+/* MultiDiscrete actor (non-reference): the loss of ddrl_ppo_loss_categorical_m, every option included, for the head, nvec and
+ * mask of ddrl_multi_categorical_head and actions [B, K].  logp = the sum of the branch log-probs, the ratio r = exp(logp - old)
+ * (or - prox) is the joint one (so are stats[0..1]), the entropy of a row is the sum of its branch entropies (loss_sums[2]: its
+ * mean over the rows), and branch i's dlogits is the categorical gradient on its slice.  K = 1 gives ddrl_ppo_loss_categorical_m's
+ * bits. */
+int ddrl_ppo_loss_multi_categorical(const float* logits, int ld, const float* actions, const float* old_logp,
+                                    const float* adv, const float* returns, const float* v, int B, int K, const int32_t* nvec,
+                                    float inv_B_global, const ddrl_ppo_hparams* hp, int shared, float* dlogits, int ld_d,
+                                    float* dv, float* loss_sums, const float* old_values, float* stats, const float* value_norm,
+                                    const float* prox_logp, float is_clip, const float* mask, void* stream);
 /* out_logp[b] (DEVICE [B]) = log-prob of the taken action under Categorical(logits) (actions [B], integer-valued) or under
  * Normal(mu, exp(log_std)) summed over A (actions [B, A]), computed by the same device code as the loss kernels above: equal
  * logits / means give equal bits.  The proximal log-probs of DECOUPLED_PPO (ddrl_net_log_prob). */
@@ -271,6 +293,10 @@ int ddrl_logp_actions_categorical_m(const float* logits, int ld, const float* ac
                                     const float* mask, void* stream);
 int ddrl_logp_actions_gaussian(const float* mu, int ld, const float* log_std, const float* actions, int B, int A,
                                float* out_logp, void* stream);
+/* the same for the MultiDiscrete actor (actions [B, K], head / nvec / mask as ddrl_multi_categorical_head): the bits of
+ * ddrl_ppo_loss_multi_categorical's log-prob, and of ddrl_multi_categorical_head's for the actions it emitted */
+int ddrl_logp_actions_multi_categorical(const float* logits, int ld, const float* actions, int B, int K, const int32_t* nvec,
+                                        float* out_logp, const float* mask, void* stream);
 /* the same for the Beta actor (actions [B, A], head / low / high as ddrl_ppo_loss_beta) */
 int ddrl_logp_actions_beta(const float* head, int ld, const float* low, const float* high, const float* actions, int B, int A,
                            float* out_logp, void* stream);
@@ -387,9 +413,14 @@ int ddrl_net_set_value_norm(ddrl_net* net, const float* applied);
  * else DDRL_E_ARG; another distribution: DDRL_E_ARG.  Until it is called, ddrl_net_forward, ddrl_net_log_prob and the backward
  * passes of a Beta net return DDRL_E_STATE.  Captured graphs read the buffer when they replay, so new bounds need no recapture. */
 int ddrl_net_set_action_bounds(ddrl_net* net, const float* low_host, const float* high_host);
-/* ACTION_MASK (DDRL_DIST_CATEGORICAL only, else DDRL_E_ARG): on != 0 adds one observation slot after the encoder's, the action
- * mask [B, act_dim] (fp32, action j allowed iff != 0), which ddrl_net_forward, ddrl_net_log_prob and the backward passes hand
- * to the _m head, log-prob and loss kernels micro-batch by micro-batch; ddrl_net_num_obs then counts it and
+/* DDRL_DIST_MULTI_CATEGORICAL: the branch sizes nvec_host[0..K) (HOST, copied into the net).  Another distribution, an invalid
+ * table (as ddrl_multi_categorical_head) or a sum other than act_dim: DDRL_E_ARG.  Call it before the first pass: once a pass has
+ * run it returns DDRL_E_STATE.  Until it is called, ddrl_net_forward, ddrl_net_log_prob and the backward passes of such a net
+ * return DDRL_E_STATE.  It adds no parameter. */
+int ddrl_net_set_action_branches(ddrl_net* net, int K, const int32_t* nvec_host);
+/* ACTION_MASK (DDRL_DIST_CATEGORICAL or DDRL_DIST_MULTI_CATEGORICAL, else DDRL_E_ARG): on != 0 adds one observation slot after
+ * the encoder's, the action mask [B, act_dim] (fp32, action j allowed iff != 0), which ddrl_net_forward, ddrl_net_log_prob and the
+ * backward passes hand to the masked head, log-prob and loss kernels micro-batch by micro-batch; ddrl_net_num_obs then counts it and
  * ddrl_net_obs_elems(mask slot) returns act_dim.  The encoders never read it.  Call it before the first pass: once a pass has
  * run it returns DDRL_E_STATE.  It adds no parameter. */
 int ddrl_net_set_action_mask(ddrl_net* net, int on);
@@ -401,8 +432,9 @@ int64_t ddrl_net_obs_elems(const ddrl_net* net, int slot);
 
 /* Forward module compute body (server/forward.py:128-146): obs[i] fp32 device [B, ...] in the
  * reference's NCHW/state-list order; draw = uniforms [B] (categorical), N(0,1) [B,A]
- * (gaussian) or uniforms [B,A] (beta), NULL => play mode.  Outputs: actions [B] or [B,A]; logp [B]; values [B] (the
- * caller views it as [V=1,B,1]); pi_out (optional) probs [B,A], mu [B,A] or alpha | beta [B,2A]. */
+ * (gaussian), uniforms [B,A] (beta) or uniforms [B,K] (multi-categorical), NULL => play mode.  Outputs: actions [B], [B,A] or
+ * [B,K]; logp [B]; values [B] (the caller views it as [V=1,B,1]); pi_out (optional) probs [B,A], mu [B,A], alpha | beta [B,2A]
+ * or the per-branch probabilities [B,A]. */
 int ddrl_net_forward(ddrl_net* net, const float* const* obs, int n_obs, int B, const float* draw,
                      float* actions, float* logp, float* values, float* pi_out, void* stream);
 
