@@ -159,6 +159,10 @@ def _lin(p, pre, name, x):
 # all differ there.  TIE_HOOK lets the parity tests (a) record every pre-activation and (b) re-run the backward with
 # the branch of chosen tie elements flipped, so that "equal up to measure-zero ties" can be asserted exactly.
 TIE_HOOK = None      # callable(layer_name, z, a, slope_neg) -> a'   (test infrastructure only)
+# The same holds for the 2 x 2 max pools of the nav encoders: two activations of one window that agree to fp32 rounding may
+# rank either way.  POOL_HOOK replaces the pool so that the tests can record those windows and route the gradient of chosen
+# ones to the runner-up.
+POOL_HOOK = None     # callable(layer_name, a) -> max_pool2d(a, 2, stride=2)   (test infrastructure only)
 
 
 def _act(name, z, slope):
@@ -190,7 +194,8 @@ class TieRecorder:
 def _conv_relu_pool(p, pre, name, x, pad):
     # nn/nav_encoder.py:29-31,100-102: max_pool2d(relu(conv(x)), 2, stride=2)
     z = F.conv2d(x, p[pre + name + ".weight"], p[pre + name + ".bias"], padding=pad)
-    return F.max_pool2d(_act(pre + name, z, 0.0), 2, stride=2)
+    a = _act(pre + name, z, 0.0)
+    return POOL_HOOK(pre + name, a) if POOL_HOOK is not None else F.max_pool2d(a, 2, stride=2)
 
 
 def encoder_forward(arch: str, p: Dict[str, Tensor], pre: str, states: Sequence[Tensor]) -> Tensor:

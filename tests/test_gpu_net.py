@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 import torch
 
+import engine_state_ref as ES
 from oracle import restate as R
 
 pytestmark = pytest.mark.gpu
@@ -99,55 +100,18 @@ def _learn_case(kind, B, seed=9):
     return spec, params, states, a, old, adv, ret
 
 
-def _oracle_grads(spec, params, states, adv, a, old, ret, flips=None):
-    """Oracle gradients; `flips` = {layer: [flat indices]} re-runs the backward with those activation branches flipped."""
-    rec = R.TieRecorder(flips)
-    R.TIE_HOOK = rec
-    try:
-        st = R.LearnState(spec, params)
-        losses, raw, norm = R.learn_iteration(st, states, adv, a, old, ret, R.PPOHyper(), apply_update=False)
-    finally:
-        R.TIE_HOOK = None
-    return losses, raw, rec.z
-
-
-TIE_EPS = 1e-6      # an activation with |z| < TIE_EPS * max|z| of its layer is zero to within fp32 rounding: a tie
-
-
 @pytest.mark.parametrize("kind,B", [("pong", 8), ("navimg", 6), ("navlaser", 4), ("pong", 40), ("navped", 5), ("navlaser3", 4)])
 def test_backward_grads_match_oracle(kind, B):
     """Every parameter gradient within 2e-5 of its tensor's max.  relu / leaky_relu are not differentiable at 0, and a
     pre-activation that is zero to fp32 rounding (|z| < 1e-6 max|z|) may take either branch depending on summation
     order (the reference itself differs between its CPU and CUDA paths there).  If the plain comparison fails, the
-    residual must be explained EXACTLY by flipping the branch of some of those tie elements in the oracle."""
+    residual must be explained EXACTLY by flipping the branch of some of those tie elements in the oracle
+    (engine_state_ref.grads_match_oracle)."""
     spec, params, states, a, old, adv, ret = _learn_case(kind, B)
-    losses, raw, zs = _oracle_grads(spec, params, states, adv, a, old, ret)
     net, _, _ = make(kind)
     net.backward_only([s.to(DEV) for s in states], adv.to(DEV), a.to(DEV), old.to(DEV), ret.to(DEV))
-    grads = {n: g.detach().cpu().double() for n, g in net.named_grads().items()}
-    scale = {n: max(float(g.abs().max()), 1e-30) for n, g in raw.items()}
-
-    def worst_err(ref):
-        return max(float((grads[n] - ref[n].double()).abs().max()) / scale[n] for n in ref)
-
-    worst = worst_err(raw)
-    if worst >= 2e-5:
-        ties = [(name, int(i)) for name, z in zs.items()
-                for i in (z.reshape(-1).abs() < TIE_EPS * float(z.abs().max())).nonzero().flatten().tolist()]
-        assert 0 < len(ties) <= 64, (worst, len(ties))
-        chosen = {}
-        for name, i in ties:
-            # flipping tie t changes the gradients by D_t; it is part of the explanation iff the residual projects onto D_t
-            _, g1, _ = _oracle_grads(spec, params, states, adv, a, old, ret, {name: [i]})
-            num = sum(float(((grads[n] - raw[n].double()) * (g1[n] - raw[n]).double()).sum()) / scale[n] ** 2 for n in raw)
-            den = sum(float(((g1[n] - raw[n]).double() ** 2).sum()) / scale[n] ** 2 for n in raw)
-            if den > 0 and abs(num / den - 1.0) < 0.2:
-                chosen.setdefault(name, []).append(i)
-        assert chosen, ("gradient mismatch not explained by activation ties", worst, ties)
-        _, raw2, _ = _oracle_grads(spec, params, states, adv, a, old, ret, chosen)
-        worst = worst_err(raw2)
-        print(kind, B, "activation ties taken on the other branch:", chosen)
-    assert worst < 2e-5, worst
+    oracle = ES.learn_oracle(spec, params, states, adv, a, old, ret, dtype=torch.float32)
+    worst, losses = ES.grads_match_oracle(net.named_grads(), oracle, label="%s B=%d" % (kind, B))
     sums = net._grads[net._P:net._P + 3].cpu().numpy()
     assert np.allclose(sums, [losses["ActorLoss"], losses["VLoss"], losses["EntLoss"]], rtol=1e-5, atol=1e-6)
     print(kind, B, "worst grad err / max|g| = %.2e" % worst)
